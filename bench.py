@@ -21,6 +21,9 @@ with sqrt(N) so that pairs per GPU stay fixed ("weak").
   weighted   (N=1) BASELINE config 3 -- weighted, 50k-leaf tree x 20k samples -- with the same keys
   sharded    (N>1) the same workload with the sample-sharded embedding (peer stores + NCCL) per rank
   strong     fixed-size run (cfg4s: 100k-leaf tree x 30k samples) for strong scaling over N
+
+--dump-outputs DIR writes the distances the `value` leg computed in its last timed step (see OutputDump), so that
+two builds can be compared output for output on the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -37,6 +40,9 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+
+DUMP_BYTES = 60_000_000  # --dump-outputs: data bytes in all, under 64 MB with the .npy headers
+DUMP_SEED = 0
 
 CONFIGS = {
     # name: (mode, leaves, samples, density, tree_seed, table_seed)
@@ -301,8 +307,62 @@ class Harness:
             self.dist.destroy_process_group()
 
 
-def device_leg(h, ctx, tree, csr, weighted, flags, steps, warmup, sampler=None):
-    """`value`: inputs resident in HBM, distances stay in HBM; CUDA events, max over ranks."""
+class _DeviceArray:
+    """A float32 device buffer of the engine, seen by torch through the CUDA array interface (no copy)."""
+
+    def __init__(self, addr, n):
+        self.__cuda_array_interface__ = {"shape": (n,), "typestr": "<f4", "data": (addr, False), "version": 2}
+
+
+class OutputDump:
+    """--dump-outputs: the flat lower triangle (IterPairs order, float32) that the `value` leg's last timed step
+    left in HBM, as DIR/distances.npy.  When it exceeds DUMP_BYTES, a fixed seeded sample of pairs instead, with
+    their flat indices (exact in float64) as DIR/distances_index.npy.  Each band is copied on the device when the
+    engine hands it out (it is complete then, and its buffer is reused after the next call); with several ranks
+    every rank fills its own bands and a sum over the ranks joins them."""
+
+    def __init__(self, directory, n_pairs, device):
+        import torch
+
+        self.torch, self.dir = torch, directory
+        self.index = None
+        m = n_pairs
+        if 4 * n_pairs > DUMP_BYTES:
+            self.index = np.unique(np.random.default_rng(DUMP_SEED).integers(0, n_pairs, DUMP_BYTES // 12))
+            self.index_dev = torch.from_numpy(self.index).to(device)
+            m = len(self.index)
+        self.out = torch.zeros(m, dtype=torch.float32, device=device)
+        self.stream = torch.cuda.Stream(device)
+        torch.cuda.synchronize(device)
+
+    def drain(self, job):
+        """job.drain() that also copies every band into the dump."""
+        while True:
+            addr, first, n = job.next_raw_f32()
+            if n == 0:
+                return
+            band = self.torch.as_tensor(_DeviceArray(addr, n), device=self.out.device)
+            with self.torch.cuda.stream(self.stream):
+                if self.index is None:
+                    self.out[first:first + n] = band
+                else:
+                    lo, hi = np.searchsorted(self.index, [first, first + n])
+                    self.out[lo:hi] = band[self.index_dev[lo:hi] - first]
+            self.stream.synchronize()
+
+    def write(self, h):
+        if h.dist is not None:
+            h.dist.all_reduce(self.out)
+        if h.rank == 0:
+            os.makedirs(self.dir, exist_ok=True)
+            np.save(os.path.join(self.dir, "distances.npy"), self.out.cpu().numpy())
+            if self.index is not None:
+                np.save(os.path.join(self.dir, "distances_index.npy"), self.index.astype(np.float64))
+
+
+def device_leg(h, ctx, tree, csr, weighted, flags, steps, warmup, sampler=None, dump=None):
+    """`value`: inputs resident in HBM, distances stay in HBM; CUDA events, max over ranks.  `dump`: an OutputDump
+    that receives the last timed step's distances."""
     from frackyfrac_b200 import engine
 
     rp, col, val = csr
@@ -314,8 +374,12 @@ def device_leg(h, ctx, tree, csr, weighted, flags, steps, warmup, sampler=None):
     h.barrier()
     t0 = time.perf_counter()
     dev_ms, launches = 0.0, 0
-    for _ in range(steps):
-        job.restart(); job.drain()
+    for s in range(steps):
+        job.restart()
+        if dump is not None and s == steps - 1:
+            dump.drain(job)
+        else:
+            job.drain()
         info = job.info()
         dev_ms += info.run_ms
         launches += info.kernel_launches
@@ -526,10 +590,13 @@ def run_ours(args, world, rank, local_rank):
     flags = uw_flags | (engine.FLAG_SHARD_EMBED if shard else 0)
 
     # ---------------------------------------------- value: inputs resident in HBM, one process per GPU
+    dump = OutputDump(args.dump_outputs, total_pairs, local_rank) if args.dump_outputs else None
     sampler = ClockSampler(local_rank)
     sampler.start()
-    dev_s, wall_s, launches, info = device_leg(h, ctx, tree, csr, weighted, flags, args.steps, args.warmup, sampler)
+    dev_s, wall_s, launches, info = device_leg(h, ctx, tree, csr, weighted, flags, args.steps, args.warmup, sampler, dump)
     value = total_pairs * args.steps / dev_s
+    if dump is not None:
+        dump.write(h)
 
     # ---------------------------------------------- sharded sub-record (N > 1): the exchange path per rank
     sharded = None
@@ -634,6 +701,7 @@ def run_ours(args, world, rank, local_rank):
 
 
 def main():
+    sys.dont_write_bytecode = True  # the tree may be read-only: leave no __pycache__ in it
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=200)
@@ -653,7 +721,13 @@ def main():
                     help="N>1: every rank rebuilds the whole embedding (no exchange) in the value leg")
     ap.add_argument("--uw-kernel", default="u8", choices=["u8", "bf16"],
                     help="operand encoding of the unweighted tensor-core kernel (FRC_FLAG_UW_BF16)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the distances of the value leg's last timed step to DIR (.npy, float32; at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
