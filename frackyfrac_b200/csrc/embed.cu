@@ -25,20 +25,26 @@ constexpr int kThreads = 256;
 // ---------------------------------------------------------------- fp64 path
 // One warp per sample: scatter its CSR row into the leaf rows.
 // Samples [s_base, s_end) go to columns [0, s_end - s_base) of E (a slab of the sample range).
+// K (may be null): the key panels of the keyed -l tiles (launch_embed_f64 in frc_internal.h): a present leaf's key is its id.
 __global__ void k_scatter_f64(const int64_t* __restrict__ row_ptr, const int32_t* __restrict__ col,
                               const double* __restrict__ val, int64_t s_base, int64_t s_end, double* E,
-                              int64_t ld) {
+                              int64_t ld, int32_t* __restrict__ K, int32_t kp) {
   int64_t s = s_base + ((static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5);
   int lane = threadIdx.x & 31;
   if (s >= s_end) return;
   int64_t b = row_ptr[s], e = row_ptr[s + 1];
-  for (int64_t k = b + lane; k < e; k += 32) E[static_cast<int64_t>(col[k]) * ld + (s - s_base)] = val[k];
+  for (int64_t k = b + lane; k < e; k += 32) {
+    E[static_cast<int64_t>(col[k]) * ld + (s - s_base)] = val[k];
+    if (K) K[((s >> 7) * kp + col[k]) * 128 + (s & 127)] = col[k];
+  }
 }
 
 // One tree level: E[v] = ((0 + E[c1]) + E[c2]) + ... in child order.
 // grid.x = nodes of the level, grid.y * blockDim.x * 2 covers the samples.
+// K (may be null): key[v] = max over the children's keys (-1 = absent): the largest present leaf id under v.
 __global__ void k_level_sum_f64(const int32_t* __restrict__ nodes, const int32_t* __restrict__ child_ptr,
-                                const int32_t* __restrict__ child_idx, double* E, int64_t ld) {
+                                const int32_t* __restrict__ child_idx, double* E, int64_t ld,
+                                int32_t* __restrict__ K, int32_t kp, int64_t s_base) {
   int32_t v = nodes[blockIdx.x];
   int64_t s = (static_cast<int64_t>(blockIdx.y) * blockDim.x + threadIdx.x) * 2;
   if (s >= ld) return;  // ld is even (multiple of 128)
@@ -50,6 +56,17 @@ __global__ void k_level_sum_f64(const int32_t* __restrict__ nodes, const int32_t
     acc.y = __dadd_rn(acc.y, x.y);
   }
   *reinterpret_cast<double2*>(E + static_cast<int64_t>(v) * ld + s) = acc;
+  if (K) {  // (s_base and s are even: the two samples sit side by side in one tile)
+    const int64_t g = s_base + s;
+    int32_t* const kt = K + (g >> 7) * kp * 128 + (g & 127);
+    int2 key = make_int2(-1, -1);
+    for (int32_t c = cb; c < ce; ++c) {
+      const int2 x = *reinterpret_cast<const int2*>(kt + static_cast<int64_t>(child_idx[c]) * 128);
+      key.x = max(key.x, x.x);
+      key.y = max(key.y, x.y);
+    }
+    *reinterpret_cast<int2*>(kt + static_cast<int64_t>(v) * 128) = key;
+  }
 }
 
 // total[s] = sum of E[v][s] over all v ascending (zeros add exactly nothing, so
@@ -626,21 +643,23 @@ __global__ void __launch_bounds__(1024) k_sum_flag_u(const double* __restrict__ 
 
 // ------------------------------------------------------------------ launchers
 int launch_embed_f64(const DevTree& t, const int32_t* level_ptr, const DevCsr& a, double* E,
-                     int64_t ld, int64_t s_base, cudaStream_t s) {
+                     int64_t ld, int64_t s_base, cudaStream_t s, int32_t* K, int32_t kp) {
   int launches = 0;
   cudaMemsetAsync(E, 0, sizeof(double) * ld * t.n_nodes, s);
+  // the slab's key panels are one contiguous range (s_base and ld are multiples of 128): all absent
+  if (K) cudaMemsetAsync(K + (s_base >> 7) * kp * 128, 0xFF, sizeof(int32_t) * ld * kp, s);
   const int64_t s_end = s_base + ld < a.n_samples ? s_base + ld : a.n_samples;
   if (s_end > s_base && a.nnz > 0) {
     int64_t threads = (s_end - s_base) * 32;
     k_scatter_f64<<<static_cast<unsigned>((threads + kThreads - 1) / kThreads), kThreads, 0, s>>>(
-        a.row_ptr, a.col, a.val, s_base, s_end, E, ld);
+        a.row_ptr, a.col, a.val, s_base, s_end, E, ld, K, kp);
     ++launches;
   }
   for (int32_t h = 1; h <= t.height; ++h) {
     int32_t b = level_ptr[h], e = level_ptr[h + 1];
     if (e == b) continue;
     dim3 grid(static_cast<unsigned>(e - b), static_cast<unsigned>((ld / 2 + kThreads - 1) / kThreads));
-    k_level_sum_f64<<<grid, kThreads, 0, s>>>(t.level_nodes + b, t.child_ptr, t.child_idx, E, ld);
+    k_level_sum_f64<<<grid, kThreads, 0, s>>>(t.level_nodes + b, t.child_ptr, t.child_idx, E, ld, K, kp, s_base);
     ++launches;
   }
   return launches;

@@ -59,8 +59,11 @@ struct Exceptions {
 // scattered from the CSR, then one pass per tree level, children summed in
 // child order starting from 0.0.  Returns launches.
 // E holds the ld samples starting at sample s_base (the whole table: s_base = 0, ld = np).
+// K (keyed -l tiles only, else null): also the int32 key panels of the same samples, in the tile-panel layout
+// K[np/128][kp][128] of the weighted operand (addressed by global sample tile): key = the largest present leaf
+// id in the node's subtree, -1 where the node is absent (E == 0) and in the padding rows [n_nodes, kp).
 int launch_embed_f64(const DevTree& t, const int32_t* level_ptr_host, const DevCsr& a, double* E,
-                     int64_t ld, int64_t s_base, cudaStream_t s);
+                     int64_t ld, int64_t s_base, cudaStream_t s, int32_t* K = nullptr, int32_t kp = 0);
 // total[s] = sum over ALL nodes in ascending id order (unifrac.go:60-63).
 int launch_totals_f64(const double* E, int32_t n_nodes, int64_t ld, int64_t n_samples,
                       double* total, cudaStream_t s);
@@ -163,7 +166,8 @@ int launch_exact_pairs(const double* E, const double* length, int32_t n_nodes, i
                        bool weighted, int64_t first, int64_t count, double* out, cudaStream_t s);
 // Flag -l AS CODED in the reference (normalize = 0): without normalizeFlatNodes the per-sample lists stay in
 // the order abundanceToFlatNodes appended them (post-order, unifrac.go:32-53) and unifracDistWeighted's
-// merge-join (:174-205) compares ids of lists that are not sorted.  Reproduced literally:
+// merge-join (:174-205) compares ids of lists that are not sorted.  Reproduced literally here; the fast form of
+// the same distances (FRC_FLAG_L_TILES) is the keyed variant of the weighted tiles (weighted.cu):
 //   launch_postorder_lists  per sample, the (id, raw subtree sum) entries with sum > 0 in post-order, from the
 //                           fp64 embedding E[B][ld] (two passes: count -> host prefix is avoided by a device
 //                           scan over samples; list_ptr has n_samples + 1 entries)
@@ -193,16 +197,19 @@ struct PanelMap {
 };
 // A is the tile-panel operand (see PanelMap; resident: Ap[np/128][kp][128]).
 // Pairs with d < flag_below are appended to flagged[] for the fix-up pass (as the unweighted kernel).
+// K non-null: normalize = 0 (-l as coded) on the keyed tiles: K are the resident key panels (launch_embed_f64) and
+// node v only counts as matched, |a - b|, where the two samples' keys agree; everywhere else a + b.
 int launch_weighted_tiles(const PanelMap& A, int64_t ld, int32_t kp, const float* lenf, bool prescaled,
                           const double* W, const Tile* tiles, int32_t n_tiles, int64_t n_samples,
                           int64_t first, float* out, double flag_below, uint32_t* flagged,
-                          unsigned long long* n_flagged, int num_sms, cudaStream_t s);
+                          unsigned long long* n_flagged, int num_sms, cudaStream_t s, const int32_t* K = nullptr);
 // fp64 / fixed-point recompute of the flagged pairs from the CSR rows (total: per-sample normaliser,
-// null for -l); ws = ws_ctas zeroed int64 arrays of n_nodes entries, left zeroed.
+// null for -l); ws = ws_ctas zeroed int64 arrays of n_nodes entries (2 * n_nodes with K), left zeroed.
+// K non-null: the keyed -l numerator, with the match decision read from the key panels K[np/128][kp][128].
 int launch_weighted_fixup(const DevCsr& a, const DevTree& t, const double* total, const double* W,
                           const uint32_t* flagged, const unsigned long long* n_flagged,
                           unsigned long long* count_host, int64_t first, long long* ws, int ws_ctas, float* out,
-                          const Exceptions& ex, cudaStream_t s);
+                          const Exceptions& ex, cudaStream_t s, const int32_t* K = nullptr, int32_t kp = 0);
 void weighted_setup();  // cudaFuncSetAttribute calls for the CURRENT device (once per device context)
 
 // ---- unweighted_tc.cu -------------------------------------------------------

@@ -201,7 +201,8 @@ struct Shared {
   int64_t N = 0, np = 0, nnz = 0;
   int32_t B = 0, kp = 0, nw = 0;
   bool exact = false, weighted = false, prescale = true, need_val = false;
-  bool unsorted_l = false;    // normalize == 0: the reference's -l as coded (post-order lists, exact.cu)
+  bool unsorted_l = false;    // normalize == 0 on the exact path: the reference's -l as coded (post-order lists, exact.cu)
+  bool keyed = false;         // normalize == 0 on the FP32 tiles (FRC_FLAG_L_TILES): key panels next to the values
   bool d2h = true;
   int n_parts = 1;
   int world = 1, rank0 = 0;   // band ownership: `world` owners; part p owns owner id rank0 + p
@@ -300,6 +301,7 @@ struct Part {
   float* d_lenf = nullptr;
   double *d_E = nullptr, *d_total = nullptr, *d_W = nullptr, *d_r = nullptr, *d_scratch = nullptr;
   float* d_A = nullptr;
+  int32_t* d_K = nullptr;     // keyed -l tiles: key panels, same layout as d_A (resident only)
   uint32_t *d_bits = nullptr, *d_node_scratch = nullptr;
   void *d_P = nullptr, *d_Bh = nullptr, *d_Bl = nullptr;
   TcOperands* tc = nullptr;
@@ -497,9 +499,11 @@ int embed_stage1(Part* p) {
       // panels are addressed by GLOBAL sample tile inside the kernel: shift the base so that the range's
       // first tile lands in its local slot (resident: slot == global tile, no shift)
       float* Ap = p->d_A + (rg.slot0 - s_begin / kTile) * static_cast<int64_t>(sh.kp) * kTile;
+      int32_t* Kp = sh.keyed ? p->d_K + (rg.slot0 - s_begin / kTile) * static_cast<int64_t>(sh.kp) * kTile : nullptr;
       for (int64_t sb = s_begin; sb < s_stop; sb += p->ws_slab) {
         const int64_t ld = std::min<int64_t>(p->ws_slab, s_stop - sb);
-        launches += launch_embed_f64(p->dtree, sh.level_ptr.data(), p->dcsr, p->d_E, ld, sb, s);
+        // (keyed: the key panels of the slab are built by the same scatter + level passes)
+        launches += launch_embed_f64(p->dtree, sh.level_ptr.data(), p->dcsr, p->d_E, ld, sb, s, Kp, sh.kp);
         if (norm) launches += launch_totals_fast_f64(p->d_E, sh.B, ld, p->d_total + sb, p->d_scratch, s);
         launches += launch_weighted_operand_panels(p->d_E, p->dtree.length, sh.B, sh.kp, ld, sb,
                                                    norm ? p->d_total + sb : nullptr, sh.prescale, Ap, p->d_W,
@@ -508,10 +512,15 @@ int embed_stage1(Part* p) {
       const size_t per = static_cast<size_t>(s_stop - s_begin);
       const size_t bytes[3] = {per * sh.kp * sizeof(float), per * sizeof(double), per * sizeof(double)};
       if (sh.exchange == Shared::kNccl) {
-        void* bufs[3] = {p->d_A, p->d_W, p->d_total};
+        // panels, denominators (+ normalisers, + key panels: as many bytes as the value panels)
+        void* bufs[4] = {p->d_A, p->d_W, nullptr, nullptr};
+        size_t bb[4] = {bytes[0], bytes[1], 0, 0};
+        int nb = 2;
+        if (norm) { bufs[nb] = p->d_total; bb[nb++] = bytes[2]; }
+        if (sh.keyed) { bufs[nb] = p->d_K; bb[nb++] = bytes[0]; }
         std::string cerr;
-        if (!comm_all_gather_inplace(c->comm, bufs, bytes, norm ? 3 : 2, s, &cerr)) return pfail(p, FRC_ERR_CUDA, cerr);
-        p->info.gather_bytes = static_cast<int64_t>(bytes[0] + bytes[1] + (norm ? bytes[2] : 0)) * (sh.world - 1);
+        if (!comm_all_gather_inplace(c->comm, bufs, bb, nb, s, &cerr)) return pfail(p, FRC_ERR_CUDA, cerr);
+        p->info.gather_bytes = static_cast<int64_t>(bb[0] + bb[1] + bb[2] + bb[3]) * (sh.world - 1);
       } else if (inproc) {
         // the shard's denominators and normalisers -- and, unless the panels stay sharded (capacity mode), the
         // panels themselves -- go to the same place in every other device's HBM: device-to-device copies over
@@ -521,11 +530,14 @@ int embed_stage1(Part* p) {
           Part* o = p->job->parts[q].get();
           if (!sh.capacity)
             PART_CUDA(p, cudaMemcpyPeerAsync(o->d_A + s_begin * sh.kp, o->dc->device, p->d_A + s_begin * sh.kp, dc->device, bytes[0], s));
+          if (sh.keyed)
+            PART_CUDA(p, cudaMemcpyPeerAsync(o->d_K + s_begin * sh.kp, o->dc->device, p->d_K + s_begin * sh.kp, dc->device, bytes[0], s));
           PART_CUDA(p, cudaMemcpyPeerAsync(o->d_W + s_begin, o->dc->device, p->d_W + s_begin, dc->device, bytes[1], s));
           if (norm)
             PART_CUDA(p, cudaMemcpyPeerAsync(o->d_total + s_begin, o->dc->device, p->d_total + s_begin, dc->device, bytes[2], s));
         }
-        p->info.gather_bytes += static_cast<int64_t>((sh.capacity ? 0 : bytes[0]) + bytes[1] + (norm ? bytes[2] : 0)) * (n_parts - 1);
+        p->info.gather_bytes += static_cast<int64_t>((sh.capacity ? 0 : bytes[0]) + bytes[1] + (norm ? bytes[2] : 0) +
+                                                     (sh.keyed ? bytes[0] : 0)) * (n_parts - 1);
       }
     }
     p->pm = PanelMap{};
@@ -538,8 +550,8 @@ int embed_stage1(Part* p) {
     } else {
       p->pm.shard[0] = p->d_A;
     }
-    // write each element once, read it once when folded into its parent (+ CSR)
-    p->info.embed_bytes = 2LL * sh.B * built * 8 + 12LL * (p->csr_k1 - p->csr_k0);
+    // write each element once, read it once when folded into its parent (+ CSR; keyed: + the int32 keys)
+    p->info.embed_bytes = 2LL * sh.B * built * (sh.keyed ? 12 : 8) + 12LL * (p->csr_k1 - p->csr_k0);
   } else if (sh.fused_embed) {
     const int cur = static_cast<int>(p->run_count & 1);
     if (p->peer_push) {
@@ -721,12 +733,13 @@ int enqueue_band(Part* p, size_t idx) {
     *sl.ex.count = 0;  // (the slot's previous band has been delivered)
     if (sh.weighted) {
       launches += launch_weighted_tiles(p->pm, sh.np, sh.kp, p->d_lenf, sh.prescale, p->d_W, p->d_tiles + b.tile_off,
-                                        b.n_tiles, sh.N, b.first, sl.dev32, kFlagBelowW, sl.flagged, cnt, dc->num_sms, s);
+                                        b.n_tiles, sh.N, b.first, sl.dev32, kFlagBelowW, sl.flagged, cnt, dc->num_sms, s,
+                                        p->d_K);
       PART_CUDA(p, cudaEventRecord(sl.k1, s));
       // (one workspace per compute stream: consecutive bands run their fix-ups concurrently)
       launches += launch_weighted_fixup(p->dcsr, p->dtree, sh.opts.normalize == 1 ? p->d_total : nullptr, p->d_W,
                                         sl.flagged, cnt, sl.n_flagged_host, b.first, p->d_fix_ws[si], kFixupCtas,
-                                        sl.dev32, sl.ex, s);
+                                        sl.dev32, sl.ex, s, p->d_K, sh.kp);
     } else if (sh.bits_feed) {
       launches += launch_unweighted_bits(p->bo, p->d_tiles + b.tile_off, b.n_tiles, sh.N, b.first, sl.dev32,
                                          sl.flagged, cnt, dc->num_sms, s);
@@ -1077,9 +1090,13 @@ int validate_header(frc_job* j, const frc_tree_t* tree, const frc_csr_t* abnd, c
   if (opts->normalize < 0 || opts->normalize > 2) return fail(j, FRC_ERR_ARG, "bad normalize");
   if (opts->normalize != 1 && opts->mode != FRC_WEIGHTED)  // frcfrc.go:84-86
     return fail(j, FRC_ERR_ARG, "-l can only be used with weighted unifrac");
-  if (opts->normalize == 0 && opts->path == FRC_PATH_FAST)
+  // normalize = 0 runs the exact list walk unless the caller accepts the key-matched tiles (within 1e-5 instead of
+  // bit-exact); the flag means nothing for the other modes
+  const bool l_tiles = opts->normalize == 0 && (opts->flags & FRC_FLAG_L_TILES) != 0;
+  if (opts->normalize == 0 && opts->path == FRC_PATH_FAST && !l_tiles)
     return fail(j, FRC_ERR_UNSUPPORTED, "normalize = 0 (flag -l as coded in the reference: unsorted merge-join) only "
-                                        "exists on the exact path; normalize = 2 is the documented -l");
+                                        "exists on the exact path unless FRC_FLAG_L_TILES selects the key-matched FP32 "
+                                        "tiles; normalize = 2 is the documented -l");
   const int world = opts->world <= 0 ? 1 : opts->world;
   const int rank = opts->world <= 0 ? 0 : opts->rank;
   if (rank < 0 || rank >= world) return fail(j, FRC_ERR_ARG, "rank outside [0, world)");
@@ -1104,10 +1121,11 @@ int validate_header(frc_job* j, const frc_tree_t* tree, const frc_csr_t* abnd, c
   sh.world = world; sh.rank0 = rank;
   sh.d2h = !(opts->flags & FRC_FLAG_NO_D2H);
   const int64_t n_pairs = N >= 2 ? tri(N) : 0;
-  sh.unsorted_l = opts->normalize == 0;
-  if (opts->path == FRC_PATH_EXACT || sh.unsorted_l) sh.exact = true;
+  if (opts->path == FRC_PATH_EXACT || (opts->normalize == 0 && !l_tiles)) sh.exact = true;
   else if (opts->path == FRC_PATH_FAST) sh.exact = false;
   else sh.exact = n_pairs == 0 || (static_cast<double>(n_pairs) * B <= static_cast<double>(kExactWorkLimit));
+  sh.unsorted_l = opts->normalize == 0 && sh.exact;
+  sh.keyed = opts->normalize == 0 && !sh.exact;
   sh.need_val = sh.exact || sh.weighted;
   return FRC_OK;
 }
@@ -1158,7 +1176,8 @@ int plan_job(frc_job* j, const frc_tree_t* tree, bool neg_len) {
   if (sh.exchange == Shared::kInProcess && sh.weighted && sh.knobs.capacity != 0 && sh.N >= 2) {
     bool want = sh.knobs.capacity == 1;
     if (!want) {
-      const double panels = 4.0 * static_cast<double>(round_up(sh.B, kKBlock)) * static_cast<double>(round_up(sh.N, kTile * 2LL * n_parts));
+      // (keyed -l tiles: an int32 key next to every fp32 value)
+      const double panels = (sh.keyed ? 8.0 : 4.0) * static_cast<double>(round_up(sh.B, kKBlock)) * static_cast<double>(round_up(sh.N, kTile * 2LL * n_parts));
       if (panels > 24.0 * (1 << 30)) {  // (cudaMemGetInfo costs milliseconds: only asked when it can matter)
         size_t free_b = 0, total_b = 0;
         cudaSetDevice(c->devs[0]->device);
@@ -1166,6 +1185,11 @@ int plan_job(frc_job* j, const frc_tree_t* tree, bool neg_len) {
         cudaGetLastError();
       }
     }
+    if (want && sh.keyed)
+      return fail(j, FRC_ERR_UNSUPPORTED, "the key-matched tiles of -l as coded (FRC_FLAG_L_TILES) keep the value and key "
+                                          "panels of all samples on every device; the capacity mode, which shards them "
+                                          "over the devices when they exceed about half of one device's free HBM (or with "
+                                          "FRC_CAPACITY=1), does not carry keys");
     sh.capacity = want;
     if (want) shards = 2 * n_parts;
   }
@@ -1361,6 +1385,7 @@ int prepare_part(Part* p) {
       // resident: the panels of all samples; capacity: of this device's two shards only
       const size_t a_samples = sh.capacity ? static_cast<size_t>(2 * sh.shard_rows) : static_cast<size_t>(sh.np);
       if (!(p->d_A = dev_alloc<float>(p, static_cast<size_t>(sh.kp) * a_samples))) return p->rc;
+      if (sh.keyed && !(p->d_K = dev_alloc<int32_t>(p, static_cast<size_t>(sh.kp) * a_samples))) return p->rc;
       if (sh.capacity) {
         for (int k = 0; k < 2; ++k)
           if (!(p->d_V[k] = dev_alloc<float>(p, static_cast<size_t>(sh.kp) * sh.shard_rows))) return p->rc;
@@ -1391,7 +1416,7 @@ int prepare_part(Part* p) {
       if (!(p->d_W = dev_alloc<double>(p, sh.np))) return p->rc;
       if (!(p->d_scratch = dev_alloc<double>(p, static_cast<size_t>(chunks) * sh.np))) return p->rc;
       if (!(p->d_flag_counts = dev_alloc<unsigned long long>(p, p->mine.size() + 1))) return p->rc;
-      const size_t ws_words = static_cast<size_t>(kFixupCtas) * B;
+      const size_t ws_words = static_cast<size_t>(kFixupCtas) * B * (sh.keyed ? 2 : 1);  // (keyed: diff + sum)
       for (int k = 0; k < 2; ++k) {
         if (!(p->d_fix_ws[k] = dev_alloc<long long>(p, ws_words))) return p->rc;
         PART_CUDA(p, cudaMemsetAsync(p->d_fix_ws[k], 0, sizeof(long long) * ws_words, s0));

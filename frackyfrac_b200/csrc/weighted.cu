@@ -18,6 +18,16 @@
 // with a 6-deep ring of TMA bulk copies (one 16 KB copy per operand slab).  Accumulation is two-level (flush the 64
 // running sums into 64 totals every 256 nodes) to keep fp32 summation error
 // well under the 1e-5 budget for contractions of 10^5..10^6 nodes.
+//
+// Keyed variant (normalize = 0, flag -l as the reference codes it, FRC_FLAG_L_TILES).  Without the id-sort the
+// reference's merge-join walks post-order lists and pairs nodes up by accident; the outcome has a closed form
+// (DESIGN.md, "-l as coded"): with key_s(v) = the largest present leaf id under v (-1 when v is absent),
+//   numer = sum_v len_v * (key_i(v) == key_j(v) ? |a - b| : a + b),   denom = W_i + W_j.
+// Since |a - b| = a + b - 2 min(a, b) for a, b >= 0, the kernel accumulates S = sum over matched v of
+// len_v * min(a, b) -- ISETP + FMNMX + predicated FADD (FFMA), 3 instructions per (pair, node) against the 2 of
+// the L1 loop -- and forms numer = W_i + W_j - 2 S in fp64.  The int32 key panels K[np/128][kp][128] ride in the
+// same TMA ring as the values, which doubles a stage to 64 KB: the ring is 3 stages deep (192 KB; 6 would need
+// 384 KB).  Keyed panels are always resident in local HBM (no capacity mode), where 2 slabs in flight suffice.
 #include "frc_internal.h"
 #include "ptx.cuh"
 #include "wire.cuh"
@@ -26,11 +36,14 @@ namespace frc {
 namespace {
 
 constexpr int KT = 32;        // nodes per smem slab
-constexpr int STAGES = 6;     // ring depth: 5 slabs (160 KB) in flight per CTA, enough to cover NVLink latency in capacity mode
 constexpr int FLUSH = 8;      // slabs between flushes (256 nodes)
 constexpr int SLAB_FLOATS = KT * kTile;             // one operand side: 16 KB
-constexpr int STAGE_FLOATS = 2 * SLAB_FLOATS + KT;  // + per-node lengths (128 B)
-constexpr int SMEM_BYTES = STAGES * STAGE_FLOATS * 4 + STAGES * 8 + 128;
+// ring depth: 5 slabs (160 KB) in flight per CTA, enough to cover NVLink latency in capacity mode; keyed: 3
+// stages of values + keys (64 KB each)
+template <bool kKeyed> constexpr int kStages = kKeyed ? 3 : 6;
+// per stage: the two value slabs, per-node lengths (128 B), keyed: the two key slabs
+template <bool kKeyed> constexpr int kStageFloats = (kKeyed ? 4 : 2) * SLAB_FLOATS + KT;
+template <bool kKeyed> constexpr int kSmemBytes = kStages<kKeyed> * kStageFloats<kKeyed> * 4 + kStages<kKeyed> * 8 + 128;
 
 // Panel of sample tile t (PanelMap in frc_internal.h): the one local array, or the place its shard currently
 // occupies in this device's HBM.
@@ -43,12 +56,14 @@ __device__ __forceinline__ const float* panel_of(const PanelMap& m, int32_t t, i
 // Operand staging: one thread issues TMA bulk copies (cp.async.bulk, 16 KB per operand slab: the tile-panel
 // layout makes a slab of 32 nodes x 128 samples contiguous) that complete on an mbarrier per stage.  The
 // FP32-issue-bound inner loop spends no slot on copies and the copy engine keeps the whole ring in flight.
-template <bool kPrescaled>
+template <bool kPrescaled, bool kKeyed>
 __global__ void __launch_bounds__(256, 1)
 k_weighted_tiles(const PanelMap A, int64_t ld, int32_t kp, const float* __restrict__ lenf,
                  const double* __restrict__ W, const Tile* __restrict__ tiles, int64_t n_samples,
                  int64_t first, float* __restrict__ out, double flag_below, uint32_t* __restrict__ flagged,
-                 unsigned long long* __restrict__ n_flagged) {
+                 unsigned long long* __restrict__ n_flagged, const int32_t* __restrict__ K) {
+  constexpr int STAGES = kStages<kKeyed>;
+  constexpr int STAGE_FLOATS = kStageFloats<kKeyed>;
   extern __shared__ __align__(128) float smem[];
   const Tile tile = tiles[blockIdx.x];
   const int64_t i0 = static_cast<int64_t>(tile.ti) * kTile;
@@ -62,15 +77,23 @@ k_weighted_tiles(const PanelMap A, int64_t ld, int32_t kp, const float* __restri
   // tile-panel layout [kp][128] per sample tile
   const float* const pa = panel_of(A, tile.ti, kp);  // row samples: this device's own shard
   const float* const pb = panel_of(A, tile.tj, kp);  // column samples: own shard or the visiting one
+  // keyed: the key panels of the same tiles (resident only: global tile index)
+  const int32_t* const ka_g = kKeyed ? K + static_cast<int64_t>(tile.ti) * kp * kTile : nullptr;
+  const int32_t* const kb_g = kKeyed ? K + static_cast<int64_t>(tile.tj) * kp * kTile : nullptr;
   auto issue = [&](int slab) {  // thread 0 only
     const int stage = slab % STAGES;
     float* sa = smem + stage * STAGE_FLOATS;
     const uint32_t bar = bar0 + 8u * stage;
     constexpr uint32_t kSlabBytes = SLAB_FLOATS * 4;
-    ptx::mbar_expect_tx(bar, 2 * kSlabBytes + (kPrescaled ? 0u : KT * 4u));
+    ptx::mbar_expect_tx(bar, (kKeyed ? 4 : 2) * kSlabBytes + (kPrescaled ? 0u : KT * 4u));
     ptx::bulk_load_1d(ptx::smem_u32(sa), pa + static_cast<int64_t>(slab) * SLAB_FLOATS, kSlabBytes, bar);
     ptx::bulk_load_1d(ptx::smem_u32(sa + SLAB_FLOATS), pb + static_cast<int64_t>(slab) * SLAB_FLOATS, kSlabBytes, bar);
     if (!kPrescaled) ptx::bulk_load_1d(ptx::smem_u32(sa + 2 * SLAB_FLOATS), lenf + slab * KT, KT * 4u, bar);
+    if (kKeyed) {
+      float* sk = sa + 2 * SLAB_FLOATS + KT;
+      ptx::bulk_load_1d(ptx::smem_u32(sk), ka_g + static_cast<int64_t>(slab) * SLAB_FLOATS, kSlabBytes, bar);
+      ptx::bulk_load_1d(ptx::smem_u32(sk + SLAB_FLOATS), kb_g + static_cast<int64_t>(slab) * SLAB_FLOATS, kSlabBytes, bar);
+    }
   };
   if (tid == 0) {
     for (int s = 0; s < STAGES; ++s) ptx::mbar_init(bar0 + 8u * s, 1);
@@ -94,6 +117,8 @@ k_weighted_tiles(const PanelMap A, int64_t ld, int32_t kp, const float* __restri
     const float* sa = smem + stage * STAGE_FLOATS;
     const float* sb = sa + SLAB_FLOATS;
     const float* sl = sb + SLAB_FLOATS;
+    const int32_t* ska = reinterpret_cast<const int32_t*>(sl + KT);
+    const int32_t* skb = ska + SLAB_FLOATS;
 #pragma unroll 4
     for (int kk = 0; kk < KT; ++kk) {
       const float4 a0 = *reinterpret_cast<const float4*>(sa + kk * kTile + ty * 4);
@@ -102,7 +127,23 @@ k_weighted_tiles(const PanelMap A, int64_t ld, int32_t kp, const float* __restri
       const float4 b1 = *reinterpret_cast<const float4*>(sb + kk * kTile + 64 + tx * 4);
       const float av[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
       const float bv[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
-      if (kPrescaled) {
+      if (kKeyed) {
+        const int4 p0 = *reinterpret_cast<const int4*>(ska + kk * kTile + ty * 4);
+        const int4 p1 = *reinterpret_cast<const int4*>(ska + kk * kTile + 64 + ty * 4);
+        const int4 q0 = *reinterpret_cast<const int4*>(skb + kk * kTile + tx * 4);
+        const int4 q1 = *reinterpret_cast<const int4*>(skb + kk * kTile + 64 + tx * 4);
+        const int32_t ka[8] = {p0.x, p0.y, p0.z, p0.w, p1.x, p1.y, p1.z, p1.w};
+        const int32_t kb[8] = {q0.x, q0.y, q0.z, q0.w, q1.x, q1.y, q1.z, q1.w};
+        const float l = kPrescaled ? 1.f : sl[kk];
+#pragma unroll
+        for (int a = 0; a < 8; ++a)
+#pragma unroll
+          for (int b = 0; b < 8; ++b)
+            if (ka[a] == kb[b]) {
+              if (kPrescaled) acc[a][b] += fminf(av[a], bv[b]);
+              else acc[a][b] = fmaf(l, fminf(av[a], bv[b]), acc[a][b]);
+            }
+      } else if (kPrescaled) {
 #pragma unroll
         for (int a = 0; a < 8; ++a)
 #pragma unroll
@@ -134,7 +175,10 @@ k_weighted_tiles(const PanelMap A, int64_t ld, int32_t kp, const float* __restri
     for (int b = 0; b < 8; ++b) {
       const int64_t j = j0 + (b < 4 ? tx * 4 + b : 64 + tx * 4 + (b - 4));
       if (j < i) {
-        const double d = static_cast<double>(tot[a][b] + acc[a][b]) / (wi + W[j]);
+        // keyed: the accumulator holds S = sum over matched nodes of len * min(a, b)
+        const double num = kKeyed ? (wi + W[j]) - 2.0 * static_cast<double>(tot[a][b] + acc[a][b])
+                                  : static_cast<double>(tot[a][b] + acc[a][b]);
+        const double d = num / (wi + W[j]);
         orow[j] = static_cast<float>(d);  // fp32 numerator: fp32 is what the value carries (wire.cu)
         // fp32 operands carry 6e-8 relative error each, so the L1 numerator is off by up to
         // 6e-8 * (W_i + W_j) = 6e-8 / d relative: small distances are recomputed (k_weighted_fixup)
@@ -153,17 +197,22 @@ k_weighted_tiles(const PanelMap A, int64_t ld, int32_t kp, const float* __restri
 //   cancel to exactly 0), then numerator = sum_v len_v * |diff[v]| in fp64 over the touched nodes (the
 //   second walk takes each node's value with an atomic exchange, which also restores the zeros).
 // ws is one zeroed int64 array of n_nodes entries per CTA.
+// Keyed (-l as coded): a second array per CTA accumulates sum[v] = a_i(v) + a_j(v) the same way, and a touched
+// node adds len * |diff| where the key panels say the two samples match at v, len * sum where they do not.
+template <bool kKeyed>
 __global__ void __launch_bounds__(256)
 k_weighted_fixup(const int64_t* __restrict__ row_ptr, const int32_t* __restrict__ col,
                  const double* __restrict__ val, const int32_t* __restrict__ parent,
                  const double* __restrict__ length, int32_t n_nodes, const double* __restrict__ total,
                  const double* __restrict__ W, const uint32_t* __restrict__ flagged,
                  const unsigned long long* __restrict__ n_flagged, unsigned long long* __restrict__ count_host,
-                 int64_t first, long long* __restrict__ ws, float* __restrict__ out, const Exceptions ex) {
+                 int64_t first, long long* __restrict__ ws, float* __restrict__ out, const Exceptions ex,
+                 const int32_t* __restrict__ K, int32_t kp) {
   __shared__ double red[8];
   const unsigned long long n = *n_flagged;
   if (blockIdx.x == 0 && threadIdx.x == 0) *count_host = n;  // mapped pinned memory
-  long long* diff = ws + static_cast<int64_t>(blockIdx.x) * n_nodes;
+  long long* diff = ws + static_cast<int64_t>(blockIdx.x) * n_nodes * (kKeyed ? 2 : 1);
+  long long* sum = diff + n_nodes;  // (keyed only)
   constexpr double kFix = 1152921504606846976.0;  // 2^60: proportions are <= 1, a node sums <= 1
   for (unsigned long long w = blockIdx.x; w < n; w += gridDim.x) {
     const uint32_t off = flagged[w];
@@ -196,11 +245,15 @@ k_weighted_fixup(const int64_t* __restrict__ row_ptr, const int32_t* __restrict_
       for (int64_t k = b + threadIdx.x; k < e; k += blockDim.x) {
         const long long x = __double2ll_rn(val[k] * inv[side] * kFix);
         const long long add = side == 0 ? x : -x;
-        for (int32_t v = col[k]; v >= 0; v = parent[v])
+        for (int32_t v = col[k]; v >= 0; v = parent[v]) {
           atomicAdd(reinterpret_cast<unsigned long long*>(diff + v), static_cast<unsigned long long>(add));
+          if (kKeyed) atomicAdd(reinterpret_cast<unsigned long long*>(sum + v), static_cast<unsigned long long>(x));
+        }
       }
     }
     __syncthreads();
+    const int32_t* const ki = kKeyed ? K + (i >> 7) * kp * 128 + (i & 127) : nullptr;
+    const int32_t* const kj = kKeyed ? K + (j >> 7) * kp * 128 + (j & 127) : nullptr;
     double num = 0.0;
 #pragma unroll
     for (int side = 0; side < 2; ++side) {
@@ -208,7 +261,14 @@ k_weighted_fixup(const int64_t* __restrict__ row_ptr, const int32_t* __restrict_
       for (int64_t k = b + threadIdx.x; k < e; k += blockDim.x)
         for (int32_t v = col[k]; v >= 0; v = parent[v]) {
           const long long x = static_cast<long long>(atomicExch(reinterpret_cast<unsigned long long*>(diff + v), 0ULL));
-          if (x != 0) num += length[v] * (fabs(static_cast<double>(x)) * unscale);
+          if (kKeyed) {
+            // (whichever thread takes a node's value adds its term: only one of the two arrays counts per node)
+            const long long y = static_cast<long long>(atomicExch(reinterpret_cast<unsigned long long*>(sum + v), 0ULL));
+            const long long t = ki[static_cast<int64_t>(v) * 128] == kj[static_cast<int64_t>(v) * 128] ? (x < 0 ? -x : x) : y;
+            if (t != 0) num += length[v] * (static_cast<double>(t) * unscale);
+          } else if (x != 0) {
+            num += length[v] * (fabs(static_cast<double>(x)) * unscale);
+          }
         }
     }
 #pragma unroll
@@ -229,29 +289,39 @@ k_weighted_fixup(const int64_t* __restrict__ row_ptr, const int32_t* __restrict_
 int launch_weighted_fixup(const DevCsr& a, const DevTree& t, const double* total, const double* W,
                           const uint32_t* flagged, const unsigned long long* n_flagged,
                           unsigned long long* count_host, int64_t first, long long* ws, int ws_ctas, float* out,
-                          const Exceptions& ex, cudaStream_t s) {
-  k_weighted_fixup<<<ws_ctas, 256, 0, s>>>(a.row_ptr, a.col, a.val, t.parent, t.length, t.n_nodes, total, W, flagged,
-                                           n_flagged, count_host, first, ws, out, ex);
+                          const Exceptions& ex, cudaStream_t s, const int32_t* K, int32_t kp) {
+  if (K)
+    k_weighted_fixup<true><<<ws_ctas, 256, 0, s>>>(a.row_ptr, a.col, a.val, t.parent, t.length, t.n_nodes, total, W,
+                                                   flagged, n_flagged, count_host, first, ws, out, ex, K, kp);
+  else
+    k_weighted_fixup<false><<<ws_ctas, 256, 0, s>>>(a.row_ptr, a.col, a.val, t.parent, t.length, t.n_nodes, total, W,
+                                                    flagged, n_flagged, count_host, first, ws, out, ex, nullptr, 0);
   return 1;
 }
 
 void weighted_setup() {
-  cudaFuncSetAttribute(k_weighted_tiles<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-  cudaFuncSetAttribute(k_weighted_tiles<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
+  cudaFuncSetAttribute(k_weighted_tiles<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes<false>);
+  cudaFuncSetAttribute(k_weighted_tiles<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes<false>);
+  cudaFuncSetAttribute(k_weighted_tiles<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes<true>);
+  cudaFuncSetAttribute(k_weighted_tiles<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes<true>);
 }
 
 int launch_weighted_tiles(const PanelMap& A, int64_t ld, int32_t kp, const float* lenf, bool prescaled,
                           const double* W, const Tile* tiles, int32_t n_tiles, int64_t n_samples,
                           int64_t first, float* out, double flag_below, uint32_t* flagged,
-                          unsigned long long* n_flagged, int num_sms, cudaStream_t s) {
+                          unsigned long long* n_flagged, int num_sms, cudaStream_t s, const int32_t* K) {
   (void)num_sms;
   if (n_tiles <= 0) return 0;
-  if (prescaled)
-    k_weighted_tiles<true><<<n_tiles, 256, SMEM_BYTES, s>>>(A, ld, kp, lenf, W, tiles, n_samples, first, out,
-                                                            flag_below, flagged, n_flagged);
-  else
-    k_weighted_tiles<false><<<n_tiles, 256, SMEM_BYTES, s>>>(A, ld, kp, lenf, W, tiles, n_samples, first, out,
-                                                             flag_below, flagged, n_flagged);
+  auto go = [&](auto kernel, int smem) {
+    kernel<<<n_tiles, 256, smem, s>>>(A, ld, kp, lenf, W, tiles, n_samples, first, out, flag_below, flagged, n_flagged, K);
+  };
+  if (K) {
+    if (prescaled) go(k_weighted_tiles<true, true>, kSmemBytes<true>);
+    else go(k_weighted_tiles<false, true>, kSmemBytes<true>);
+  } else {
+    if (prescaled) go(k_weighted_tiles<true, false>, kSmemBytes<false>);
+    else go(k_weighted_tiles<false, false>, kSmemBytes<false>);
+  }
   return 1;
 }
 

@@ -23,6 +23,7 @@ FLAG_NO_D2H = 1
 FLAG_UW_BF16 = 2
 FLAG_SHARD_EMBED = 4
 FLAG_UW_BITS = 8
+FLAG_L_TILES = 16  # normalize=0 (-l as coded) may run the key-matched FP32 tiles (within 1e-5, not bit-exact)
 COMM_ID_BYTES = 128
 
 NORM_L_AS_CODED, NORM_DEFAULT, NORM_L_DOCUMENTED = 0, 1, 2  # frc_opts_t.normalize
@@ -189,8 +190,9 @@ class Job:
     def __init__(self, parent, length, row_ptr, col, val, *, weighted: bool, normalize=True,
                  path: int = PATH_AUTO, ctx: Context | None = None, device: int = -1, rank: int = 0,
                  world: int = 1, band_rows: int = 0, flags: int = 0, devices=None):
-        """normalize: True / 1 = default; False / 0 = flag -l as CODED in the reference (unsorted merge-join,
-        exact path only); 2 = flag -l as documented.  devices: None = one GPU (`device` or the context's);
+        """normalize: True / 1 = default; False / 0 = flag -l as CODED in the reference (unsorted merge-join:
+        the bit-exact list walk, or with flags=FLAG_L_TILES the key-matched FP32 tiles wherever `path` picks the
+        fast kernels); 2 = flag -l as documented.  devices: None = one GPU (`device` or the context's);
         a list of ordinals or -1 (all) = this process drives several GPUs, one ordered stream."""
         self._keep = [np.ascontiguousarray(parent, np.int32), np.ascontiguousarray(length, np.float64),
                       np.ascontiguousarray(row_ptr, np.int64), np.ascontiguousarray(col, np.int32),

@@ -136,6 +136,9 @@ int main(int argc, char** argv) {
       if (const char* e = getenv("FRCFRC_L")) fo.normalize = !strcmp(e, "documented") ? 2 : 0;
     fo.path = FRC_PATH_AUTO;
     if (const char* e = getenv("FRCFRC_PATH")) fo.path = !strcmp(e, "exact") ? FRC_PATH_EXACT : !strcmp(e, "fast") ? FRC_PATH_FAST : FRC_PATH_AUTO;
+    // -l as coded with FRCFRC_PATH=fast: the key-matched FP32 tiles (within 1e-5 of the reference, not bit-exact);
+    // without FRCFRC_PATH, -l runs the bit-exact list walk
+    if (fo.normalize == 0 && fo.path == FRC_PATH_FAST) fo.flags |= FRC_FLAG_L_TILES;
     fo.device = -1;
     fo.world = 1;
     // every visible B200 works on the job; the engine hands their bands out as ONE ordered stream

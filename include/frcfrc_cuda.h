@@ -105,6 +105,18 @@ typedef struct {
                               the pair kernel from the presence bits instead of materialising
                               them in HBM (3 bytes per (sample, node) saved; info.operand_kind 3) */
 
+#define FRC_FLAG_L_TILES 16u /* normalize == 0 (-l as coded): allow the FP32 tile kernel instead of the
+                               exact list walk.  The walk's mis-pairing has a closed form: node v is
+                               matched iff both samples hold it and the largest present leaf id under v
+                               is the same for both (DESIGN.md); the tiles carry that key per (node,
+                               sample) next to the values.  Within 1e-5 relative of the reference
+                               instead of bit-exact.  path FAST: always the tiles; AUTO: exact for small
+                               inputs (the AUTO rule of every mode), tiles above.  Without the flag
+                               normalize == 0 always runs the exact walk and FAST is refused.  Ignored
+                               for normalize 1 and 2.  One process over several GPUs and
+                               FRC_FLAG_SHARD_EMBED are supported; the capacity mode (panels sharded
+                               over devices) is not: FRC_ERR_UNSUPPORTED where it would be chosen.  */
+
 typedef struct {
   int32_t mode;       /* frc_mode                                               */
   int32_t normalize;  /* flag -l (frcfrc.go:25):
@@ -112,7 +124,8 @@ typedef struct {
                          0 = -l AS CODED in the reference: normalizeFlatNodes is skipped
                              (unifrac.go:108-110) and with it the id-sort (:57), so the
                              merge-join (:178-203) walks POST-ORDER lists and mis-pairs nodes;
-                             reproduced bit for bit by a dedicated kernel (csrc/exact.cu)
+                             reproduced bit for bit by a dedicated kernel (csrc/exact.cu), or
+                             within 1e-5 by the key-matched FP32 tiles (FRC_FLAG_L_TILES)
                          2 = -l as documented: id-sorted lists, raw values
                          0 and 2 need mode == FRC_WEIGHTED (frcfrc.go:84-86)            */
   int32_t path;       /* frc_path                                               */
