@@ -209,7 +209,7 @@ struct Shared {
   enum Exchange { kNone, kInProcess, kNccl } exchange = kNone;  // how the sample shards of the embedding meet
   bool fused_embed = true, bits_feed = false;
   bool capacity = false;      // fast weighted over several devices: panels stay sharded (PanelMap), tiles read peers' HBM
-  int64_t shard_rows = 0;     // capacity: samples per shard (np / 2G)
+  ShardPlan shards;           // which samples each owner builds (np = shards.np)
   ColumnPlan cols;
   std::vector<Band> bands;   // whole triangle (owners filled in)
   std::vector<int32_t> level_ptr;
@@ -245,12 +245,9 @@ struct Part {
   std::vector<Band> bands;  // copies of the bands in `mine` with this part's tile offsets
   std::vector<Tile> tiles;
 
-  // sample shard of the embedding this part builds (word columns of 32 samples; everything unless sharded)
+  // first sample shard of the embedding this part builds (word columns of 32 samples; everything unless sharded)
   int32_t shard_w0 = 0, shard_nw = 0;
   int64_t csr_k0 = 0, csr_k1 = 0;  // CSR entries this part uploads
-  // fast weighted: the sample ranges whose panels this part builds, and where their first tile sits in d_A
-  struct Range { int64_t s0, s1, slot0; };
-  std::vector<Range> ranges;
   PanelMap pm;
   // capacity mode: the rows of each of this part's (two) shards form one GROUP with one output buffer for the whole
   // pass (the column shards visit one at a time, so all rows advance together) and ONE launch per visiting shard:
@@ -449,6 +446,48 @@ int sym_sync(Part* p, bool* usable) {
 }
 
 // ------------------------------------------------------------------ embedding
+// A per-sample array of the embedding that every part reads for ALL samples, at the same sample offsets everywhere.
+struct ShardArray {
+  void* (*on)(const Part*);  // the array on a part
+  size_t sample_bytes;
+  bool copy = true;  // false: the producing kernel stored the shard into every part itself (counted, not copied)
+};
+template <auto M> void* part_array(const Part* q) { return q->*M; }
+
+// Makes the samples [rg.s0, rg.s1) of every array in `arrs`, built by this part, visible to the other parts (stream s)
+// and adds the bytes that reach them to info.gather_bytes.  kNccl: one in-place all-gather group (rank r's slice is the
+// r-th: the sharded plan puts shard r there), a barrier when nothing is copied; kInProcess: copies over NVLink.
+int exchange_shard(Part* p, const std::vector<ShardArray>& arrs, const Range& rg, cudaStream_t s) {
+  const Shared& sh = *p->sh;
+  if (sh.exchange == Shared::kNone) return FRC_OK;
+  const size_t n = static_cast<size_t>(rg.s1 - rg.s0);
+  const int others = (sh.exchange == Shared::kNccl ? sh.world : sh.n_parts) - 1;
+  std::vector<void*> bufs;
+  std::vector<size_t> bytes;
+  for (const ShardArray& a : arrs) {
+    p->info.gather_bytes += static_cast<int64_t>(n * a.sample_bytes) * others;
+    if (a.copy) { bufs.push_back(a.on(p)); bytes.push_back(n * a.sample_bytes); }
+  }
+  if (sh.exchange == Shared::kNccl) {
+    Comm* comm = p->job->ctx->comm;
+    std::string cerr;
+    const bool ok = bufs.empty() ? comm_barrier(comm, s, &cerr)
+                                 : comm_all_gather_inplace(comm, bufs.data(), bytes.data(), static_cast<int>(bufs.size()), s, &cerr);
+    return ok ? FRC_OK : pfail(p, FRC_ERR_CUDA, cerr);
+  }
+  for (int q = 0; q < sh.n_parts; ++q) {
+    if (q == p->index) continue;
+    const Part* o = p->job->parts[q].get();
+    for (const ShardArray& a : arrs) {
+      if (!a.copy) continue;
+      const size_t off = rg.s0 * a.sample_bytes;
+      PART_CUDA(p, cudaMemcpyPeerAsync(static_cast<char*>(a.on(o)) + off, o->dc->device, static_cast<char*>(a.on(p)) + off,
+                                       p->dc->device, n * a.sample_bytes, s));
+    }
+  }
+  return FRC_OK;
+}
+
 // Stage 1 of the embedding on stream 0 of the part: everything up to (and including) the point where this
 // part's sample shard has been made visible to the other devices.  Unsharded jobs run the whole embedding here.
 int embed_stage1(Part* p) {
@@ -461,8 +500,8 @@ int embed_stage1(Part* p) {
   if (p->d_flag_counts)
     PART_CUDA(p, cudaMemsetAsync(p->d_flag_counts, 0, sizeof(unsigned long long) * (p->mine.size() + 1), s));
   PART_CUDA(p, cudaEventRecord(p->ev_embed0, s));
+  p->info.gather_bytes = 0;
   const bool inproc = sh.exchange == Shared::kInProcess;
-  const int n_parts = sh.n_parts;
   if (sh.exact) {
     launches += launch_embed_f64(p->dtree, sh.level_ptr.data(), p->dcsr, p->d_E, sh.np, 0, s);
     // (normalisation cannot change membership, which is all the unweighted kernel reads -- and a
@@ -491,17 +530,23 @@ int embed_stage1(Part* p) {
     // <= 2 GB whatever the sample count) and leaves as the fp32 tile-panel operand + denominators;
     // a part of a sharded job only builds the slabs of its own sample shard
     const bool norm = sh.opts.normalize == 1;
+    // what the other devices read of a shard, in the order of the NCCL group: panels (unless they stay sharded:
+    // capacity mode), denominators, normalisers, key panels
+    std::vector<ShardArray> arrs;
+    if (!sh.capacity) arrs.push_back({part_array<&Part::d_A>, sizeof(float) * sh.kp});
+    arrs.push_back({part_array<&Part::d_W>, sizeof(double)});
+    if (norm) arrs.push_back({part_array<&Part::d_total>, sizeof(double)});
+    if (sh.keyed) arrs.push_back({part_array<&Part::d_K>, sizeof(int32_t) * sh.kp});
     int64_t built = 0;
-    p->info.gather_bytes = 0;
-    for (const Part::Range& rg : p->ranges) {
-      const int64_t s_begin = rg.s0, s_stop = rg.s1;
-      built += s_stop - s_begin;
-      // panels are addressed by GLOBAL sample tile inside the kernel: shift the base so that the range's
-      // first tile lands in its local slot (resident: slot == global tile, no shift)
-      float* Ap = p->d_A + (rg.slot0 - s_begin / kTile) * static_cast<int64_t>(sh.kp) * kTile;
-      int32_t* Kp = sh.keyed ? p->d_K + (rg.slot0 - s_begin / kTile) * static_cast<int64_t>(sh.kp) * kTile : nullptr;
-      for (int64_t sb = s_begin; sb < s_stop; sb += p->ws_slab) {
-        const int64_t ld = std::min<int64_t>(p->ws_slab, s_stop - sb);
+    for (const Range& rg : sh.shards.ranges[p->owner]) {
+      built += rg.s1 - rg.s0;
+      // panels are addressed by GLOBAL sample inside the kernel: shift the base so that the range lands in its
+      // local slot (resident: the slot is the range's global place, no shift)
+      const int64_t shift = (rg.slot * sh.shards.shard_rows - rg.s0) * sh.kp;
+      float* Ap = p->d_A + shift;
+      int32_t* Kp = sh.keyed ? p->d_K + shift : nullptr;
+      for (int64_t sb = rg.s0; sb < rg.s1; sb += p->ws_slab) {
+        const int64_t ld = std::min<int64_t>(p->ws_slab, rg.s1 - sb);
         // (keyed: the key panels of the slab are built by the same scatter + level passes)
         launches += launch_embed_f64(p->dtree, sh.level_ptr.data(), p->dcsr, p->d_E, ld, sb, s, Kp, sh.kp);
         if (norm) launches += launch_totals_fast_f64(p->d_E, sh.B, ld, p->d_total + sb, p->d_scratch, s);
@@ -509,44 +554,15 @@ int embed_stage1(Part* p) {
                                                    norm ? p->d_total + sb : nullptr, sh.prescale, Ap, p->d_W,
                                                    p->d_scratch, s);
       }
-      const size_t per = static_cast<size_t>(s_stop - s_begin);
-      const size_t bytes[3] = {per * sh.kp * sizeof(float), per * sizeof(double), per * sizeof(double)};
-      if (sh.exchange == Shared::kNccl) {
-        // panels, denominators (+ normalisers, + key panels: as many bytes as the value panels)
-        void* bufs[4] = {p->d_A, p->d_W, nullptr, nullptr};
-        size_t bb[4] = {bytes[0], bytes[1], 0, 0};
-        int nb = 2;
-        if (norm) { bufs[nb] = p->d_total; bb[nb++] = bytes[2]; }
-        if (sh.keyed) { bufs[nb] = p->d_K; bb[nb++] = bytes[0]; }
-        std::string cerr;
-        if (!comm_all_gather_inplace(c->comm, bufs, bb, nb, s, &cerr)) return pfail(p, FRC_ERR_CUDA, cerr);
-        p->info.gather_bytes = static_cast<int64_t>(bb[0] + bb[1] + bb[2] + bb[3]) * (sh.world - 1);
-      } else if (inproc) {
-        // the shard's denominators and normalisers -- and, unless the panels stay sharded (capacity mode), the
-        // panels themselves -- go to the same place in every other device's HBM: device-to-device copies over
-        // NVLink on the copy engines
-        for (int q = 0; q < n_parts; ++q) {
-          if (q == p->index) continue;
-          Part* o = p->job->parts[q].get();
-          if (!sh.capacity)
-            PART_CUDA(p, cudaMemcpyPeerAsync(o->d_A + s_begin * sh.kp, o->dc->device, p->d_A + s_begin * sh.kp, dc->device, bytes[0], s));
-          if (sh.keyed)
-            PART_CUDA(p, cudaMemcpyPeerAsync(o->d_K + s_begin * sh.kp, o->dc->device, p->d_K + s_begin * sh.kp, dc->device, bytes[0], s));
-          PART_CUDA(p, cudaMemcpyPeerAsync(o->d_W + s_begin, o->dc->device, p->d_W + s_begin, dc->device, bytes[1], s));
-          if (norm)
-            PART_CUDA(p, cudaMemcpyPeerAsync(o->d_total + s_begin, o->dc->device, p->d_total + s_begin, dc->device, bytes[2], s));
-        }
-        p->info.gather_bytes += static_cast<int64_t>((sh.capacity ? 0 : bytes[0]) + bytes[1] + (norm ? bytes[2] : 0) +
-                                                     (sh.keyed ? bytes[0] : 0)) * (n_parts - 1);
-      }
+      if (exchange_shard(p, arrs, rg, s)) return p->rc;
     }
     p->pm = PanelMap{};
     if (sh.capacity) {
       // own shards in their slots; the visiting shards are filled in by the rotation (start_pairs_capacity)
-      p->pm.n_shards = 2 * n_parts;
-      p->pm.tiles_per_shard = static_cast<int32_t>(sh.shard_rows / kTile);
-      for (const Part::Range& rg : p->ranges)
-        p->pm.shard[rg.s0 / sh.shard_rows] = p->d_A + rg.slot0 * static_cast<int64_t>(sh.kp) * kTile;
+      p->pm.n_shards = sh.shards.n_shards;
+      p->pm.tiles_per_shard = static_cast<int32_t>(sh.shards.shard_rows / kTile);
+      for (int k = 0; k < sh.shards.n_shards; ++k)
+        if (sh.shards.owner[k] == p->owner) p->pm.shard[k] = p->d_A + sh.shards.slot[k] * sh.shards.shard_rows * sh.kp;
     } else {
       p->pm.shard[0] = p->d_A;
     }
@@ -567,8 +583,8 @@ int embed_stage1(Part* p) {
     else if (inproc && !sh.bits_feed) {
       // in-process sharding: the kernel stores its finished bit columns straight into every device's
       // bitsT (peer access over NVLink): the all-gather is fused into the producing kernel
-      peers.n = n_parts; peers.self = p->index;
-      for (int q = 0; q < n_parts; ++q) peers.p[q] = p->job->parts[q]->d_bits;
+      peers.n = sh.n_parts; peers.self = p->index;
+      for (int q = 0; q < sh.n_parts; ++q) peers.p[q] = p->job->parts[q]->d_bits;
     }
     launches += launch_embed_presence_fused(p->dtree, p->d_level_ptr, p->dcsr, sh.nw, p->shard_w0, p->shard_nw,
                                             sh.kp, p->d_order, p->d_node_scratch, p->d_bits, p->d_bitsS, peers, s);
@@ -588,47 +604,14 @@ int embed_stage1(Part* p) {
       launches += launch_presence_rowsum_t(p->d_bits, sh.B, sh.nw, p->shard_w0, p->shard_nw, sh.kp, p->d_lenq,
                                            sh.cols.i8 ? p->d_qam : nullptr, p->d_col_exp, p->d_scratch, p->d_r,
                                            sh.cols.e_min, sh.cols.intacc ? p->d_r_int : nullptr, rs);
-    const size_t rbytes = rowsum_in_expand ? 0 : static_cast<size_t>(p->shard_nw) * 32 * sizeof(double);
-    const size_t bbytes = static_cast<size_t>(p->shard_nw) * sh.kp * sizeof(uint32_t);
-    if (sh.exchange == Shared::kNccl) {
-      // the one exchange step of the path: presence bit columns (+ row sums) of every rank's sample
-      // shard, concatenated over NVLink (2.5 GB at cfg4 instead of 120 GB of operands)
-      // (bits-fed kernel: the sample-major bit rows are what is exchanged, same size)
-      void* bufs[2];
-      size_t bytes[2];
-      int nb = 0;
-      if (!rowsum_in_expand) {
-        bufs[nb] = sh.cols.intacc ? static_cast<void*>(p->d_r_int) : static_cast<void*>(p->d_r);
-        bytes[nb++] = rbytes;
-      }
-      // peer_push: the bit columns already sit in every rank's bitsT (stored there by the embedding
-      // kernel itself); the ranks then only have to MEET before anyone reads bitsT
-      if (!p->peer_push) { bufs[nb] = sh.bits_feed ? p->d_bitsS : p->d_bits; bytes[nb++] = bbytes; }
-      std::string cerr;
-      if (nb > 0 ? !comm_all_gather_inplace(c->comm, bufs, bytes, nb, s, &cerr) : !comm_barrier(c->comm, s, &cerr))
-        return pfail(p, FRC_ERR_CUDA, cerr);
-      p->info.gather_bytes = static_cast<int64_t>(rbytes + bbytes) * (sh.world - 1);
-    } else if (inproc) {
-      // row sums of the shard (8 bytes per sample) and, for the bits-fed kernel, the shard's bit rows:
-      // small device-to-device copies to every other device
-      const int64_t s_begin = static_cast<int64_t>(p->shard_w0) * 32;
-      for (int q = 0; q < n_parts; ++q) {
-        if (q == p->index) continue;
-        Part* o = p->job->parts[q].get();
-        if (rowsum_in_expand) {
-        } else if (sh.cols.intacc) {
-          PART_CUDA(p, cudaMemcpyPeerAsync(o->d_r_int + s_begin, o->dc->device, p->d_r_int + s_begin, dc->device, rbytes, s));
-        } else {
-          PART_CUDA(p, cudaMemcpyPeerAsync(o->d_r + s_begin, o->dc->device, p->d_r + s_begin, dc->device, rbytes, s));
-        }
-        if (sh.bits_feed) {
-          const size_t roww = static_cast<size_t>(sh.kp / 32);
-          PART_CUDA(p, cudaMemcpyPeerAsync(o->d_bitsS + s_begin * roww, o->dc->device, p->d_bitsS + s_begin * roww,
-                                           dc->device, bbytes, s));
-        }
-      }
-      p->info.gather_bytes = static_cast<int64_t>(rbytes + bbytes) * (n_parts - 1);
-    }
+    // what the other parts read of the shard: row sums (unless the expansion makes them) and bit columns (2.5 GB at
+    // cfg4 instead of 120 GB of operands; bits-fed: the bit rows, same size), unless the kernel above stored them.
+    std::vector<ShardArray> arrs;
+    if (!rowsum_in_expand)
+      arrs.push_back({sh.cols.intacc ? part_array<&Part::d_r_int> : part_array<&Part::d_r>, sizeof(double)});
+    arrs.push_back({sh.bits_feed ? part_array<&Part::d_bitsS> : part_array<&Part::d_bits>, sizeof(uint32_t) * sh.kp / 32,
+                    peers.n == 0});
+    if (exchange_shard(p, arrs, sh.shards.ranges[p->owner][0], s)) return p->rc;
     if (sh.exchange != Shared::kNone) {
       // bits written + read once per level pass (+ CSR cols): this part's shard
       p->info.embed_bytes = 2LL * sh.B * p->shard_nw * 4 + 4LL * (p->csr_k1 - p->csr_k0);
@@ -793,9 +776,8 @@ int start_pairs_capacity(Part* p) {
   const Shared& sh = *p->sh;
   DevCtx* dc = p->dc;
   cudaStream_t s = dc->stream[0], cin = dc->stream[3];
-  const int G = sh.n_parts, n_shards = 2 * G;
-  const int64_t T = sh.shard_rows / kTile;
-  const size_t shard_floats = static_cast<size_t>(T) * kTile * sh.kp;
+  const ShardPlan& sp = sh.shards;
+  const size_t shard_floats = static_cast<size_t>(sp.shard_rows) * sh.kp;
   int launches = 0, n_remote = 0, last_c = 0;
   for (const Part::CapGroup& cb : p->cap) last_c = std::max(last_c, cb.shard);
   PanelMap pm = p->pm;  // own shards set by the embedding stage
@@ -804,12 +786,11 @@ int start_pairs_capacity(Part* p) {
   for (Part::CapGroup& cb : p->cap) { *cb.ex.count = 0; cb.counted = false; }
   PART_CUDA(p, cudaMemsetAsync(p->cap[0].cnt, 0, sizeof(unsigned long long) * p->cap.size(), s));
   for (int c = 0; c <= last_c; ++c) {
-    const int owner = c < G ? c : n_shards - 1 - c;
-    bool remote = owner != p->index;
+    const bool remote = sp.owner[c] != p->index;
     if (remote) {
       const int buf = n_remote++ & 1;
-      Part* o = p->job->parts[owner].get();
-      const float* src = o->d_A + (c < G ? 0 : shard_floats);
+      Part* o = p->job->parts[sp.owner[c]].get();
+      const float* src = o->d_A + sp.slot[c] * shard_floats;
       if (prev_user[buf] >= 0) PART_CUDA(p, cudaStreamWaitEvent(cin, p->ev_used[prev_user[buf]], 0));
       PART_CUDA(p, cudaStreamWaitEvent(cin, o->ev_shard, 0));  // the owner has built it
       PART_CUDA(p, cudaMemcpyPeerAsync(p->d_V[buf], dc->device, src, o->dc->device, shard_floats * sizeof(float), cin));
@@ -1169,7 +1150,8 @@ int plan_job(frc_job* j, const frc_tree_t* tree, bool neg_len) {
       sh.exchange = Shared::kNccl;
     }
   }
-  int shards = sh.exchange == Shared::kInProcess ? n_parts : sh.exchange == Shared::kNccl ? sh.world : 1;
+  const int owners = sh.n_parts > 1 ? sh.n_parts : sh.world;
+  ShardPlan::Mode mode = sh.exchange == Shared::kNone ? ShardPlan::kWhole : ShardPlan::kSharded;
   // Capacity mode of the fast weighted path: the fp32 panels of ALL samples (kp x np x 4 bytes: 320 GB at
   // BASELINE config 5) would not fit one device -> they stay sharded where they are built (two shards per
   // device) and the pair tiles read remote column panels over NVLink (PanelMap, weighted.cu).
@@ -1177,7 +1159,7 @@ int plan_job(frc_job* j, const frc_tree_t* tree, bool neg_len) {
     bool want = sh.knobs.capacity == 1;
     if (!want) {
       // (keyed -l tiles: an int32 key next to every fp32 value)
-      const double panels = (sh.keyed ? 8.0 : 4.0) * static_cast<double>(round_up(sh.B, kKBlock)) * static_cast<double>(round_up(sh.N, kTile * 2LL * n_parts));
+      const double panels = (sh.keyed ? 8.0 : 4.0) * static_cast<double>(round_up(sh.B, kKBlock)) * static_cast<double>(plan_shards(sh.N, n_parts, ShardPlan::kCapacity).np);
       if (panels > 24.0 * (1 << 30)) {  // (cudaMemGetInfo costs milliseconds: only asked when it can matter)
         size_t free_b = 0, total_b = 0;
         cudaSetDevice(c->devs[0]->device);
@@ -1191,11 +1173,10 @@ int plan_job(frc_job* j, const frc_tree_t* tree, bool neg_len) {
                                           "over the devices when they exceed about half of one device's free HBM (or with "
                                           "FRC_CAPACITY=1), does not carry keys");
     sh.capacity = want;
-    if (want) shards = 2 * n_parts;
+    if (want) mode = ShardPlan::kCapacity;
   }
-  // sharded: every owner builds np / shards samples, a whole number of tiles
-  sh.np = std::max<int64_t>(kTile, round_up(sh.N, kTile * static_cast<int64_t>(shards)));
-  sh.shard_rows = sh.capacity ? sh.np / shards : 0;
+  sh.shards = plan_shards(sh.N, owners, mode);
+  sh.np = sh.shards.np;
   sh.nw = static_cast<int32_t>(sh.np / 32);
   sh.kp = static_cast<int32_t>(round_up(sh.B, kKBlock));
   sh.prescale = !neg_len;
@@ -1217,8 +1198,7 @@ int plan_job(frc_job* j, const frc_tree_t* tree, bool neg_len) {
       }
     }
   }
-  const int owners = sh.n_parts > 1 ? sh.n_parts : sh.world;
-  sh.bands = sh.capacity ? make_bands_capacity(sh.N, sh.np, n_parts, sh.opts.band_rows, sh.d2h)
+  sh.bands = sh.capacity ? make_bands_capacity(sh.N, sh.shards, sh.opts.band_rows, sh.d2h)
                          : make_bands(sh.N, sh.opts.band_rows, owners, sh.d2h, sh.knobs.bands_per_rank, 8);
   for (const Band& b : sh.bands)
     if (b.count >= (1LL << 32)) return fail(j, FRC_ERR_UNSUPPORTED, "band too large; lower band_rows");
@@ -1280,7 +1260,7 @@ int prepare_part(Part* p) {
     // one group per row shard of this part (csrc/plan.cpp): its bands, and its tiles grouped by COLUMN SHARD (the
     // order the shards visit in), column-major inside a column shard (the CTAs of a wave share a column panel)
     const std::vector<CapGroupPlan> groups =
-        plan_capacity_groups(p->bands, sh.N, sh.shard_rows, 2 * sh.n_parts, p->tiles, p->band_group);
+        plan_capacity_groups(p->bands, sh.N, sh.shards.shard_rows, sh.shards.n_shards, p->tiles, p->band_group);
     for (const CapGroupPlan& gp : groups) {
       if (gp.count >= (1LL << 32)) return pfail(p, FRC_ERR_UNSUPPORTED, "capacity mode: a row shard holds 2^32 pairs or more");
       Part::CapGroup g;
@@ -1290,32 +1270,19 @@ int prepare_part(Part* p) {
   } else if (!sh.exact) {
     for (Band& b : p->bands) append_band_tiles(b, fast_uw, p->tiles);
   }
-  const int owners = sh.n_parts > 1 ? sh.n_parts : sh.world;
   std::vector<uint8_t> need;
-  if (fast_uw && owners > 1 && sh.fused_embed) need = operand_need_blocks(p->tiles, sh.np, true);
-  // ---- sample shard
-  const int shards = sh.exchange == Shared::kNone ? 1 : owners;
-  p->shard_nw = sh.nw / shards;
-  p->shard_w0 = sh.exchange == Shared::kNone ? 0 : p->owner * p->shard_nw;
-  if (sh.capacity) {
-    // two shards per device (d and 2G-1-d: balanced pair counts), panels in slots 0 and 1 of the local array
-    const int64_t R = sh.shard_rows;
-    const int64_t a = p->owner, b = 2LL * sh.n_parts - 1 - p->owner;
-    p->ranges = {{a * R, (a + 1) * R, 0}, {b * R, (b + 1) * R, R / kTile}};
-    p->shard_nw = static_cast<int32_t>(R / 32);  // (slab sizing below)
-  } else {
-    p->ranges = {{static_cast<int64_t>(p->shard_w0) * 32, (static_cast<int64_t>(p->shard_w0) + p->shard_nw) * 32,
-                  static_cast<int64_t>(p->shard_w0) * 32 / kTile}};
-  }
+  if (fast_uw && sh.shards.ranges.size() > 1 && sh.fused_embed) need = operand_need_blocks(p->tiles, sh.np, true);
+  // ---- sample shard: the first range of this owner (capacity: the second one is as large)
+  const Range& own = sh.shards.ranges[p->owner][0];
+  p->shard_w0 = static_cast<int32_t>(own.s0 / 32);
+  p->shard_nw = static_cast<int32_t>((own.s1 - own.s0) / 32);
   // CSR entries this part uploads: its own rows when only the embedding reads the table (the weighted
   // fix-up walks the rows of any flagged pair, so weighted parts keep the whole table)
   p->csr_k0 = 0; p->csr_k1 = sh.nnz;
   if (sh.exchange != Shared::kNone && fast_uw && sh.N > 0) {
     const int64_t* rp = reinterpret_cast<const int64_t*>(sh.stage_in + sh.in_rowptr.off);
-    const int64_t s0 = std::min<int64_t>(sh.N, static_cast<int64_t>(p->shard_w0) * 32);
-    const int64_t s1 = std::min<int64_t>(sh.N, s0 + static_cast<int64_t>(p->shard_nw) * 32);
     // (row_ptr is copied into the staging buffer before any task starts)
-    p->csr_k0 = rp[s0]; p->csr_k1 = rp[s1];
+    p->csr_k0 = rp[std::min(sh.N, own.s0)]; p->csr_k1 = rp[std::min(sh.N, own.s1)];
   }
   // ---- per-part staging: tiles + need blocks
   SegAlloc seg;
@@ -1383,15 +1350,15 @@ int prepare_part(Part* p) {
     if (sh.unsorted_l && !(p->d_list_ptr = dev_alloc<int64_t>(p, sh.N + 2))) return p->rc;
     if (!sh.exact) {
       // resident: the panels of all samples; capacity: of this device's two shards only
-      const size_t a_samples = sh.capacity ? static_cast<size_t>(2 * sh.shard_rows) : static_cast<size_t>(sh.np);
+      const size_t a_samples = sh.capacity ? static_cast<size_t>(2 * sh.shards.shard_rows) : static_cast<size_t>(sh.np);
       if (!(p->d_A = dev_alloc<float>(p, static_cast<size_t>(sh.kp) * a_samples))) return p->rc;
       if (sh.keyed && !(p->d_K = dev_alloc<int32_t>(p, static_cast<size_t>(sh.kp) * a_samples))) return p->rc;
       if (sh.capacity) {
         for (int k = 0; k < 2; ++k)
-          if (!(p->d_V[k] = dev_alloc<float>(p, static_cast<size_t>(sh.kp) * sh.shard_rows))) return p->rc;
-        p->ev_fetch.assign(2 * sh.n_parts, nullptr);
-        p->ev_used.assign(2 * sh.n_parts, nullptr);
-        for (int k = 0; k < 2 * sh.n_parts; ++k) {
+          if (!(p->d_V[k] = dev_alloc<float>(p, static_cast<size_t>(sh.kp) * sh.shards.shard_rows))) return p->rc;
+        p->ev_fetch.assign(sh.shards.n_shards, nullptr);
+        p->ev_used.assign(sh.shards.n_shards, nullptr);
+        for (int k = 0; k < sh.shards.n_shards; ++k) {
           PART_CUDA(p, cudaEventCreateWithFlags(&p->ev_fetch[k], cudaEventDisableTiming));
           PART_CUDA(p, cudaEventCreateWithFlags(&p->ev_used[k], cudaEventDisableTiming));
         }
@@ -1746,13 +1713,11 @@ int frc_create(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
 #endif
     csr_us[t] += std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - w0).count();
   };
-  // multi-process sharded unweighted: the rows of this rank's shard only (decided before the tasks start;
-  // np is not planned yet, so the shard bounds are computed here the way plan_job will)
+  // multi-process sharded unweighted: the rows of this rank's shard only (decided before the tasks start, from the
+  // shard plan that plan_job will make)
   if (!sh.exact && !sh.weighted && sh.n_parts == 1 && sh.world > 1 && (opts->flags & FRC_FLAG_SHARD_EMBED) && N > 0) {
-    const int64_t np = std::max<int64_t>(kTile, round_up(N, kTile * static_cast<int64_t>(sh.world)));
-    const int64_t per = np / sh.world;
-    const int64_t s0 = std::min<int64_t>(N, sh.rank0 * per), s1 = std::min<int64_t>(N, s0 + per);
-    stage_k0 = abnd->row_ptr[s0]; stage_k1 = abnd->row_ptr[s1];
+    const Range own = plan_shards(N, sh.world, ShardPlan::kSharded).ranges[sh.rank0][0];
+    stage_k0 = abnd->row_ptr[std::min(N, own.s0)]; stage_k1 = abnd->row_ptr[std::min(N, own.s1)];
   }
   const int n_workers = c->pool->size() - 1;
   if (n_workers > 0) {

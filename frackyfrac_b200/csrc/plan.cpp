@@ -115,15 +115,34 @@ std::vector<Band> make_bands(int64_t N, int64_t requested, int world, bool d2h, 
   return bands;
 }
 
-std::vector<Band> make_bands_capacity(int64_t N, int64_t np, int G, int64_t requested, bool d2h) {
+ShardPlan plan_shards(int64_t N, int owners, ShardPlan::Mode mode) {
+  ShardPlan sp;
+  owners = std::max(1, owners);
+  sp.n_shards = mode == ShardPlan::kWhole ? 1 : mode == ShardPlan::kCapacity ? 2 * owners : owners;
+  sp.np = std::max<int64_t>(kTile, round_up(N, kTile * static_cast<int64_t>(sp.n_shards)));
+  sp.shard_rows = sp.np / sp.n_shards;
+  sp.ranges.resize(owners);
+  for (int s = 0; s < sp.n_shards; ++s) {
+    const int owner = mode == ShardPlan::kWhole ? -1 : s < owners ? s : sp.n_shards - 1 - s;
+    const int slot = mode == ShardPlan::kCapacity ? (s < owners ? 0 : 1) : s;
+    sp.owner.push_back(owner);
+    sp.slot.push_back(slot);
+    const Range rg{s * sp.shard_rows, (s + 1) * sp.shard_rows, slot};  // (ascending s: every owner's in slot order)
+    if (owner >= 0) sp.ranges[owner].push_back(rg);
+    else for (std::vector<Range>& r : sp.ranges) r.push_back(rg);
+  }
+  return sp;
+}
+
+std::vector<Band> make_bands_capacity(int64_t N, const ShardPlan& sp, int64_t requested, bool d2h) {
   std::vector<Band> bands;
-  if (N < 2 || G < 1) return bands;
-  const int64_t R = np / (2 * static_cast<int64_t>(G));  // rows per shard, a multiple of the tile size
+  if (N < 2) return bands;
+  const int64_t R = sp.shard_rows;
   const double band_cap = (d2h ? 96.0 : 1536.0) * 1024 * 1024 / 8.0;  // pairs per band, as in band_boundaries
-  for (int s = 0; s < 2 * G; ++s) {
+  for (int s = 0; s < sp.n_shards; ++s) {
     const int64_t r0 = s * R, r1 = std::min<int64_t>(N, (s + 1) * R);
     if (r0 >= r1) break;
-    const int owner = s < G ? s : 2 * G - 1 - s;
+    const int owner = sp.owner[s];
     std::vector<int64_t> rows;
     rows.push_back(r0);
     if (requested > 0) {
@@ -380,48 +399,69 @@ void tree_post_order(const int32_t* parent, int32_t B, int32_t* post_order) {
 // ---------------------------------------------------------------- CPU test entry points
 // Not part of the C ABI (include/frcfrc_cuda.h): they let tests/test_plan.py exercise the planning
 // units on the CPU-only box.
+static int64_t write_bands(const std::vector<frc::Band>& bands, int64_t* out5, int64_t cap) {
+  for (size_t k = 0; k < bands.size() && static_cast<int64_t>(k) < cap; ++k) {
+    out5[5 * k] = bands[k].row0; out5[5 * k + 1] = bands[k].row1; out5[5 * k + 2] = bands[k].first;
+    out5[5 * k + 3] = bands[k].count; out5[5 * k + 4] = bands[k].owner;
+  }
+  return static_cast<int64_t>(bands.size());
+}
+
 extern "C" {
 
 // Bands of the whole triangle: writes up to `cap` (row0, row1, first, count, owner) quintuples; returns the count.
 int64_t frc_debug_bands(int64_t n_samples, int64_t band_rows, int32_t world, int32_t d2h, int32_t per_rank,
                         int32_t value_bytes, int64_t* out5, int64_t cap) {
-  const std::vector<frc::Band> bands = frc::make_bands(n_samples, band_rows, world, d2h != 0, per_rank, value_bytes);
-  for (size_t k = 0; k < bands.size() && static_cast<int64_t>(k) < cap; ++k) {
-    out5[5 * k] = bands[k].row0; out5[5 * k + 1] = bands[k].row1; out5[5 * k + 2] = bands[k].first;
-    out5[5 * k + 3] = bands[k].count; out5[5 * k + 4] = bands[k].owner;
-  }
-  return static_cast<int64_t>(bands.size());
+  return write_bands(frc::make_bands(n_samples, band_rows, world, d2h != 0, per_rank, value_bytes), out5, cap);
 }
 
-// Capacity-mode bands (2G row shards, owner s or 2G-1-s): same output layout as frc_debug_bands.
+// Sample shards (plan_shards; mode 0 whole, 1 sharded, 2 capacity): info = {np, n_shards, shard_rows}, (owner, slot)
+// per shard into out2 (cap_shards of them), (owner, s0, s1, slot) per range of every owner in turn into out4 (cap of
+// them).  Returns the number of ranges (negative: a cap was too small).
+int64_t frc_debug_shards(int64_t n_samples, int32_t owners, int32_t mode, int64_t* info, int32_t* out2, int64_t cap_shards,
+                         int64_t* out4, int64_t cap) {
+  const frc::ShardPlan sp = frc::plan_shards(n_samples, owners, static_cast<frc::ShardPlan::Mode>(mode));
+  info[0] = sp.np; info[1] = sp.n_shards; info[2] = sp.shard_rows;
+  if (sp.n_shards > cap_shards) return -1;
+  for (int s = 0; s < sp.n_shards; ++s) { out2[2 * s] = sp.owner[s]; out2[2 * s + 1] = sp.slot[s]; }
+  int64_t k = 0;
+  for (size_t r = 0; r < sp.ranges.size(); ++r)
+    for (const frc::Range& rg : sp.ranges[r]) {
+      if (k == cap) return -1;
+      out4[4 * k] = static_cast<int64_t>(r); out4[4 * k + 1] = rg.s0; out4[4 * k + 2] = rg.s1; out4[4 * k + 3] = rg.slot;
+      ++k;
+    }
+  return k;
+}
+
+// Capacity-mode bands (the capacity shards of n_dev devices): same output layout as frc_debug_bands (-1: np is not theirs).
 int64_t frc_debug_bands_capacity(int64_t n_samples, int64_t np, int32_t n_dev, int64_t band_rows, int32_t d2h,
                                  int64_t* out5, int64_t cap) {
-  const std::vector<frc::Band> bands = frc::make_bands_capacity(n_samples, np, n_dev, band_rows, d2h != 0);
-  for (size_t k = 0; k < bands.size() && static_cast<int64_t>(k) < cap; ++k) {
-    out5[5 * k] = bands[k].row0; out5[5 * k + 1] = bands[k].row1; out5[5 * k + 2] = bands[k].first;
-    out5[5 * k + 3] = bands[k].count; out5[5 * k + 4] = bands[k].owner;
-  }
-  return static_cast<int64_t>(bands.size());
+  const frc::ShardPlan sp = frc::plan_shards(n_samples, n_dev, frc::ShardPlan::kCapacity);
+  if (sp.np != np) return -1;
+  return write_bands(frc::make_bands_capacity(n_samples, sp, band_rows, d2h != 0), out5, cap);
 }
 
 // Capacity-mode groups of device `dev`: out_groups holds (shard, first, count, tile_off) quadruples, out_coff
 // (n_shards + 1) offsets per group, out_tiles (ti, tj) pairs; returns the number of groups, *n_tiles the tile count
-// (negative: a cap was too small).
+// (negative: a cap was too small, or np is not the plan's padded sample count).
 int64_t frc_debug_capacity_groups(int64_t n_samples, int64_t np, int32_t n_dev, int32_t dev, int64_t band_rows, int32_t d2h,
                                   int64_t* out_groups, int32_t* out_coff, int64_t cap_groups, int32_t* out_tiles,
                                   int64_t cap_tiles, int64_t* n_tiles) {
-  const std::vector<frc::Band> all = frc::make_bands_capacity(n_samples, np, n_dev, band_rows, d2h != 0);
+  const frc::ShardPlan sp = frc::plan_shards(n_samples, n_dev, frc::ShardPlan::kCapacity);
+  if (sp.np != np) return -1;
+  const std::vector<frc::Band> all = frc::make_bands_capacity(n_samples, sp, band_rows, d2h != 0);
   std::vector<frc::Band> mine;
   for (const frc::Band& b : all)
     if (b.owner == dev) mine.push_back(b);
   std::vector<frc::Tile> tiles;
   std::vector<int> band_group;
-  const std::vector<frc::CapGroupPlan> g = frc::plan_capacity_groups(mine, n_samples, np / (2 * n_dev), 2 * n_dev, tiles, band_group);
+  const std::vector<frc::CapGroupPlan> g = frc::plan_capacity_groups(mine, n_samples, sp.shard_rows, sp.n_shards, tiles, band_group);
   *n_tiles = static_cast<int64_t>(tiles.size());
   if (static_cast<int64_t>(g.size()) > cap_groups || static_cast<int64_t>(tiles.size()) > cap_tiles) return -1;
   for (size_t k = 0; k < g.size(); ++k) {
     out_groups[4 * k] = g[k].shard; out_groups[4 * k + 1] = g[k].first; out_groups[4 * k + 2] = g[k].count; out_groups[4 * k + 3] = g[k].tile_off;
-    for (int c = 0; c <= 2 * n_dev; ++c) out_coff[k * (2 * n_dev + 1) + c] = g[k].coff[c];
+    for (int c = 0; c <= sp.n_shards; ++c) out_coff[k * (sp.n_shards + 1) + c] = g[k].coff[c];
   }
   for (size_t k = 0; k < tiles.size(); ++k) { out_tiles[2 * k] = tiles[k].ti; out_tiles[2 * k + 1] = tiles[k].tj; }
   return static_cast<int64_t>(g.size());

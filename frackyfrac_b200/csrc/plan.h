@@ -36,10 +36,25 @@ std::vector<int> band_owners(const std::vector<int64_t>& rows, int world);
 // Every non-empty band of the triangle, in flat-index order, with its owner.
 std::vector<Band> make_bands(int64_t N, int64_t requested, int world, bool d2h, int per_rank, int value_bytes);
 
-// Capacity mode of the fast weighted path (PanelMap in frc_internal.h): the padded sample range [0, np) is cut
-// into 2G shards of np / 2G rows; shard s belongs to device s (s < G) or 2G-1-s, which balances the pair counts
-// (row r has r columns: the two shards of a device add up to the same total).  Bands never straddle a shard.
-std::vector<Band> make_bands_capacity(int64_t N, int64_t np, int G, int64_t requested, bool d2h);
+// Sample shards of the embedding: the padded samples [0, np) in n_shards shards of shard_rows samples (whole tiles).
+// A shard sits in its owner's per-sample arrays at [slot * shard_rows, +shard_rows).
+//   kWhole    one shard, built by every owner;
+//   kSharded  shard r on owner r at its global place (slot r), as the in-place all-gather needs it;
+//   kCapacity 2G shards, device d holds shards d and 2G-1-d in slots 0 and 1: row r has r columns, so the two
+//             shards of every device add up to the same pair count.
+struct Range { int64_t s0, s1, slot; };  // samples [s0, s1) in slot `slot` of their owner
+struct ShardPlan {
+  enum Mode { kWhole, kSharded, kCapacity };
+  int64_t np = 0, shard_rows = 0;
+  int n_shards = 1;
+  std::vector<int> owner, slot;            // per shard (owner -1: every owner)
+  std::vector<std::vector<Range>> ranges;  // per owner, in slot order
+};
+ShardPlan plan_shards(int64_t N, int owners, ShardPlan::Mode mode);
+
+// Capacity mode of the fast weighted path (PanelMap in frc_internal.h): the bands of every shard of `sp`, owned by
+// the shard's device.  Bands never straddle a shard.
+std::vector<Band> make_bands_capacity(int64_t N, const ShardPlan& sp, int64_t requested, bool d2h);
 
 // Capacity mode, one device: its bands (in row order) grouped by row shard, and per group the tile list ordered by
 // the COLUMN shard the tiles read (the order the shards visit in), column-major inside a column shard.

@@ -241,3 +241,54 @@ def test_capacity_groups_cover_every_tile_once_in_visiting_order(L):
         nt_rows = (n + 127) // 128
         assert pairs == n * (n - 1) // 2
         assert set(seen) == {(ti, tj) for ti in range(nt_rows) for tj in range(ti + 1)}
+
+
+def _bands_capacity(L, n, np_, G, band_rows=0, d2h=1):
+    L.frc_debug_bands_capacity.argtypes = [C.c_int64, C.c_int64, C.c_int32, C.c_int64, C.c_int32, C.c_void_p, C.c_int64]
+    L.frc_debug_bands_capacity.restype = C.c_int64
+    out = np.zeros((1 << 14, 5), np.int64)
+    k = L.frc_debug_bands_capacity(n, np_, G, band_rows, d2h, out.ctypes.data, len(out))
+    assert 0 <= k <= len(out)
+    return out[:k]
+
+
+def _shards(L, n, owners, mode):
+    L.frc_debug_shards.argtypes = [C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64]
+    L.frc_debug_shards.restype = C.c_int64
+    info, shards, ranges = np.zeros(3, np.int64), np.zeros((64, 2), np.int32), np.zeros((64, 4), np.int64)
+    k = L.frc_debug_shards(n, owners, mode, info.ctypes.data, shards.ctypes.data, len(shards), ranges.ctypes.data,
+                           len(ranges))
+    assert k > 0
+    np_, n_shards, shard_rows = info.tolist()
+    return np_, n_shards, shard_rows, shards[:n_shards], ranges[:k]
+
+
+@pytest.mark.parametrize("mode", [0, 1, 2])
+def test_sample_shards_partition_the_padded_samples(L, mode):
+    """The sample shards of the embedding (0: every owner builds everything, 1: one shard per owner, 2: capacity
+    mode, two per device): padded to whole tiles of every shard, every sample built once (mode 0: by every owner)."""
+    for n in (1, 127, 128, 1000, 14142, 100_000):
+        for owners in range(1, 9):
+            np_, n_shards, R, shards, ranges = _shards(L, n, owners, mode)
+            assert n_shards == (1, owners, 2 * owners)[mode]
+            assert np_ >= n and np_ % (128 * n_shards) == 0 and R * n_shards == np_
+            assert sorted(set(ranges[:, 0].tolist())) == list(range(owners))
+            assert (ranges[:, 1:3] % 128 == 0).all()
+            if mode == 0:
+                assert shards.tolist() == [[-1, 0]]
+                assert ranges.tolist() == [[r, 0, np_, 0] for r in range(owners)]
+                continue
+            cover = np.zeros(np_, np.int32)
+            for owner, s0, s1, slot in ranges.tolist():
+                cover[s0:s1] += 1
+                assert s1 == s0 + R and shards[s0 // R].tolist() == [owner, slot]
+            assert (cover == 1).all()
+            if mode == 1:
+                # what the in-place all-gather relies on: owner r holds exactly shard r, at its global place
+                assert ranges.tolist() == [[r, r * R, (r + 1) * R, r] for r in range(owners)]
+            else:
+                # device d holds shards d and 2G-1-d, in slots 0 and 1
+                assert ranges.tolist() == [x for d in range(owners) for x in
+                                           ([d, d * R, (d + 1) * R, 0], [d, (2 * owners - 1 - d) * R, (2 * owners - d) * R, 1])]
+                for row0, row1, _, _, owner in _bands_capacity(L, n, np_, owners).tolist():
+                    assert (row1 - 1) // R == row0 // R and owner == shards[row0 // R, 0]
