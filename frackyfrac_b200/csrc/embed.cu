@@ -101,22 +101,29 @@ __global__ void k_normalize_f64(double* E, int32_t n_nodes, int64_t ld, int64_t 
 
 // Fast-path totals: partial[c][s] = sum of E[v][s] over the nodes of chunk c (any order will do off
 // the exact path; the sequential ascending-id loop of k_totals_f64 is one dependent fp64 chain per
-// sample and was latency-bound).
+// sample and was latency-bound).  kMult (pruned tree, FRC_FLAG_PRUNE): node v stands for mult[v] original nodes
+// that all hold E[v][s], and the default normaliser counts each of them.
+template <bool kMult>
 __global__ void k_totals_partial_f64(const double* __restrict__ E, int32_t n_nodes, int64_t ld,
-                                     double* __restrict__ partial) {
+                                     const double* __restrict__ mult, double* __restrict__ partial) {
   int64_t s = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (s >= ld) return;
   int32_t per = (n_nodes + gridDim.y - 1) / gridDim.y;
   int32_t v0 = blockIdx.y * per, v1 = min(n_nodes, v0 + per);
+  auto term = [&](int32_t u) {
+    const double x = E[static_cast<int64_t>(u) * ld + s];
+    if constexpr (kMult) return mult[u] * x;
+    else return x;
+  };
   double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0;
   int32_t v = v0;
   for (; v + 4 <= v1; v += 4) {
-    a0 += E[static_cast<int64_t>(v) * ld + s];
-    a1 += E[static_cast<int64_t>(v + 1) * ld + s];
-    a2 += E[static_cast<int64_t>(v + 2) * ld + s];
-    a3 += E[static_cast<int64_t>(v + 3) * ld + s];
+    a0 += term(v);
+    a1 += term(v + 1);
+    a2 += term(v + 2);
+    a3 += term(v + 3);
   }
-  for (; v < v1; ++v) a0 += E[static_cast<int64_t>(v) * ld + s];
+  for (; v < v1; ++v) a0 += term(v);
   partial[static_cast<int64_t>(blockIdx.y) * ld + s] = (a0 + a1) + (a2 + a3);
 }
 
@@ -670,11 +677,12 @@ static int pick_chunks(int32_t n_nodes) {
   return c < 1 ? 1 : (c > 64 ? 64 : c);
 }
 
-int launch_totals_fast_f64(const double* E, int32_t n_nodes, int64_t ld, double* total, double* scratch,
-                           cudaStream_t s) {
+int launch_totals_fast_f64(const double* E, int32_t n_nodes, int64_t ld, const double* mult, double* total,
+                           double* scratch, cudaStream_t s) {
   const int chunks = pick_chunks(n_nodes);
   dim3 grid(static_cast<unsigned>((ld + kThreads - 1) / kThreads), chunks);
-  k_totals_partial_f64<<<grid, kThreads, 0, s>>>(E, n_nodes, ld, scratch);
+  if (mult) k_totals_partial_f64<true><<<grid, kThreads, 0, s>>>(E, n_nodes, ld, mult, scratch);
+  else k_totals_partial_f64<false><<<grid, kThreads, 0, s>>>(E, n_nodes, ld, nullptr, scratch);
   k_reduce_partials<<<static_cast<unsigned>((ld + kThreads - 1) / kThreads), kThreads, 0, s>>>(scratch, chunks, ld, ld,
                                                                                              total);
   return 2;

@@ -68,8 +68,9 @@ int launch_embed_f64(const DevTree& t, const int32_t* level_ptr_host, const DevC
 int launch_totals_f64(const double* E, int32_t n_nodes, int64_t ld, int64_t n_samples,
                       double* total, cudaStream_t s);
 // Same totals for the fast path (chunked partial sums, any order; scratch as for launch_weighted_operand).
-int launch_totals_fast_f64(const double* E, int32_t n_nodes, int64_t ld, double* total, double* scratch,
-                           cudaStream_t s);
+// mult (merged tree, FRC_FLAG_PRUNE; else nullptr): total[s] = sum of mult[v] * E[v][s].
+int launch_totals_fast_f64(const double* E, int32_t n_nodes, int64_t ld, const double* mult, double* total,
+                           double* scratch, cudaStream_t s);
 // E[v][s] /= total[s] for non-zero entries (unifrac.go:64-66).
 int launch_normalize_f64(double* E, int32_t n_nodes, int64_t ld, int64_t n_samples,
                          const double* total, cudaStream_t s);

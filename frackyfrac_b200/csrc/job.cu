@@ -203,6 +203,7 @@ struct Shared {
   bool exact = false, weighted = false, prescale = true, need_val = false;
   bool unsorted_l = false;    // normalize == 0 on the exact path: the reference's -l as coded (post-order lists, exact.cu)
   bool keyed = false;         // normalize == 0 on the FP32 tiles (FRC_FLAG_L_TILES): key panels next to the values
+  bool node_mult = false;     // FRC_FLAG_PRUNE, fast weighted, normalize == 1: the totals weigh node v by mult[v]
   bool d2h = true;
   int n_parts = 1;
   int world = 1, rank0 = 0;   // band ownership: `world` owners; part p owns owner id rank0 + p
@@ -216,7 +217,7 @@ struct Shared {
   int32_t tree_height = 0;
   // inputs: [row_ptr | tree arrays ... | col | val] in one pinned buffer, same layout on every device
   char* stage_in = nullptr;
-  Seg in_rowptr, in_parent, in_len, in_cptr, in_cidx, in_lvl, in_lpar, in_lptr, in_lenf, in_post, in_col, in_val;
+  Seg in_rowptr, in_parent, in_len, in_cptr, in_cidx, in_lvl, in_lpar, in_lptr, in_lenf, in_post, in_mult, in_col, in_val;
   size_t in_bytes = 0;
   // plan: operand columns, chunks
   char* stage_plan = nullptr;
@@ -296,6 +297,7 @@ struct Part {
   double *d_lenq = nullptr, *d_len_col = nullptr, *d_flag_u = nullptr, *d_qerr = nullptr;
   TcChunks d_chunks;
   float* d_lenf = nullptr;
+  const double* d_mult = nullptr;  // FRC_FLAG_PRUNE: original nodes per node of the merged tree (Shared::node_mult)
   double *d_E = nullptr, *d_total = nullptr, *d_W = nullptr, *d_r = nullptr, *d_scratch = nullptr;
   float* d_A = nullptr;
   int32_t* d_K = nullptr;     // keyed -l tiles: key panels, same layout as d_A (resident only)
@@ -549,7 +551,7 @@ int embed_stage1(Part* p) {
         const int64_t ld = std::min<int64_t>(p->ws_slab, rg.s1 - sb);
         // (keyed: the key panels of the slab are built by the same scatter + level passes)
         launches += launch_embed_f64(p->dtree, sh.level_ptr.data(), p->dcsr, p->d_E, ld, sb, s, Kp, sh.kp);
-        if (norm) launches += launch_totals_fast_f64(p->d_E, sh.B, ld, p->d_total + sb, p->d_scratch, s);
+        if (norm) launches += launch_totals_fast_f64(p->d_E, sh.B, ld, p->d_mult, p->d_total + sb, p->d_scratch, s);
         launches += launch_weighted_operand_panels(p->d_E, p->dtree.length, sh.B, sh.kp, ld, sb,
                                                    norm ? p->d_total + sb : nullptr, sh.prescale, Ap, p->d_W,
                                                    p->d_scratch, s);
@@ -1126,6 +1128,7 @@ void layout_inputs(Shared& sh) {
   sh.in_lptr = seg(sizeof(int32_t) * (static_cast<size_t>(B) + 2));
   sh.in_lenf = seg(sizeof(float) * kp_pad);
   sh.in_post = seg(sh.unsorted_l ? sizeof(int32_t) * B : 0);
+  sh.in_mult = seg(sh.node_mult ? sizeof(double) * B : 0);
   sh.in_col = seg(sizeof(int32_t) * sh.nnz);   // the two bulk arrays last: a sharded part uploads a slice of them
   sh.in_val = seg(sh.need_val ? sizeof(double) * sh.nnz : 0);
   sh.in_bytes = seg.total;
@@ -1321,6 +1324,7 @@ int prepare_part(Part* p) {
   p->d_level_ptr = reinterpret_cast<int32_t*>(di + sh.in_lptr.off);
   p->d_lenf = reinterpret_cast<float*>(di + sh.in_lenf.off);
   p->d_post = sh.unsorted_l ? reinterpret_cast<int32_t*>(di + sh.in_post.off) : nullptr;
+  p->d_mult = sh.node_mult ? reinterpret_cast<const double*>(di + sh.in_mult.off) : nullptr;
   p->d_q0 = d + sh.pl_q0.off;
   p->d_q1 = d + sh.pl_hi.off;
   p->d_q2 = d + sh.pl_lo.off;
@@ -1577,7 +1581,7 @@ int frc_create(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
   // ------------------------------------------------------------ (1) options, table header
   int rc = validate_header(j, tree, abnd, opts);
   if (rc) return bail(rc);
-  const int32_t B = sh.B;
+  const int32_t B0 = sh.B;  // the caller's tree (FRC_FLAG_PRUNE: B = the pruned one)
   const int64_t N = sh.N, nnz = sh.nnz;
 
   // ------------------------------------------------------------ context
@@ -1601,6 +1605,42 @@ int frc_create(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
     p->job = j; p->sh = &sh; p->dc = c->devs[k]; p->index = k;
     p->owner = sh.n_parts > 1 ? k : sh.rank0;
   }
+
+  // ------------------------------------------------------------ FRC_FLAG_PRUNE: the subtree the table observes
+  // Everything from the layout on runs on the pruned tree; the entries are still checked against the caller's tree
+  // (same checks, same node ids in the messages) and staged with their new ids.
+  const frc_tree_t* const tree0 = tree;
+  PrunedTree pruned;
+  frc_tree_t ptree{};
+  if (opts->flags & FRC_FLAG_PRUNE) {
+    std::vector<int32_t> depth(B0);
+    int32_t bad_parent = 0, bad_order = 0;
+    // (a tree that fails the check is not pruned: the tree walks below report it as they do without the flag)
+    if (check_preorder(tree0->parent, B0, depth.data(), &bad_parent, &bad_order)) {
+      // the leaves listed in ANY row: every rank of a sharded multi-process job derives the same tree (out-of-range
+      // entries are left to the staging checks)
+      std::vector<uint8_t> marks(B0, 0);
+      const int T = nnz >= 65536 ? c->pool->size() : 1;
+      const std::function<void(int)> mark_leaves = [&](int t) {
+        const int64_t k1 = nnz * (t + 1) / T;
+        for (int64_t k = nnz * t / T; k < k1; ++k) {
+          const int32_t cc = abnd->col[k];
+          // (read first: storing into lines that are already marked would bounce them between the cores)
+          if (cc >= 0 && cc < B0 && !__atomic_load_n(&marks[cc], __ATOMIC_RELAXED))
+            __atomic_store_n(&marks[cc], uint8_t{1}, __ATOMIC_RELAXED);
+        }
+      };
+      c->pool->run(T, mark_leaves);
+      // merging reorders the fp64 sums of the exact path: it is only pruned
+      pruned = prune_tree(tree0->parent, tree0->length, B0, marks.data(), !sh.exact);
+      ptree = frc_tree_t{pruned.n_nodes, pruned.parent.data(), pruned.length.data()};
+      tree = &ptree;
+      sh.B = pruned.n_nodes;
+      sh.node_mult = !sh.exact && sh.weighted && opts->normalize == 1;
+    }
+  }
+  const int32_t B = sh.B;
+  const int32_t* const new_of_old = pruned.new_of_old.empty() ? nullptr : pruned.new_of_old.data();
 
   // ------------------------------------------------------------ (2) staging buffer; row_ptr right away
   layout_inputs(sh);
@@ -1628,6 +1668,10 @@ int frc_create(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
     const int32_t kp_pad = static_cast<int32_t>(round_up(B, kKBlock));
     for (int32_t v = 0; v < kp_pad; ++v) lf[v] = v < B ? static_cast<float>(tree->length[v]) : 0.f;
     if (sh.unsorted_l) tree_post_order(tree->parent, B, reinterpret_cast<int32_t*>(stage_in + sh.in_post.off));
+    if (sh.node_mult) {
+      double* m = reinterpret_cast<double*>(stage_in + sh.in_mult.off);
+      for (int32_t v = 0; v < B; ++v) m[v] = pruned.mult[v];
+    }
     children_ok = true;
   };
   auto tree_levels_share = [&]() {
@@ -1657,12 +1701,12 @@ int frc_create(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
     const int TS = csr_chunks;
     // a leaf listed twice in a row only matters when values are used (presence is an OR)
     const bool check_dup = sh.need_val;
-    const int32_t* parent = tree->parent;
+    const int32_t* parent = tree0->parent;  // (checked against the caller's tree, staged with new_of_old ids)
     auto row_at = [&](int64_t target) {
       return static_cast<int64_t>(std::lower_bound(abnd->row_ptr, abnd->row_ptr + N, target) - abnd->row_ptr);
     };
     std::vector<int64_t>& stamp = c->stamps[t];
-    if (check_dup && static_cast<int32_t>(stamp.size()) < B) stamp.assign(B, -1);
+    if (check_dup && static_cast<int32_t>(stamp.size()) < B0) stamp.assign(B0, -1);
     for (int task = task_next.fetch_add(1, std::memory_order_relaxed); task < n_tasks;
          task = task_next.fetch_add(1, std::memory_order_relaxed)) {
       if (task == 0) { tree_levels_share(); continue; }
@@ -1684,10 +1728,10 @@ int frc_create(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
           const int32_t cc = abnd->col[k];
           const double v = abnd->val[k];
           const char* what = nullptr;
-          if (cc < 0 || cc >= B) what = "node id out of range";
+          if (cc < 0 || cc >= B0) what = "node id out of range";
           // pre-order ids: the first child of a node is the next id (the numbering itself is being
           // checked by another task at this moment; a bad tree fails the call before this result counts)
-          else if (cc + 1 < B && parent[cc + 1] == cc) what = "node is not a leaf";
+          else if (cc + 1 < B0 && parent[cc + 1] == cc) what = "node is not a leaf";
           else if (!(v > 0) || std::isinf(v)) what = "bad value";
           else if (check_dup && stamp[cc] == mark_s) what = "leaf listed twice";
           if (what) {
@@ -1697,12 +1741,13 @@ int frc_create(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
             break;
           }
           if (check_dup) stamp[cc] = mark_s;
+          const int32_t id = new_of_old ? new_of_old[cc] : cc;
 #if defined(__x86_64__)
           // streaming stores: the staging buffer is read next by the DMA engines, not by a core
-          _mm_stream_si32(dcol + k, cc);
+          _mm_stream_si32(dcol + k, id);
           if (dval) _mm_stream_si64(reinterpret_cast<long long*>(dval + k), static_cast<long long>(__builtin_bit_cast(int64_t, v)));
 #else
-          dcol[k] = cc;
+          dcol[k] = id;
           if (dval) dval[k] = v;
 #endif
         }
@@ -1727,11 +1772,15 @@ int frc_create(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
   mark("header checks, context, workers started");
 
   // ------------------------------------------------------------ (3) plan (the walks and the staging run in the pool)
+  // (refused on the caller's lengths; the sign test is on the lengths the kernels use)
   bool neg_len = false, bad_len = false;
+  for (int32_t v = 0; v < B0; ++v) {
+    const double l = tree0->length[v];
+    if (!(l == l) || std::isinf(l)) bad_len = true;
+  }
   for (int32_t v = 0; v < B; ++v) {
     const double l = tree->length[v];
-    if (!(l == l) || std::isinf(l)) bad_len = true;
-    else if (l < 0) neg_len = true;
+    if (l < 0 && !std::isinf(l)) neg_len = true;
   }
   auto plan_failed = [&](int code) { plan_ready.store(-1, std::memory_order_release); return bail(code); };
   if (!sh.exact && bad_len)

@@ -344,19 +344,26 @@ std::vector<uint8_t> operand_need_blocks(const std::vector<Tile>& tiles, int64_t
   return need;
 }
 
-TreeLevels tree_levels(const int32_t* parent, int32_t B, int32_t* lvl, int32_t* lpar) {
-  TreeLevels out;
+bool check_preorder(const int32_t* parent, int32_t B, int32_t* depth, int32_t* bad_parent, int32_t* bad_order) {
+  *bad_parent = 0; *bad_order = 0;
   // Branch-free per node (the stack-popping form cost 14 ns per node in mispredictions).
-  std::vector<int32_t> depth(B, 0), on_path(B + 1, 0), height(B, 0);  // on_path[d] = node at depth d of the current path
+  std::vector<int32_t> on_path(B + 1, 0);  // on_path[d] = node at depth d of the current path
+  depth[0] = 0;
   for (int32_t v = 1; v < B; ++v) {
     const int32_t p = parent[v];
-    if (p < 0 || p >= v) { out.bad_parent = v; return out; }
+    if (p < 0 || p >= v) { *bad_parent = v; return false; }
     const int32_t d = depth[p];
-    if ((d > depth[v - 1] || on_path[d] != p) && !out.bad_order) out.bad_order = v;
+    if ((d > depth[v - 1] || on_path[d] != p) && !*bad_order) *bad_order = v;
     depth[v] = d + 1;
     on_path[d + 1] = v;
   }
-  if (out.bad_order) return out;
+  return !*bad_order;
+}
+
+TreeLevels tree_levels(const int32_t* parent, int32_t B, int32_t* lvl, int32_t* lpar) {
+  TreeLevels out;
+  std::vector<int32_t> depth(B, 0), height(B, 0);
+  if (!check_preorder(parent, B, depth.data(), &out.bad_parent, &out.bad_order)) return out;
   for (int32_t v = B - 1; v >= 1; --v) height[parent[v]] = std::max(height[parent[v]], height[v] + 1);
   const int32_t H = height[0];
   out.level_ptr.assign(H + 2, 0);
@@ -392,6 +399,41 @@ void tree_post_order(const int32_t* parent, int32_t B, int32_t* post_order) {
   for (int32_t v = B - 1; v >= 1; --v) size[parent[v]] += size[v];
   for (int32_t v = 1; v < B; ++v) depth[v] = depth[parent[v]] + 1;
   for (int32_t v = 0; v < B; ++v) post_order[v + size[v] - 1 - depth[v]] = v;
+}
+
+PrunedTree prune_tree(const int32_t* parent, const double* length, int32_t B, const uint8_t* marks, bool merge) {
+  // keep: 0 = outside the support, 1 = survives, 2 = in the support but merged into the chain below it
+  std::vector<uint8_t> keep(B);
+  std::vector<int32_t> kids(B, 0);  // surviving children
+  for (int32_t v = 0; v < B; ++v) keep[v] = marks[v] ? 1 : 0;
+  if (B > 0) keep[0] = 1;
+  for (int32_t v = B - 1; v >= 1; --v)
+    if (keep[v]) { keep[parent[v]] = 1; kids[parent[v]]++; }
+  if (merge)
+    for (int32_t v = 1; v < B; ++v)
+      if (keep[v] && kids[v] == 1) keep[v] = 2;
+  // pre-order: a merged node's chain state (lengths summed from its top, node count, the survivor above the chain)
+  // is complete before its child is visited
+  PrunedTree t;
+  t.new_of_old.assign(B, -1);
+  std::vector<double> acc(merge ? B : 0);
+  std::vector<int32_t> cnt(merge ? B : 0), up(merge ? B : 0);
+  for (int32_t v = 0; v < B; ++v) {
+    if (!keep[v]) continue;
+    const int32_t p = v ? parent[v] : -1;
+    const bool chain = p >= 0 && keep[p] == 2;
+    if (keep[v] == 2) {
+      acc[v] = chain ? acc[p] + length[v] : length[v];
+      cnt[v] = (chain ? cnt[p] : 0) + 1;
+      up[v] = chain ? up[p] : p;
+      continue;
+    }
+    t.new_of_old[v] = t.n_nodes++;
+    t.parent.push_back(p < 0 ? -1 : t.new_of_old[chain ? up[p] : p]);
+    t.length.push_back(chain ? acc[p] + length[v] : length[v]);  // (verbatim unless merged)
+    t.mult.push_back((chain ? cnt[p] : 0) + 1);
+  }
+  return t;
 }
 
 }  // namespace frc
@@ -509,6 +551,20 @@ int32_t frc_debug_tree(const int32_t* parent, int32_t n_nodes, int32_t* level_no
   if (!frc::tree_children(parent, n_nodes, child_ptr, child_idx)) return -1;
   frc::tree_post_order(parent, n_nodes, post_order);
   return t.height;
+}
+
+// Pruned tree (prune_tree; marks[n_nodes] = 1 on the listed leaves): out_parent / out_length / out_mult hold n_nodes
+// entries (the pruned tree is never larger), new_of_old n_nodes.  Returns the pruned node count, or -1 - (offending
+// node) when parent[] is not a pre-order numbering (frc_create then prunes nothing).
+int32_t frc_debug_prune(const int32_t* parent, const double* length, int32_t n_nodes, const uint8_t* marks, int32_t merge,
+                        int32_t* out_parent, double* out_length, int32_t* out_mult, int32_t* new_of_old) {
+  std::vector<int32_t> depth(n_nodes);
+  int32_t bad_parent = 0, bad_order = 0;
+  if (!frc::check_preorder(parent, n_nodes, depth.data(), &bad_parent, &bad_order)) return -1 - (bad_parent ? bad_parent : bad_order);
+  const frc::PrunedTree t = frc::prune_tree(parent, length, n_nodes, marks, merge != 0);
+  for (int32_t v = 0; v < t.n_nodes; ++v) { out_parent[v] = t.parent[v]; out_length[v] = t.length[v]; out_mult[v] = t.mult[v]; }
+  for (int32_t v = 0; v < n_nodes; ++v) new_of_old[v] = t.new_of_old[v];
+  return t.n_nodes;
 }
 
 }  // extern "C"

@@ -99,13 +99,29 @@ struct TreeLevels {
   int32_t bad_parent = 0, bad_order = 0;  // first offending node ids
   std::vector<int32_t> level_ptr;  // [height + 2]
 };
-// Pre-order check (parent[v] must be the node of its depth on the current root-to-(v-1) path) and the
-// level order: level_nodes[B] grouped by height (leaves first), level_parent[k] = parent of level_nodes[k].
+// Pre-order check: parent[v] must be a smaller id (else *bad_parent = the first v that breaks it) and the node of its
+// depth on the current root-to-(v-1) path (else *bad_order = the first such v).  depth[n_nodes] receives the depths.
+bool check_preorder(const int32_t* parent, int32_t n_nodes, int32_t* depth, int32_t* bad_parent, int32_t* bad_order);
+// check_preorder, then the level order: level_nodes[B] grouped by height (leaves first), level_parent[k] = parent of
+// level_nodes[k].
 TreeLevels tree_levels(const int32_t* parent, int32_t n_nodes, int32_t* level_nodes, int32_t* level_parent);
 // Children lists in ascending id (= file order).  false when a parent id is out of range.
 bool tree_children(const int32_t* parent, int32_t n_nodes, int32_t* child_ptr, int32_t* child_idx);
 // post_order[k] = node visited k-th by abundanceToFlatNodes' recursion (children first, in file order,
 // then the node: unifrac.go:32-53).
 void tree_post_order(const int32_t* parent, int32_t n_nodes, int32_t* post_order);
+
+// FRC_FLAG_PRUNE (DESIGN.md, "Pruning to the table's support").  The support S is the root and every node with a
+// marked node in its subtree; the survivors keep their order, which is again a pre-order numbering.  With `merge`, a
+// non-root survivor with exactly one surviving child is dropped as well: the lowest node of such a chain takes the
+// parent above the chain, the chain's lengths summed top-down in fp64, and mult = the number of original nodes it
+// stands for (the mults add up to |S|).  parent[] must satisfy 0 <= parent[v] < v for v > 0 (check_preorder).
+struct PrunedTree {
+  int32_t n_nodes = 0;
+  std::vector<int32_t> parent, new_of_old;  // new_of_old[v] = id in the pruned tree, -1 if v was dropped
+  std::vector<double> length;
+  std::vector<int32_t> mult;
+};
+PrunedTree prune_tree(const int32_t* parent, const double* length, int32_t n_nodes, const uint8_t* marks, bool merge);
 
 }  // namespace frc

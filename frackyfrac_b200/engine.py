@@ -24,6 +24,7 @@ FLAG_UW_BF16 = 2
 FLAG_SHARD_EMBED = 4
 FLAG_UW_BITS = 8
 FLAG_L_TILES = 16  # normalize=0 (-l as coded) may run the key-matched FP32 tiles (within 1e-5, not bit-exact)
+FLAG_PRUNE = 32    # run on the subtree the table observes (exact path: the same bytes; fast paths: within 1e-5)
 COMM_ID_BYTES = 128
 
 NORM_L_AS_CODED, NORM_DEFAULT, NORM_L_DOCUMENTED = 0, 1, 2  # frc_opts_t.normalize

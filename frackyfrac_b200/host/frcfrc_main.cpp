@@ -139,6 +139,8 @@ int main(int argc, char** argv) {
     // -l as coded with FRCFRC_PATH=fast: the key-matched FP32 tiles (within 1e-5 of the reference, not bit-exact);
     // without FRCFRC_PATH, -l runs the bit-exact list walk
     if (fo.normalize == 0 && fo.path == FRC_PATH_FAST) fo.flags |= FRC_FLAG_L_TILES;
+    // FRCFRC_PRUNE=1: run on the subtree the table observes (a large reference tree, a small table)
+    if (const char* e = getenv("FRCFRC_PRUNE")) if (!strcmp(e, "1")) fo.flags |= FRC_FLAG_PRUNE;
     fo.device = -1;
     fo.world = 1;
     // every visible B200 works on the job; the engine hands their bands out as ONE ordered stream

@@ -117,6 +117,17 @@ typedef struct {
                                FRC_FLAG_SHARD_EMBED are supported; the capacity mode (panels sharded
                                over devices) is not: FRC_ERR_UNSUPPORTED where it would be chosen.  */
 
+#define FRC_FLAG_PRUNE 32u /* run on the subtree the table observes: the root and every node with a listed leaf
+                             below it (any row of col[], also rows another rank of a FRC_FLAG_SHARD_EMBED job
+                             stages).  The other nodes hold 0 in every sample and add nothing.  The fast paths
+                             also merge every unary chain that is left into its lowest node (lengths summed,
+                             the default normaliser counts the chain's nodes), so the kernels run over at most
+                             2 x (listed leaves) nodes instead of n_nodes.  Exact path: pruned, never merged,
+                             bit-identical to the unpruned run.  Fast paths: within 1e-5 of the reference, but
+                             not byte-identical to the unpruned run.  The path choice (AUTO), every error and
+                             its message (original node ids) are the same as without the flag;
+                             info.n_nodes_padded and info.tree_height describe the tree that ran (DESIGN.md). */
+
 typedef struct {
   int32_t mode;       /* frc_mode                                               */
   int32_t normalize;  /* flag -l (frcfrc.go:25):
