@@ -21,7 +21,7 @@ OUT = os.path.join(HERE, "_build")
 CSRC = os.path.join(HERE, "csrc")
 HOST = os.path.join(HERE, "host")
 
-CUDA_SOURCES = ["job.cu", "plan.cpp", "embed.cu", "exact.cu", "weighted.cu", "unweighted_tc.cu", "unweighted_bits.cu", "comm.cu", "wire.cu"]
+CUDA_SOURCES = ["job.cu", "plan.cpp", "embed.cu", "exact.cu", "weighted.cu", "unweighted_tc.cu", "comm.cu", "wire.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr", "-Xptxas", "-v",

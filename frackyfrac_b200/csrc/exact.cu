@@ -11,18 +11,10 @@
 // CPU fallback; it is selected for small problems (or on request) because it
 // does O(pairs * nodes) fp64 work without tensor cores.
 #include "frc_internal.h"
+#include "wire.cuh"
 
 namespace frc {
 namespace {
-
-__device__ __forceinline__ void pair_of(int64_t p, int64_t& i, int64_t& j) {
-  // largest i with i(i-1)/2 <= p
-  int64_t g = static_cast<int64_t>((1.0 + sqrt(1.0 + 8.0 * static_cast<double>(p))) * 0.5);
-  while (g * (g - 1) / 2 > p) --g;
-  while ((g + 1) * g / 2 <= p) ++g;
-  i = g;
-  j = p - g * (g - 1) / 2;
-}
 
 template <bool kWeighted>
 __global__ void k_exact_pairs(const double* __restrict__ E, const double* __restrict__ length,

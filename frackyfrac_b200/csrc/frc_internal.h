@@ -214,7 +214,9 @@ int launch_weighted_fixup(const DevCsr& a, const DevTree& t, const double* total
 void weighted_setup();  // cudaFuncSetAttribute calls for the CURRENT device (once per device context)
 
 // ---- unweighted_tc.cu -------------------------------------------------------
-struct TcOperands;  // opaque: tensor maps + chunk table
+// The unweighted pair stage has two operand feeds; the handle records which one a job uses, and the launches
+// below dispatch on it.
+struct TcOperands;  // opaque: operand feed, tensor maps, chunk table
 // Runs of 128-byte K blocks that accumulate uninterrupted in TMEM; device arrays.
 struct TcChunks {
   const int32_t* end = nullptr;
@@ -223,10 +225,17 @@ struct TcChunks {
   int32_t n = 0;
   bool biased = false;  // u8 fp64 mode: all scales within 2^8 -> single-instruction biased accumulation
 };
+// Materialised feed: the three K-major operands [np][kp] (bf16 or u8) in HBM.
 // flag_u: device scalar; pairs with unique length below it are recomputed exactly (null: none).
 TcOperands* tc_operands_create(const void* P, const void* Bh, const void* Bl, int64_t np, int32_t kp,
                                bool i8, const TcChunks& chunks, const double* len_col, const double* flag_u,
                                std::string* err);
+// Bits feed (u8 integer mode only): the u8 operand tiles are expanded inside the pair kernel from the bit rows
+// bitsS[np][kp / 32] and the per-column factors qa / qh / ql: no operand arrays in HBM.
+TcOperands* tc_operands_create_bits(const uint32_t* bitsS, int64_t np, int32_t kp, const uint8_t* qa,
+                                    const uint8_t* qh, const uint8_t* ql, const TcChunks& chunks,
+                                    const double* len_col, const double* flag_u, const long long* r_int,
+                                    double unit, std::string* err);
 // u8 integer mode (chunk scales within 2^16): row sums as integers in units of `unit` = the smallest scale.
 void tc_operands_set_int(TcOperands* o, const long long* r_int, double unit);
 void tc_operands_destroy(TcOperands* o);
@@ -234,30 +243,14 @@ int tc_chunk_kblocks();  // bf16: K blocks per fp32 accumulation run (FRC_TC_CHU
 // Distances of the tiles in `tiles` into out[index - first]; the band offset of
 // every pair with d < flag_below is appended to flagged[] (count in *n_flagged;
 // capacity = pairs of the band, so it cannot overflow) for the fix-up pass.
+// Integer mode (either feed) flags by flag_u alone; the bits feed does not read r or flag_below.
 int launch_unweighted_tc(const TcOperands* ops, const double* r, const Tile* tiles, int32_t n_tiles,
                          int64_t n_samples, int64_t first, float* out, double flag_below,
                          uint32_t* flagged, unsigned long long* n_flagged, int num_sms, cudaStream_t s);
-// fp64 recompute of the flagged pairs from the presence rows and true lengths.
+// fp64 recompute of the flagged pairs from the feed's presence rows and true lengths.
 int launch_unweighted_fixup(const TcOperands* ops, const uint32_t* flagged,
                             const unsigned long long* n_flagged, unsigned long long* count_host,
                             int64_t first, float* out, const Exceptions& ex, int num_sms, cudaStream_t s);
 bool tc_setup(std::string* err);  // driver entry point (once per process) + smem attributes for the CURRENT device
-
-// ---- unweighted_bits.cu -----------------------------------------------------
-// The same pair tiles with the u8 operand tiles expanded inside the kernel from the bit rows
-// bitsS[np][kp / 32] (integer mode only): no operand arrays in HBM.
-struct BitsOperands;
-BitsOperands* bits_operands_create(const uint32_t* bitsS, int64_t np, int32_t kp, const uint8_t* qa,
-                                   const uint8_t* qh, const uint8_t* ql, const TcChunks& chunks,
-                                   const double* len_col, const double* flag_u, const long long* r_int,
-                                   double unit, std::string* err);
-void bits_operands_destroy(BitsOperands* o);
-int launch_unweighted_bits(const BitsOperands* ops, const Tile* tiles, int32_t n_tiles, int64_t n_samples,
-                           int64_t first, float* out, uint32_t* flagged, unsigned long long* n_flagged,
-                           int num_sms, cudaStream_t s);
-int launch_unweighted_fixup_bits(const BitsOperands* ops, const uint32_t* flagged, const unsigned long long* n_flagged,
-                                 unsigned long long* count_host, int64_t first, float* out, const Exceptions& ex,
-                                 int num_sms, cudaStream_t s);
-bool bits_setup(std::string* err);  // as tc_setup, for the bits-fed kernel
 
 }  // namespace frc

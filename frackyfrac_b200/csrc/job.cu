@@ -290,7 +290,6 @@ struct Part {
   int32_t *d_order = nullptr, *d_col_exp = nullptr;
   uint32_t* d_qam = nullptr;
   uint32_t* d_bitsS = nullptr;
-  BitsOperands* bo = nullptr;
   long long* d_r_int = nullptr;
   long long* d_fix_ws[2] = {nullptr, nullptr};  // weighted fix-up: one zeroed int64[B] per CTA, per compute stream
   uint8_t* d_need = nullptr;
@@ -725,12 +724,6 @@ int enqueue_band(Part* p, size_t idx) {
       launches += launch_weighted_fixup(p->dcsr, p->dtree, sh.opts.normalize == 1 ? p->d_total : nullptr, p->d_W,
                                         sl.flagged, cnt, sl.n_flagged_host, b.first, p->d_fix_ws[si], kFixupCtas,
                                         sl.dev32, sl.ex, s, p->d_K, sh.kp);
-    } else if (sh.bits_feed) {
-      launches += launch_unweighted_bits(p->bo, p->d_tiles + b.tile_off, b.n_tiles, sh.N, b.first, sl.dev32,
-                                         sl.flagged, cnt, dc->num_sms, s);
-      PART_CUDA(p, cudaEventRecord(sl.k1, s));
-      launches += launch_unweighted_fixup_bits(p->bo, sl.flagged, cnt, sl.n_flagged_host, b.first, sl.dev32, sl.ex,
-                                               dc->num_sms, s);
     } else {
       launches += launch_unweighted_tc(p->tc, p->d_r, p->d_tiles + b.tile_off, b.n_tiles, sh.N, b.first, sl.dev32,
                                        kFlagBelow, sl.flagged, cnt, dc->num_sms, s);
@@ -864,7 +857,6 @@ void destroy_part(Part* p) {
   for (cudaEvent_t e : p->ev_used) if (e) cudaEventDestroy(e);
   for (auto& cb : p->cap) if (cb.done) cudaEventDestroy(cb.done);
   tc_operands_destroy(p->tc);
-  bits_operands_destroy(p->bo);
   if (p->dc) {
     p->dc->dev.reset();
     p->dc->pin.reset();
@@ -920,7 +912,7 @@ int make_dev_ctx(int device, DevCtx** out) {
     }
   // function attributes live in the device's context: once per device, not once per process
   std::string terr;
-  if (!tc_setup(&terr) || !bits_setup(&terr)) { g_create_error = terr; return FRC_ERR_CUDA; }
+  if (!tc_setup(&terr)) { g_create_error = terr; return FRC_ERR_CUDA; }
   weighted_setup();
   embed_setup();
   if ((e = cudaGetLastError()) != cudaSuccess) {
@@ -1438,16 +1430,16 @@ int prepare_part(Part* p) {
     if (i8 && !(p->d_qam = dev_alloc<uint32_t>(p, sh.kp))) return p->rc;
     if (intacc && !(p->d_r_int = dev_alloc<long long>(p, sh.np))) return p->rc;
     std::string terr;
-    if (!sh.bits_feed) {
-      p->tc = tc_operands_create(p->d_P, p->d_Bh, p->d_Bl, sh.np, sh.kp, i8, p->d_chunks, p->d_len_col, p->d_flag_u, &terr);
-      if (!p->tc) return pfail(p, FRC_ERR_CUDA, terr);
-      if (intacc) tc_operands_set_int(p->tc, p->d_r_int, std::ldexp(1.0, sh.cols.e_min));
+    if (sh.bits_feed) {
+      p->tc = tc_operands_create_bits(p->d_bitsS, sh.np, sh.kp, static_cast<const uint8_t*>(p->d_q0),
+                                      static_cast<const uint8_t*>(p->d_q1), static_cast<const uint8_t*>(p->d_q2),
+                                      p->d_chunks, p->d_len_col, p->d_flag_u, p->d_r_int,
+                                      std::ldexp(1.0, sh.cols.e_min), &terr);
     } else {
-      p->bo = bits_operands_create(p->d_bitsS, sh.np, sh.kp, static_cast<const uint8_t*>(p->d_q0),
-                                   static_cast<const uint8_t*>(p->d_q1), static_cast<const uint8_t*>(p->d_q2),
-                                   p->d_chunks, p->d_len_col, p->d_flag_u, p->d_r_int, std::ldexp(1.0, sh.cols.e_min), &terr);
-      if (!p->bo) return pfail(p, FRC_ERR_CUDA, terr);
+      p->tc = tc_operands_create(p->d_P, p->d_Bh, p->d_Bl, sh.np, sh.kp, i8, p->d_chunks, p->d_len_col, p->d_flag_u, &terr);
+      if (p->tc && intacc) tc_operands_set_int(p->tc, p->d_r_int, std::ldexp(1.0, sh.cols.e_min));
     }
+    if (!p->tc) return pfail(p, FRC_ERR_CUDA, terr);
     if (i8) {  // a function of the tree only: once per job, not per restart
       p->info.kernel_launches += launch_quantize_lengths(
           p->d_len_col, p->d_col_exp, sh.kp, static_cast<uint8_t*>(p->d_q0), static_cast<uint8_t*>(p->d_q1),

@@ -9,7 +9,8 @@
 //     d(i,j)      = unique / (unique + shared) = (R - 2s) / (R - s),  R = r_i + r_j
 // so the pairwise part is the dense contraction S = P diag(len) P^T: a GEMM.
 //
-// Kernels in this file (DESIGN.md, "Pair stage, unweighted"):
+// Kernels in this file (DESIGN.md, "Pair stage, unweighted"), two operand feeds of one pair stage
+// (TcOperands says which):
 //   k_unweighted_tc2<2>  default.  CTA pairs (cta_group::2), u8 block-floating-point operands
 //                        (len ~= a * m * 2^e), tcgen05 kind::i8 M256 x N256 x K32, exact int32
 //                        accumulation in TMEM, 64-bit integer chunk accumulation and an integer / fp32
@@ -18,7 +19,10 @@
 //                        scales span more than 2^16.
 //   k_unweighted_tc2<0>  bf16 operands (P exact, len = hi + lo planes), kind::f16 K16, fp32
 //                        accumulators restarted every K-chunk (FRC_FLAG_UW_BF16; negative lengths).
-//   k_unweighted_fixup   exact fp64 recompute of the pairs the epilogues flag.
+//   k_unweighted_bits2   the integer mode of k_unweighted_tc2<2> with the u8 operand tiles expanded
+//                        inside the kernel from the presence bits (capacity mode, FRC_FLAG_UW_BITS):
+//                        no operand arrays in HBM.
+//   k_unweighted_fixup   exact fp64 recompute of the pairs the epilogues flag, from either feed's rows.
 //
 // bf16: why two accumulator halves and K-chunks: the tensor core's fp32 accumulate
 // loses the addend bits below the accumulator's ulp (measured: a bias, not
@@ -98,8 +102,10 @@ constexpr int BKB = 128;  // bytes of K per block and operand row
 // ratio epilogue + stores, [7] its total.
 // Built only with -DFRC_TC_TIMELINE (scripts/exp_timeline.py); FRC_TC_DEBUG then also accepts
 // 1 = do not load B, 2 = do not load A, 4 = no ratio epilogue (timing attribution; garbage results).
+// k_unweighted_bits2 accumulates its own counters into g_bits_dbg (scripts/exp_bits_timeline.py).
 #ifdef FRC_TC_TIMELINE
 __device__ unsigned long long g_tc_dbg[512 * 8];
+__device__ unsigned long long g_bits_dbg[512 * 8];
 #define TL(x) x
 #define TL_ON(mask) ((dbg & (mask)) != 0)
 #else
@@ -109,6 +115,74 @@ __device__ unsigned long long g_tc_dbg[512 * 8];
 constexpr int EPI2_WARPS = 16;
 constexpr int EPI2_COLS = 128 / (EPI2_WARPS / 4);  // accumulator columns per thread and plane
 constexpr int THREADS2 = 32 * (EPI_WARP0 + EPI2_WARPS);
+
+// ---- integer-mode epilogue, shared by k_unweighted_tc2<2> and k_unweighted_bits2
+// One chunk's accumulators into acc: exact 64-bit accumulation in units of the smallest chunk scale, two
+// 32x32+64 integer multiply-adds per element, (256*hi + lo) << shift with shift <= 16 (host-checked range).
+// taddr is this thread's first hi-plane column; the lo plane is BN columns on.  Two register sets: the
+// tcgen05.ld of batch c+1 is in flight while batch c is folded in.
+__device__ __forceinline__ void drain_int(uint32_t taddr, uint32_t shift, unsigned long long (&acc)[EPI2_COLS]) {
+  const uint32_t m0 = 1u << shift, m1 = 256u << shift;
+  uint32_t v[2][8], w[2][8];
+  ptx::tmem_ld_32x8(taddr, v[0]);
+  ptx::tmem_ld_32x8(taddr + BN, w[0]);
+#pragma unroll
+  for (int cc = 0; cc < EPI2_COLS / 8; ++cc) {
+    ptx::tmem_ld_wait();
+    if (cc + 1 < EPI2_COLS / 8) {
+      ptx::tmem_ld_32x8(taddr + (cc + 1) * 8, v[(cc + 1) & 1]);
+      ptx::tmem_ld_32x8(taddr + BN + (cc + 1) * 8, w[(cc + 1) & 1]);
+    }
+#pragma unroll
+    for (int x = 0; x < 8; ++x)
+      acc[cc * 8 + x] += static_cast<unsigned long long>(v[cc & 1][x]) * m1 +
+                         static_cast<unsigned long long>(w[cc & 1][x]) * m0;
+  }
+}
+
+// The exact ratios of column sample j (this thread's TMEM lane) and row samples i0 + [0, EPI2_COLS) (its
+// registers), stored from out[off] on (off: band offset of (i0, j)); pairs with U below flag_u_int are flagged.
+__device__ __forceinline__ void ratio_int(const unsigned long long (&acc)[EPI2_COLS], const long long* __restrict__ r_int,
+                                          int64_t i0, int64_t j, int lane, int64_t n_samples, int64_t off,
+                                          long long flag_u_int, float* __restrict__ out, uint32_t* __restrict__ flagged,
+                                          unsigned long long* __restrict__ n_flagged) {
+  const long long rj = j < n_samples ? r_int[j] : 0;
+  const long long ri_lane = r_int[i0 + lane];
+#pragma unroll
+  for (int n0 = 0; n0 < EPI2_COLS; n0 += 8) {
+    float dv[8];
+    bool fu[8];
+#pragma unroll
+    for (int x = 0; x < 8; ++x) {
+      const long long ri = __shfl_sync(0xffffffffu, ri_lane, n0 + x);
+      const long long sh = static_cast<long long>(acc[n0 + x]);
+      // exact: U = (r_i - s) + (r_j - s) >= 0 (the reference's `result`), V = U + common
+      const unsigned long long U = static_cast<unsigned long long>(ri + rj - 2 * sh);
+      const unsigned long long V = U + static_cast<unsigned long long>(sh);
+      const float Uf = fmaf(__uint2float_rn(static_cast<uint32_t>(U >> 32)), 4294967296.f,
+                            __uint2float_rn(static_cast<uint32_t>(U)));
+      const float Vf = fmaf(__uint2float_rn(static_cast<uint32_t>(V >> 32)), 4294967296.f,
+                            __uint2float_rn(static_cast<uint32_t>(V)));
+      dv[x] = __fdividef(Uf, Vf);  // unifrac.go:169; 0/0 -> NaN (A8)
+      fu[x] = static_cast<long long>(U) < flag_u_int;
+    }
+#pragma unroll
+    for (int x = 0; x < 8; ++x) {
+      const int64_t i = i0 + n0 + x;
+      if (i < n_samples && j < i) {
+        out[off] = dv[x];  // fp32 is what the ratio is; the host widens (wire.cu)
+        // U and V are exact integer sums of the quantised lengths: no cancellation error, so a small d
+        // needs no recompute here (identical samples give U = 0 exactly); only the absolute-error rule of
+        // the merged small-length columns applies
+        if (fu[x]) {
+          unsigned long long slot = atomicAdd(n_flagged, 1ULL);
+          flagged[slot] = static_cast<uint32_t>(off);
+        }
+      }
+      off += i;  // row i+1 starts i entries later
+    }
+  }
+}
 
 // kMode: 0 = bf16 planes (fp32 accumulators), 1 = u8 planes with fp64 chunk accumulation (chunk scales
 // spanning more than 2^16), 2 = u8 planes with 64-bit INTEGER accumulation and an integer / fp32 ratio
@@ -274,24 +348,7 @@ k_unweighted_tc2(const __grid_constant__ CUtensorMap mapP, const __grid_constant
         ptx::tc_fence_after();
         const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + buf * DN + cg * EPI2_COLS;
         if constexpr (kInt) {
-          // exact 64-bit accumulation in units of the smallest chunk scale: two 32x32+64 integer
-          // multiply-adds per element, (256*hi + lo) << shift with shift <= 16 (host-checked range)
-          const uint32_t m0 = 1u << shift, m1 = 256u << shift;
-          uint32_t v[2][8], w[2][8];
-          ptx::tmem_ld_32x8(taddr, v[0]);
-          ptx::tmem_ld_32x8(taddr + BN, w[0]);
-#pragma unroll
-          for (int cc = 0; cc < EPI2_COLS / 8; ++cc) {
-            ptx::tmem_ld_wait();
-            if (cc + 1 < EPI2_COLS / 8) {
-              ptx::tmem_ld_32x8(taddr + (cc + 1) * 8, v[(cc + 1) & 1]);
-              ptx::tmem_ld_32x8(taddr + BN + (cc + 1) * 8, w[(cc + 1) & 1]);
-            }
-#pragma unroll
-            for (int x = 0; x < 8; ++x)
-              acc[cc * 8 + x] += static_cast<unsigned long long>(v[cc & 1][x]) * m1 +
-                                 static_cast<unsigned long long>(w[cc & 1][x]) * m0;
-          }
+          drain_int(taddr, shift, acc);
         } else if constexpr (kI8) {
           // both plane sums are in [0, 2^31): S = 256*hi + lo < 2^40 comes from one 32x32->64 integer
           // multiply-add; OR-ing it into the mantissa of 2^52 gives the double 2^52 + S without any
@@ -352,42 +409,7 @@ k_unweighted_tc2(const __grid_constant__ CUtensorMap mapP, const __grid_constant
         // Batches of 8 row samples: first the arithmetic of all 8 (independent chains the scheduler can
         // interleave), then the stores and the (rare) fix-up flags.
         if constexpr (kInt) {
-          const long long rj = j < n_samples ? r_int[j] : 0;
-          const long long ri_lane = r_int[i0 + lane];
-#pragma unroll
-          for (int n0 = 0; n0 < EPI2_COLS; n0 += 8) {
-            float dv[8];
-            bool fu[8];
-#pragma unroll
-            for (int x = 0; x < 8; ++x) {
-              const long long ri = __shfl_sync(0xffffffffu, ri_lane, n0 + x);
-              const long long sh = static_cast<long long>(acc[n0 + x]);
-              // exact: U = (r_i - s) + (r_j - s) >= 0 (the reference's `result`), V = U + common
-              const unsigned long long U = static_cast<unsigned long long>(ri + rj - 2 * sh);
-              const unsigned long long V = U + static_cast<unsigned long long>(sh);
-              const float Uf = fmaf(__uint2float_rn(static_cast<uint32_t>(U >> 32)), 4294967296.f,
-                                    __uint2float_rn(static_cast<uint32_t>(U)));
-              const float Vf = fmaf(__uint2float_rn(static_cast<uint32_t>(V >> 32)), 4294967296.f,
-                                    __uint2float_rn(static_cast<uint32_t>(V)));
-              dv[x] = __fdividef(Uf, Vf);  // unifrac.go:169; 0/0 -> NaN (A8)
-              fu[x] = static_cast<long long>(U) < flag_u_int;
-            }
-#pragma unroll
-            for (int x = 0; x < 8; ++x) {
-              const int64_t i = i0 + n0 + x;
-              if (i < n_samples && j < i) {
-                out[off] = dv[x];  // fp32 is what the ratio is; the host widens (wire.cu)
-                // U and V are exact integer sums of the quantised lengths: no cancellation error, so a
-                // small d needs no recompute here (identical samples give U = 0 exactly); only the
-                // absolute-error rule of the merged small-length columns applies
-                if (fu[x]) {
-                  unsigned long long slot = atomicAdd(n_flagged, 1ULL);
-                  flagged[slot] = static_cast<uint32_t>(off);
-                }
-              }
-              off += i;  // row i+1 starts i entries later
-            }
-          }
+          ratio_int(acc, r_int, i0, j, lane, n_samples, off, flag_u_int, out, flagged, n_flagged);
         } else {
           const double rj = j < n_samples ? r[j] : 0.0;
           const double ri_lane = r[i0 + lane];
@@ -436,49 +458,331 @@ k_unweighted_tc2(const __grid_constant__ CUtensorMap mapP, const __grid_constant
   }
 }
 
-// Exact recompute of flagged pairs from the presence rows of the A operand (bf16 P, or u8
-// P*a which is non-zero exactly where the node is present and has a non-zero length): one
-// warp per pair, fp64, TRUE branch lengths (len_col[k] = length of the node in operand column
-// k, 0 in padding columns).  Identical samples give exactly 0.
-template <bool kI8>
+// ----------------------------------------------------------------------------
+// Bits feed (capacity mode): the CTA-pair kind::i8 GEMM and integer epilogue of k_unweighted_tc2<2>, but the
+// u8 operand tiles are never materialised in HBM.  Producer warps expand them straight into the 128-byte
+// swizzled shared-memory layout the MMA reads (the same A and B stage tiles of 128 rows x BKB bytes):
+//     A[j][k]  = bit(j, k) ? qa[k] : 0      (this CTA's 128 column samples)
+//     B[i][k]  = bit(i, k) ? qh[k] | ql[k]  (the 128 row samples; leader: high plane, peer: low plane)
+// from sample-major bit rows bitsS[np][kp / 8] (1 bit per (sample, operand column); column k is bit
+// k % 8 of byte k / 8) and the per-column quantised factors.  Per 128-column K block a CTA reads
+// 4 KB of bits + 256 B of factors instead of 32 KB of operand bytes: the operand expansion kernel,
+// its HBM traffic (3 bytes per (sample, column): 60 GB at cfg4) and the per-rank expansion of every
+// sample in a multi-GPU run disappear.
+//
+// Warps: 0 = TMA loader of bit tiles, 1 = MMA issuer, 4..11 = producers (expansion), 12..27 =
+// epilogue.  Registers move from the control / producer warp groups to the epilogue ones
+// (setmaxnreg), which keep the 96 they have in k_unweighted_tc2.
+namespace bits {
+constexpr int OSTAGES = 5;                     // operand ring (written by the producers)
+constexpr int OSTAGE_BYTES = A_BYTES + B_BYTES;
+constexpr int BSTAGES = 8;                     // bit-tile ring (written by TMA)
+constexpr int BITS_TILE = 128 * 16;            // 128 samples x 128 columns / 8
+constexpr int BSTAGE_BYTES = 2 * BITS_TILE + 2 * BKB;  // A bits, B bits, qa, q(h|l)
+constexpr int NUM_BARS = 3 * OSTAGES + 2 * BSTAGES + 4;
+constexpr int SMEM_BYTES = OSTAGES * OSTAGE_BYTES + BSTAGES * BSTAGE_BYTES + NUM_BARS * 8 + 16 + 1024;
+constexpr int PROD_WARP0 = 4, PROD_WARPS = 8;
+constexpr int EPI_WARP0 = 12;                  // EPI2_WARPS epilogue warps, as in k_unweighted_tc2
+constexpr int THREADS = 32 * (EPI_WARP0 + EPI2_WARPS);  // 896
+
+// 4 bits (b0..b3 of `nib`, other bits must be zero) -> byte masks 0xFF / 0x00: one multiply puts bit g
+// into the sign of byte g, one PRMT replicates the signs.
+__device__ __forceinline__ uint32_t mask4(uint32_t nib) {
+  uint32_t m;
+  asm("prmt.b32 %0, %1, 0, 0xBA98;" : "=r"(m) : "r"(nib * 0x10204080u));
+  return m;
+}
+}  // namespace bits
+
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(bits::THREADS, 1)
+k_unweighted_bits2(const __grid_constant__ CUtensorMap mapBits, const uint8_t* __restrict__ qa,
+                   const uint8_t* __restrict__ qh, const uint8_t* __restrict__ ql,
+                   const int32_t* __restrict__ chunk_end, const int32_t* __restrict__ chunk_shift,
+                   int32_t n_chunks, const long long* __restrict__ r_int, double unit,
+                   const Tile* __restrict__ tiles, int32_t n_tiles, int64_t n_samples, int64_t first,
+                   float* __restrict__ out, const double* __restrict__ flag_u_ptr,
+                   uint32_t* __restrict__ flagged, unsigned long long* __restrict__ n_flagged) {
+  using namespace bits;  // (EPI_WARP0 is written bits::EPI_WARP0: k_unweighted_tc2 has its own)
+  extern __shared__ uint8_t smem_raw[];
+  const uint32_t raw = ptx::smem_u32(smem_raw);
+  const uint32_t pad = ((raw + 1023u) & ~1023u) - raw;
+  uint8_t* smem = smem_raw + pad;
+  const uint32_t smem_base = raw + pad;                               // operand ring (1024-aligned)
+  const uint32_t bits_base = smem_base + OSTAGES * OSTAGE_BYTES;      // bit-tile ring
+  const uint32_t bar_base = bits_base + BSTAGES * BSTAGE_BYTES;
+  auto ofull_bar = [&](int s) { return bar_base + 8u * s; };
+  auto oempty_bar = [&](int s) { return bar_base + 8u * (OSTAGES + s); };
+  auto bfull_bar = [&](int s) { return bar_base + 8u * (2 * OSTAGES + s); };
+  auto bempty_bar = [&](int s) { return bar_base + 8u * (2 * OSTAGES + BSTAGES + s); };
+  auto tfull_bar = [&](int b) { return bar_base + 8u * (2 * OSTAGES + 2 * BSTAGES + b); };
+  auto tempty_bar = [&](int b) { return bar_base + 8u * (2 * OSTAGES + 2 * BSTAGES + 2 + b); };
+  // peer CTA only: its producer warps arrive here (CTA scope); one forwarder thread then tells the leader
+  auto pfull_bar = [&](int s) { return bar_base + 8u * (2 * OSTAGES + 2 * BSTAGES + 4 + s); };
+  volatile uint32_t* tmem_slot = reinterpret_cast<volatile uint32_t*>(
+      smem + OSTAGES * OSTAGE_BYTES + BSTAGES * BSTAGE_BYTES + NUM_BARS * 8);
+
+  const int warp = threadIdx.x >> 5;
+  const int lane = threadIdx.x & 31;
+  const uint32_t cta = ptx::cluster_ctarank();  // 0 = leader
+  const int pair = blockIdx.x >> 1;
+  const int n_pairs = gridDim.x >> 1;
+
+  if (warp == 0 && lane == 0) {
+    ptx::prefetch_tensormap(&mapBits);
+    for (int s = 0; s < OSTAGES; ++s) {
+      ptx::mbar_init(ofull_bar(s), PROD_WARPS + 1);  // leader: its producer warps + the peer's forwarder
+      ptx::mbar_init(oempty_bar(s), 1);              // multicast tcgen05.commit
+      ptx::mbar_init(pfull_bar(s), PROD_WARPS);
+    }
+    for (int s = 0; s < BSTAGES; ++s) {
+      ptx::mbar_init(bfull_bar(s), 1);
+      ptx::mbar_init(bempty_bar(s), PROD_WARPS);
+    }
+    for (int b = 0; b < 2; ++b) {
+      ptx::mbar_init(tfull_bar(b), 1);
+      ptx::mbar_init(tempty_bar(b), 2 * EPI2_WARPS);
+    }
+    ptx::fence_barrier_init();
+    ptx::fence_proxy_async();
+  }
+  if (warp == 1) {
+    ptx::tmem_alloc<2>(ptx::smem_u32(const_cast<uint32_t*>(tmem_slot)), TMEM_COLS);
+    ptx::tmem_relinquish<2>();
+  }
+  ptx::tc_fence_before();
+  ptx::cluster_sync_all();
+  ptx::tc_fence_after();
+  const uint32_t tmem_base = *tmem_slot;
+  const int n_kblocks = chunk_end[n_chunks - 1];
+
+  if (warp == 0) {
+    ptx::setmaxnreg_dec<24>();
+    // ------------------------------------------------ TMA loader: bit tiles + factors of each K block
+    if (lane == 0) {
+      int stage = 0;
+      uint32_t phase = 0;
+      const uint8_t* qb = cta == 0 ? qh : ql;
+      for (int t = pair; t < n_tiles; t += n_pairs) {
+        const Tile tile = tiles[t];
+        const int row_a = (tile.tj + static_cast<int>(cta)) * BM, row_b = tile.ti * BN;
+        for (int kb = 0; kb < n_kblocks; ++kb) {
+          TL(const long long c0 = clock64();)
+          ptx::mbar_wait(bempty_bar(stage), phase ^ 1u);
+          TL(g_bits_dbg[blockIdx.x * 8 + 0] += clock64() - c0;)
+          const uint32_t sb = bits_base + stage * BSTAGE_BYTES;
+          ptx::mbar_expect_tx(bfull_bar(stage), BSTAGE_BYTES);
+          ptx::tma_load_2d(sb, &mapBits, bfull_bar(stage), kb * 16, row_a);
+          ptx::tma_load_2d(sb + BITS_TILE, &mapBits, bfull_bar(stage), kb * 16, row_b);
+          ptx::bulk_load_1d(sb + 2 * BITS_TILE, qa + static_cast<int64_t>(kb) * BKB, BKB, bfull_bar(stage));
+          ptx::bulk_load_1d(sb + 2 * BITS_TILE + BKB, qb + static_cast<int64_t>(kb) * BKB, BKB, bfull_bar(stage));
+          if (++stage == BSTAGES) { stage = 0; phase ^= 1u; }
+        }
+      }
+    }
+    __syncwarp();
+  } else if (warp == 1) {
+    ptx::setmaxnreg_dec<24>();
+    // -------------------------------------------------- MMA issuer (leader only)
+    if (lane == 0 && cta == 0) {
+      constexpr uint32_t idesc = ptx::umma_idesc_u8(2 * BM, DN);
+      int stage = 0;
+      uint32_t phase = 0;
+      uint32_t chunk = 0;
+      for (int t = pair; t < n_tiles; t += n_pairs) {
+        int kb = 0;
+        for (int ch = 0; ch < n_chunks; ++ch, ++chunk) {
+          const uint32_t buf = chunk & 1u;
+          TL(const long long c0 = clock64();)
+          ptx::mbar_wait(tempty_bar(buf), ((chunk >> 1) & 1u) ^ 1u);
+          TL(g_bits_dbg[blockIdx.x * 8 + 1] += clock64() - c0;)
+          ptx::tc_fence_after();
+          const uint32_t d_tmem = tmem_base + buf * DN;
+          const int kb_begin = kb, kb_end = chunk_end[ch];
+          for (; kb < kb_end; ++kb) {
+            TL(const long long c1 = clock64();)
+            ptx::mbar_wait(ofull_bar(stage), phase);
+            TL(g_bits_dbg[blockIdx.x * 8 + 2] += clock64() - c1;)
+            ptx::tc_fence_after();
+            const uint32_t sa = smem_base + stage * OSTAGE_BYTES;
+            const uint64_t da = ptx::umma_desc_k_sw128(sa);
+            const uint64_t db = ptx::umma_desc_k_sw128(sa + A_BYTES);
+#pragma unroll
+            for (int k = 0; k < 4; ++k)
+              ptx::umma_i8<2>(d_tmem, da + 2u * k, db + 2u * k, idesc, (kb > kb_begin || k > 0) ? 1u : 0u);
+            ptx::umma_commit_2sm(oempty_bar(stage), 3);
+            if (++stage == OSTAGES) { stage = 0; phase ^= 1u; }
+          }
+          ptx::umma_commit_2sm(tfull_bar(buf), 3);
+        }
+      }
+    }
+    __syncwarp();
+  } else if (warp < PROD_WARP0) {
+    ptx::setmaxnreg_dec<24>();
+    // warp 2 of the PEER forwards "my half of the stage is written" to the leader: one cluster-scope
+    // release per K block instead of one per producer warp (a remote arrive with release.cluster
+    // semantics costs ~1 us; eight of them per K block made the producers 4x too slow)
+    if (warp == 2 && cta == 1 && lane == 0) {
+      int stage = 0;
+      uint32_t phase = 0;
+      for (int t = pair; t < n_tiles; t += n_pairs)
+        for (int kb = 0; kb < n_kblocks; ++kb) {
+          ptx::mbar_wait(pfull_bar(stage), phase);
+          ptx::mbar_arrive_cluster_relaxed(ofull_bar(stage), 0);
+          if (++stage == OSTAGES) { stage = 0; phase ^= 1u; }
+        }
+    }
+    __syncwarp();
+  } else if (warp < PROD_WARP0 + PROD_WARPS) {
+    ptx::setmaxnreg_dec<48>();
+    // ---------------------------------------------------------------- producers
+    // thread -> 16-byte chunk c of the K block (16 columns) and rows base, base + 32, ... of both tiles
+    const int pt = threadIdx.x - PROD_WARP0 * 32;  // 0..255
+    const int c = pt & 7;
+    const int rbase = pt >> 3;                     // 0..31
+    int ostage = 0, bstage = 0;
+    uint32_t ophase = 0, bphase = 0;
+    for (int t = pair; t < n_tiles; t += n_pairs) {
+      for (int kb = 0; kb < n_kblocks; ++kb) {
+        TL(const long long c0 = clock64();)
+        ptx::mbar_wait(bfull_bar(bstage), bphase);
+        TL(const long long c1 = clock64();)
+        ptx::mbar_wait(oempty_bar(ostage), ophase ^ 1u);
+        TL(const long long c2 = clock64();)
+        const uint8_t* sb = smem + OSTAGES * OSTAGE_BYTES + bstage * BSTAGE_BYTES;
+        uint8_t* so = smem + ostage * OSTAGE_BYTES;
+        const uint4 qA = *reinterpret_cast<const uint4*>(sb + 2 * BITS_TILE + c * 16);
+        const uint4 qB = *reinterpret_cast<const uint4*>(sb + 2 * BITS_TILE + BKB + c * 16);
+#pragma unroll
+        for (int tile_sel = 0; tile_sel < 2; ++tile_sel) {
+          const uint4 q = tile_sel == 0 ? qA : qB;
+          const uint8_t* tile_bits = sb + tile_sel * BITS_TILE;
+          uint8_t* dst = so + tile_sel * A_BYTES;
+#pragma unroll
+          for (int m = 0; m < 4; ++m) {
+            const int r = rbase + 32 * m;
+            const uint32_t b16 = *reinterpret_cast<const uint16_t*>(tile_bits + r * 16 + c * 2);
+            const uint32_t lo8 = b16 & 0xFFu, hi8 = b16 >> 8;
+            uint4 v;
+            v.x = q.x & mask4(lo8 & 0xFu);
+            v.y = q.y & mask4(lo8 >> 4);
+            v.z = q.z & mask4(hi8 & 0xFu);
+            v.w = q.w & mask4(hi8 >> 4);
+            // SWIZZLE_128B K-major: row r at (r / 8) * 1024 + (r % 8) * 128, 16-byte chunk c at c ^ (r % 8)
+            *reinterpret_cast<uint4*>(dst + (r >> 3) * 1024 + (r & 7) * 128 + ((c ^ (r & 7)) << 4)) = v;
+          }
+        }
+        ptx::fence_proxy_async();  // generic-proxy stores -> visible to the tensor core's async proxy
+        __syncwarp();
+        if (lane == 0) {
+          ptx::mbar_arrive(cta == 0 ? ofull_bar(ostage) : pfull_bar(ostage));
+          ptx::mbar_arrive(bempty_bar(bstage));
+        }
+        TL(if (pt == 0) {
+          g_bits_dbg[blockIdx.x * 8 + 3] += c1 - c0;             // waiting for bits
+          g_bits_dbg[blockIdx.x * 8 + 4] += c2 - c1;             // waiting for a free operand stage
+          g_bits_dbg[blockIdx.x * 8 + 5] += clock64() - c2;      // expanding + fence + arrive
+        })
+        if (++ostage == OSTAGES) { ostage = 0; ophase ^= 1u; }
+        if (++bstage == BSTAGES) { bstage = 0; bphase ^= 1u; }
+      }
+    }
+  } else {
+    ptx::setmaxnreg_inc<96>();
+    // ---------------------------------------------------------------- epilogue (integer mode)
+    const int q = warp & 3;
+    const int cg = (warp - bits::EPI_WARP0) >> 2;
+    const long long flag_u_int = flag_u_ptr ? static_cast<long long>(*flag_u_ptr / unit) : 0;
+    uint32_t chunk = 0;
+    for (int t = pair; t < n_tiles; t += n_pairs) {
+      const Tile tile = tiles[t];
+      unsigned long long acc[EPI2_COLS];
+#pragma unroll
+      for (int n = 0; n < EPI2_COLS; ++n) acc[n] = 0;
+      for (int ch = 0; ch < n_chunks; ++ch, ++chunk) {
+        const uint32_t buf = chunk & 1u;
+        const uint32_t shift = static_cast<uint32_t>(chunk_shift[ch]);
+        ptx::mbar_wait(tfull_bar(buf), (chunk >> 1) & 1u);
+        ptx::tc_fence_after();
+        drain_int(tmem_base + (static_cast<uint32_t>(q * 32) << 16) + buf * DN + cg * EPI2_COLS, shift, acc);
+        ptx::tc_fence_before();
+        __syncwarp();
+        if (lane == 0) ptx::mbar_arrive_cluster(tempty_bar(buf), 0);
+      }
+      const int64_t j = static_cast<int64_t>(tile.tj + static_cast<int>(cta)) * BM + q * 32 + lane;
+      const int64_t i0 = static_cast<int64_t>(tile.ti) * BN + cg * EPI2_COLS;
+      if (static_cast<int64_t>(tile.tj + static_cast<int>(cta)) * BM + q * 32 < i0 + EPI2_COLS)  // warp-uniform
+        ratio_int(acc, r_int, i0, j, lane, n_samples, i0 * (i0 - 1) / 2 - first + j, flag_u_int, out, flagged,
+                  n_flagged);
+    }
+  }
+
+  ptx::tc_fence_before();
+  ptx::cluster_sync_all();
+  if (warp == 1) {
+    __syncwarp();
+    ptx::tmem_dealloc<2>(tmem_base, TMEM_COLS);
+  }
+}
+
+// Exact recompute of flagged pairs: one warp per pair, fp64, TRUE branch lengths (len_col[k] = length of the
+// node in operand column k, 0 in padding columns).  Identical samples give exactly 0.  The presence of a node
+// is read from `rows`, in one of three formats:
+enum class Rows {
+  kBf16,  // the A operand [np][kp] of the materialised bf16 feed: P
+  kU8,    // the A operand [np][kp] of the materialised u8 feed: P*a, non-zero exactly where the node is present
+          // and has a non-zero length
+  kBits,  // the bit rows bitsS[np][kp / 32] of the bits feed
+};
+template <Rows kRows>
 __global__ void __launch_bounds__(256)
-k_unweighted_fixup(const void* __restrict__ Pv, int32_t kp, const double* __restrict__ len_col,
+k_unweighted_fixup(const void* __restrict__ rows, int32_t kp, const double* __restrict__ len_col,
                    const uint32_t* __restrict__ flagged, const unsigned long long* __restrict__ n_flagged,
                    unsigned long long* __restrict__ count_host, int64_t first, float* __restrict__ out,
                    const Exceptions ex) {
-  constexpr int kPer = kI8 ? 16 : 8;  // operand columns per 16-byte load
   const unsigned long long total = *n_flagged;
   if (blockIdx.x == 0 && threadIdx.x == 0) *count_host = total;  // mapped pinned memory
   const int lane = threadIdx.x & 31;
   const unsigned long long warps = (static_cast<unsigned long long>(gridDim.x) * blockDim.x) >> 5;
-  const int64_t row_bytes = static_cast<int64_t>(kp) * (kI8 ? 1 : 2);
+  const int32_t words = kp / 32;  // (kBits: 32-bit words per row)
   for (unsigned long long w = (static_cast<unsigned long long>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
        w < total; w += warps) {
     const uint32_t off = flagged[w];
-    const int64_t p = first + off;
-    int64_t i = static_cast<int64_t>((1.0 + sqrt(1.0 + 8.0 * static_cast<double>(p))) * 0.5);
-    while (i * (i - 1) / 2 > p) --i;
-    while ((i + 1) * i / 2 <= p) ++i;
-    const int64_t j = p - i * (i - 1) / 2;
-    const uint4* pi = reinterpret_cast<const uint4*>(static_cast<const uint8_t*>(Pv) + i * row_bytes);
-    const uint4* pj = reinterpret_cast<const uint4*>(static_cast<const uint8_t*>(Pv) + j * row_bytes);
+    int64_t i, j;
+    pair_of(first + off, i, j);
     double uniq = 0.0, comm = 0.0;
-    for (int32_t c = lane; c * kPer < kp; c += 32) {
-      const uint4 a = pi[c], b = pj[c];
-      const uint32_t aw[4] = {a.x, a.y, a.z, a.w}, bw[4] = {b.x, b.y, b.z, b.w};
+    if constexpr (kRows == Rows::kBits) {
+      const uint32_t* bi = static_cast<const uint32_t*>(rows) + i * words;
+      const uint32_t* bj = static_cast<const uint32_t*>(rows) + j * words;
+      for (int32_t c = lane; c < words; c += 32) {
+        const uint32_t a = bi[c], b = bj[c];
+        uint32_t x = a ^ b, y = a & b;
+        while (x) { const int k = __ffs(x) - 1; uniq += len_col[c * 32 + k]; x &= x - 1; }
+        while (y) { const int k = __ffs(y) - 1; comm += len_col[c * 32 + k]; y &= y - 1; }
+      }
+    } else {
+      constexpr bool kI8 = kRows == Rows::kU8;
+      constexpr int kPer = kI8 ? 16 : 8;  // operand columns per 16-byte load
+      const int64_t row_bytes = static_cast<int64_t>(kp) * (kI8 ? 1 : 2);
+      const uint4* pi = reinterpret_cast<const uint4*>(static_cast<const uint8_t*>(rows) + i * row_bytes);
+      const uint4* pj = reinterpret_cast<const uint4*>(static_cast<const uint8_t*>(rows) + j * row_bytes);
+      for (int32_t c = lane; c * kPer < kp; c += 32) {
+        const uint4 a = pi[c], b = pj[c];
+        const uint32_t aw[4] = {a.x, a.y, a.z, a.w}, bw[4] = {b.x, b.y, b.z, b.w};
 #pragma unroll
-      for (int h = 0; h < kPer; ++h) {
-        const int32_t k = c * kPer + h;
-        bool pa, pb;
-        if constexpr (kI8) {
-          pa = ((aw[h >> 2] >> ((h & 3) * 8)) & 0xFFu) != 0;
-          pb = ((bw[h >> 2] >> ((h & 3) * 8)) & 0xFFu) != 0;
-        } else {
-          pa = ((aw[h >> 1] >> ((h & 1) * 16)) & 0xFFFFu) != 0;
-          pb = ((bw[h >> 1] >> ((h & 1) * 16)) & 0xFFFFu) != 0;
+        for (int h = 0; h < kPer; ++h) {
+          const int32_t k = c * kPer + h;
+          bool pa, pb;
+          if constexpr (kI8) {
+            pa = ((aw[h >> 2] >> ((h & 3) * 8)) & 0xFFu) != 0;
+            pb = ((bw[h >> 2] >> ((h & 3) * 8)) & 0xFFu) != 0;
+          } else {
+            pa = ((aw[h >> 1] >> ((h & 1) * 16)) & 0xFFFFu) != 0;
+            pb = ((bw[h >> 1] >> ((h & 1) * 16)) & 0xFFFFu) != 0;
+          }
+          if (pa && pb) comm += len_col[k];
+          else if (pa || pb) uniq += len_col[k];
         }
-        if (pa && pb) comm += len_col[k];
-        else if (pa || pb) uniq += len_col[k];
       }
     }
 #pragma unroll
@@ -518,8 +822,12 @@ bool make_map(CUtensorMap* m, const void* base, int64_t rows, int32_t kp, int bo
 }  // namespace
 
 struct TcOperands {
-  CUtensorMap mapP, mapBh, mapBl;
-  const void* P;
+  bool from_bits = false;  // the operand feed: false = materialised (k_unweighted_tc2), true = bits (k_unweighted_bits2)
+  CUtensorMap mapP, mapBh, mapBl;  // materialised: the three K-major operands
+  const void* P = nullptr;         // materialised: the A operand (the fix-up reads presence from it)
+  CUtensorMap mapBits;             // bits: 128-sample x 16-byte tiles of bitsS
+  const uint32_t* bitsS = nullptr; // bits: the bit rows [np][kp / 32] (the fix-up reads presence from them)
+  const uint8_t *qa = nullptr, *qh = nullptr, *ql = nullptr;  // bits: per-column u8 factors (k_quantize_lengths)
   bool i8;
   int32_t kp;
   TcChunks chunks;
@@ -551,6 +859,11 @@ bool tc_setup(std::string* err) {
     if (err) *err = std::string("cudaFuncSetAttribute(k_unweighted_tc2): ") + cudaGetErrorString(e);
     return false;
   }
+  e = cudaFuncSetAttribute(k_unweighted_bits2, cudaFuncAttributeMaxDynamicSharedMemorySize, bits::SMEM_BYTES);
+  if (e != cudaSuccess) {
+    if (err) *err = std::string("cudaFuncSetAttribute(k_unweighted_bits2): ") + cudaGetErrorString(e);
+    return false;
+  }
   return true;
 }
 
@@ -573,11 +886,36 @@ TcOperands* tc_operands_create(const void* P, const void* Bh, const void* Bl, in
   }
   return o;
 }
+TcOperands* tc_operands_create_bits(const uint32_t* bitsS, int64_t np, int32_t kp, const uint8_t* qa,
+                                    const uint8_t* qh, const uint8_t* ql, const TcChunks& chunks,
+                                    const double* len_col, const double* flag_u, const long long* r_int,
+                                    double unit, std::string* err) {
+  if (!g_encode) { if (err) *err = "tc_setup has not run on this device context"; return nullptr; }
+  TcOperands* o = new TcOperands();
+  o->from_bits = true;
+  o->bitsS = bitsS; o->qa = qa; o->qh = qh; o->ql = ql;
+  o->i8 = true; o->kp = kp; o->chunks = chunks;
+  o->len_col = len_col; o->flag_u = flag_u; o->r_int = r_int; o->unit = unit;
+  cuuint64_t dims[2] = {static_cast<cuuint64_t>(kp / 8), static_cast<cuuint64_t>(np)};
+  cuuint64_t strides[1] = {static_cast<cuuint64_t>(kp / 8)};
+  cuuint32_t box[2] = {16, 128};
+  cuuint32_t estr[2] = {1, 1};
+  CUresult rc = g_encode(&o->mapBits, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<uint32_t*>(bitsS), dims, strides,
+                         box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
+                         CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (rc != CUDA_SUCCESS) {
+    if (err) *err = "cuTensorMapEncodeTiled(bits) failed with CUresult " + std::to_string(static_cast<int>(rc));
+    delete o;
+    return nullptr;
+  }
+  return o;
+}
 void tc_operands_set_int(TcOperands* o, const long long* r_int, double unit) { o->r_int = r_int; o->unit = unit; }
 void tc_operands_destroy(TcOperands* o) { delete o; }
 
 }  // namespace frc
-// Debug helper (not part of the C ABI): copies the FRC_TC_DEBUG=8 timeline counters.
+// Debug helpers (not part of the C ABI): copy the timeline counters of k_unweighted_tc2 (FRC_TC_DEBUG=8) and
+// of k_unweighted_bits2 (always accumulated; clear != 0 zeroes them after the copy).
 extern "C" int frc_debug_tc_counters(unsigned long long* out, int n) {
 #ifdef FRC_TC_TIMELINE
   if (n > 512 * 8) n = 512 * 8;
@@ -585,6 +923,17 @@ extern "C" int frc_debug_tc_counters(unsigned long long* out, int n) {
 #else
   (void)out; (void)n;
   return -1;  // built without -DFRC_TC_TIMELINE
+#endif
+}
+extern "C" int frc_debug_bits_counters(unsigned long long* out, int n, int clear) {
+#ifdef FRC_TC_TIMELINE
+  if (n > 512 * 8) n = 512 * 8;
+  int rc = static_cast<int>(cudaMemcpyFromSymbol(out, frc::g_bits_dbg, sizeof(unsigned long long) * n));
+  if (clear) { static unsigned long long z[512 * 8] = {0}; cudaMemcpyToSymbol(frc::g_bits_dbg, z, sizeof(z)); }
+  return rc;
+#else
+  (void)out; (void)n; (void)clear;
+  return -1;
 #endif
 }
 namespace frc {
@@ -604,6 +953,12 @@ int launch_unweighted_tc(const TcOperands* ops, const double* r, const Tile* til
   const int pairs = num_sms / 2;
   const int grid = 2 * (n_tiles < pairs ? n_tiles : pairs);
   const TcChunks& c = ops->chunks;
+  if (ops->from_bits) {  // integer mode: U and V are exact, so r and flag_below play no part
+    k_unweighted_bits2<<<grid, bits::THREADS, bits::SMEM_BYTES, s>>>(
+        ops->mapBits, ops->qa, ops->qh, ops->ql, c.end, c.shift, c.n, ops->r_int, ops->unit, tiles, n_tiles, n_samples,
+        first, out, ops->flag_u, flagged, n_flagged);
+    return 1;
+  }
 #define FRC_TC2_ARGS ops->mapP, ops->mapBh, ops->mapBl, c.end, c.scale, c.shift, c.n, c.biased ? 1 : 0, r, ops->r_int, \
                      ops->unit, tiles, n_tiles, n_samples, first, out, flag_below, ops->flag_u, flagged, n_flagged, ops->dbg
   if (ops->i8 && ops->r_int) k_unweighted_tc2<2><<<grid, THREADS2, SMEM2_BYTES, s>>>(FRC_TC2_ARGS);
@@ -616,12 +971,11 @@ int launch_unweighted_tc(const TcOperands* ops, const double* r, const Tile* til
 int launch_unweighted_fixup(const TcOperands* ops, const uint32_t* flagged, const unsigned long long* n_flagged,
                             unsigned long long* count_host, int64_t first, float* out, const Exceptions& ex,
                             int num_sms, cudaStream_t s) {
-  if (ops->i8)
-    k_unweighted_fixup<true><<<num_sms * 4, 256, 0, s>>>(ops->P, ops->kp, ops->len_col, flagged, n_flagged,
-                                                         count_host, first, out, ex);
-  else
-    k_unweighted_fixup<false><<<num_sms * 4, 256, 0, s>>>(ops->P, ops->kp, ops->len_col, flagged, n_flagged,
-                                                          count_host, first, out, ex);
+  const auto kernel = ops->from_bits ? k_unweighted_fixup<Rows::kBits>
+                      : ops->i8      ? k_unweighted_fixup<Rows::kU8>
+                                     : k_unweighted_fixup<Rows::kBf16>;
+  const void* rows = ops->from_bits ? static_cast<const void*>(ops->bitsS) : ops->P;
+  kernel<<<num_sms * 4, 256, 0, s>>>(rows, ops->kp, ops->len_col, flagged, n_flagged, count_host, first, out, ex);
   return 1;
 }
 

@@ -216,11 +216,8 @@ k_weighted_fixup(const int64_t* __restrict__ row_ptr, const int32_t* __restrict_
   constexpr double kFix = 1152921504606846976.0;  // 2^60: proportions are <= 1, a node sums <= 1
   for (unsigned long long w = blockIdx.x; w < n; w += gridDim.x) {
     const uint32_t off = flagged[w];
-    const int64_t p = first + off;
-    int64_t i = static_cast<int64_t>((1.0 + sqrt(1.0 + 8.0 * static_cast<double>(p))) * 0.5);
-    while (i * (i - 1) / 2 > p) --i;
-    while ((i + 1) * i / 2 <= p) ++i;
-    const int64_t j = p - i * (i - 1) / 2;
+    int64_t i, j;
+    pair_of(first + off, i, j);
     const int64_t smp[2] = {i, j};
     // without normalisation (-l) raw values are summed: scale them into the fixed-point range
     double inv[2];

@@ -1,9 +1,21 @@
-// Device side of the fp32 output format (see wire.cu): how the exact fix-up kernels store a recomputed
-// distance into an fp32 band.
+// Device side of the flat lower triangle and of the fp32 output format (see wire.cu): how a pair kernel
+// finds the samples of a flat pair index, and how the exact fix-up kernels store a recomputed distance
+// into an fp32 band.
 #pragma once
 #include "frc_internal.h"
 
 namespace frc {
+
+// Flat pair index p -> samples (i, j), j < i, p = i(i-1)/2 + j (the inverse of tri()).  The fp64 square
+// root is only a first guess; the two integer loops make the result exact for every p.
+__device__ __forceinline__ void pair_of(int64_t p, int64_t& i, int64_t& j) {
+  // largest i with i(i-1)/2 <= p
+  int64_t g = static_cast<int64_t>((1.0 + sqrt(1.0 + 8.0 * static_cast<double>(p))) * 0.5);
+  while (g * (g - 1) / 2 > p) --g;
+  while ((g + 1) * g / 2 <= p) ++g;
+  i = g;
+  j = p - g * (g - 1) / 2;
+}
 
 // out[off] = float(d).  A value fp32 cannot carry to 2^-23 relative (underflow: |d| < 1.2e-38) is also
 // appended to the band's exception list in mapped pinned host memory (rare: a system-scope atomic and two
