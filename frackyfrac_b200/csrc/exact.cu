@@ -16,14 +16,14 @@
 namespace frc {
 namespace {
 
-template <bool kWeighted>
+template <bool kWeighted, bool kRect>
 __global__ void k_exact_pairs(const double* __restrict__ E, const double* __restrict__ length,
                               int32_t n_nodes, int64_t ld, int64_t first, int64_t count,
-                              double* __restrict__ out) {
+                              double* __restrict__ out, const Geometry geo) {
   int64_t t = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (t >= count) return;
   int64_t i, j;
-  pair_of(first + t, i, j);
+  pair_at<kRect>(first + t, geo, i, j);
   const double* ea = E + i;  // a = sample i (first of the pair, common.go:25)
   const double* eb = E + j;
   if (kWeighted) {
@@ -105,13 +105,14 @@ __global__ void k_list_fill(const double* __restrict__ E, const int32_t* __restr
 
 // One thread per pair: the two-pointer walk of unifrac.go:178-203 over lists that are NOT id-sorted,
 // every product and sum a separate IEEE operation.
+template <bool kRect>
 __global__ void k_unsorted_pairs(const int64_t* __restrict__ list_ptr, const int32_t* __restrict__ list_id,
                                  const double* __restrict__ list_val, const double* __restrict__ length,
-                                 int64_t first, int64_t count, double* __restrict__ out) {
+                                 int64_t first, int64_t count, double* __restrict__ out, const Geometry geo) {
   const int64_t t = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (t >= count) return;
   int64_t si, sj;
-  pair_of(first + t, si, sj);
+  pair_at<kRect>(first + t, geo, si, sj);
   int64_t i = list_ptr[si], j = list_ptr[sj];
   const int64_t ie = list_ptr[si + 1], je = list_ptr[sj + 1];
   double numer = 0.0, denom = 0.0;
@@ -166,21 +167,22 @@ int launch_postorder_lists(const double* E, const int32_t* post_order, int32_t n
 }
 
 int launch_unsorted_pairs(const int64_t* list_ptr, const int32_t* list_id, const double* list_val,
-                          const double* length, int64_t first, int64_t count, double* out, cudaStream_t s) {
+                          const double* length, int64_t first, const Geometry& geo, int64_t count, double* out,
+                          cudaStream_t s) {
   if (count <= 0) return 0;
-  k_unsorted_pairs<<<static_cast<unsigned>((count + 127) / 128), 128, 0, s>>>(list_ptr, list_id, list_val, length,
-                                                                              first, count, out);
+  const auto kernel = geo.rect ? k_unsorted_pairs<true> : k_unsorted_pairs<false>;
+  kernel<<<static_cast<unsigned>((count + 127) / 128), 128, 0, s>>>(list_ptr, list_id, list_val, length, first, count,
+                                                                    out, geo);
   return 1;
 }
 
 int launch_exact_pairs(const double* E, const double* length, int32_t n_nodes, int64_t ld,
-                       bool weighted, int64_t first, int64_t count, double* out, cudaStream_t s) {
+                       bool weighted, int64_t first, const Geometry& geo, int64_t count, double* out, cudaStream_t s) {
   if (count <= 0) return 0;
   unsigned grid = static_cast<unsigned>((count + 127) / 128);
-  if (weighted)
-    k_exact_pairs<true><<<grid, 128, 0, s>>>(E, length, n_nodes, ld, first, count, out);
-  else
-    k_exact_pairs<false><<<grid, 128, 0, s>>>(E, length, n_nodes, ld, first, count, out);
+  const auto kernel = weighted ? (geo.rect ? k_exact_pairs<true, true> : k_exact_pairs<true, false>)
+                               : (geo.rect ? k_exact_pairs<false, true> : k_exact_pairs<false, false>);
+  kernel<<<grid, 128, 0, s>>>(E, length, n_nodes, ld, first, count, out, geo);
   return 1;
 }
 

@@ -44,6 +44,16 @@ struct PeerPtrs {
 // One tile of the lower triangle: rows [128*ti, +128) x cols [128*tj, +128), tj <= ti.
 struct Tile { int32_t ti, tj; };
 
+// Which pairs a job computes.  Triangle (rect == false): (i, j), j < i, of the whole table, flat index
+// i(i-1)/2 + j.  Rectangle (frc_create_cross): the table is [reference rows; empty rows up to q0; query rows]
+// with q0 a multiple of 256 (a CTA-pair tile), and the pairs are (i, j) for every query row i >= q0 and
+// reference row j < n_ref, flat index (i - q0) * n_ref + j.  The kernels take it as a compile-time choice
+// (Tri / Rect instantiations) plus this argument; the launchers below pick the instantiation from `rect`.
+struct Geometry {
+  bool rect = false;
+  int64_t q0 = 0, n_ref = 0;
+};
+
 // The fast paths store fp32 distances.  A fix-up kernel that meets a value fp32 cannot carry to 2^-23
 // relative (|d| < 1.2e-38: pathological trees only) also reports it here, in mapped pinned host memory:
 // frc_next patches it into the widened doubles, frc_chunk_exceptions hands it to fp32 consumers.
@@ -162,9 +172,9 @@ bool comm_all_gather_host(Comm* c, const void* mine, size_t bytes, void* all, cu
 bool comm_barrier(Comm* c, cudaStream_t s, std::string* err);
 
 // ---- exact.cu ---------------------------------------------------------------
-// fp64 reference-order distances for pairs [first, first+count) of the triangle.
+// fp64 reference-order distances for pairs [first, first+count) of the job's geometry.
 int launch_exact_pairs(const double* E, const double* length, int32_t n_nodes, int64_t ld,
-                       bool weighted, int64_t first, int64_t count, double* out, cudaStream_t s);
+                       bool weighted, int64_t first, const Geometry& geo, int64_t count, double* out, cudaStream_t s);
 // Flag -l AS CODED in the reference (normalize = 0): without normalizeFlatNodes the per-sample lists stay in
 // the order abundanceToFlatNodes appended them (post-order, unifrac.go:32-53) and unifracDistWeighted's
 // merge-join (:174-205) compares ids of lists that are not sorted.  Reproduced literally here; the fast form of
@@ -176,7 +186,8 @@ int launch_exact_pairs(const double* E, const double* length, int32_t n_nodes, i
 int launch_postorder_lists(const double* E, const int32_t* post_order, int32_t n_nodes, int64_t ld, int64_t n_samples,
                            int64_t* list_ptr, int32_t* list_id, double* list_val, cudaStream_t s);
 int launch_unsorted_pairs(const int64_t* list_ptr, const int32_t* list_id, const double* list_val,
-                          const double* length, int64_t first, int64_t count, double* out, cudaStream_t s);
+                          const double* length, int64_t first, const Geometry& geo, int64_t count, double* out,
+                          cudaStream_t s);
 
 // ---- wire.cu ----------------------------------------------------------------
 // fp32 on PCIe for the fast paths: the pair kernels store fp32, frc_next widens on the host.
@@ -202,15 +213,16 @@ struct PanelMap {
 // node v only counts as matched, |a - b|, where the two samples' keys agree; everywhere else a + b.
 int launch_weighted_tiles(const PanelMap& A, int64_t ld, int32_t kp, const float* lenf, bool prescaled,
                           const double* W, const Tile* tiles, int32_t n_tiles, int64_t n_samples,
-                          int64_t first, float* out, double flag_below, uint32_t* flagged,
+                          int64_t first, const Geometry& geo, float* out, double flag_below, uint32_t* flagged,
                           unsigned long long* n_flagged, int num_sms, cudaStream_t s, const int32_t* K = nullptr);
 // fp64 / fixed-point recompute of the flagged pairs from the CSR rows (total: per-sample normaliser,
 // null for -l); ws = ws_ctas zeroed int64 arrays of n_nodes entries (2 * n_nodes with K), left zeroed.
 // K non-null: the keyed -l numerator, with the match decision read from the key panels K[np/128][kp][128].
 int launch_weighted_fixup(const DevCsr& a, const DevTree& t, const double* total, const double* W,
                           const uint32_t* flagged, const unsigned long long* n_flagged,
-                          unsigned long long* count_host, int64_t first, long long* ws, int ws_ctas, float* out,
-                          const Exceptions& ex, cudaStream_t s, const int32_t* K = nullptr, int32_t kp = 0);
+                          unsigned long long* count_host, int64_t first, const Geometry& geo, long long* ws,
+                          int ws_ctas, float* out, const Exceptions& ex, cudaStream_t s, const int32_t* K = nullptr,
+                          int32_t kp = 0);
 void weighted_setup();  // cudaFuncSetAttribute calls for the CURRENT device (once per device context)
 
 // ---- unweighted_tc.cu -------------------------------------------------------
@@ -245,12 +257,13 @@ int tc_chunk_kblocks();  // bf16: K blocks per fp32 accumulation run (FRC_TC_CHU
 // capacity = pairs of the band, so it cannot overflow) for the fix-up pass.
 // Integer mode (either feed) flags by flag_u alone; the bits feed does not read r or flag_below.
 int launch_unweighted_tc(const TcOperands* ops, const double* r, const Tile* tiles, int32_t n_tiles,
-                         int64_t n_samples, int64_t first, float* out, double flag_below,
+                         int64_t n_samples, int64_t first, const Geometry& geo, float* out, double flag_below,
                          uint32_t* flagged, unsigned long long* n_flagged, int num_sms, cudaStream_t s);
 // fp64 recompute of the flagged pairs from the feed's presence rows and true lengths.
 int launch_unweighted_fixup(const TcOperands* ops, const uint32_t* flagged,
                             const unsigned long long* n_flagged, unsigned long long* count_host,
-                            int64_t first, float* out, const Exceptions& ex, int num_sms, cudaStream_t s);
+                            int64_t first, const Geometry& geo, float* out, const Exceptions& ex, int num_sms,
+                            cudaStream_t s);
 bool tc_setup(std::string* err);  // driver entry point (once per process) + smem attributes for the CURRENT device
 
 }  // namespace frc

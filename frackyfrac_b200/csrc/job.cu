@@ -205,6 +205,7 @@ struct Shared {
   bool keyed = false;         // normalize == 0 on the FP32 tiles (FRC_FLAG_L_TILES): key panels next to the values
   bool node_mult = false;     // FRC_FLAG_PRUNE, fast weighted, normalize == 1: the totals weigh node v by mult[v]
   bool d2h = true;
+  Geometry geo;               // frc_create_cross: the query x reference block of the staged table (n_q = N - geo.q0)
   int n_parts = 1;
   int world = 1, rank0 = 0;   // band ownership: `world` owners; part p owns owner id rank0 + p
   enum Exchange { kNone, kInProcess, kNccl } exchange = kNone;  // how the sample shards of the embedding meet
@@ -212,7 +213,7 @@ struct Shared {
   bool capacity = false;      // fast weighted over several devices: panels stay sharded (PanelMap), tiles read peers' HBM
   ShardPlan shards;           // which samples each owner builds (np = shards.np)
   ColumnPlan cols;
-  std::vector<Band> bands;   // whole triangle (owners filled in)
+  std::vector<Band> bands;   // every band of the job (owners filled in)
   std::vector<int32_t> level_ptr;
   int32_t tree_height = 0;
   // inputs: [row_ptr | tree arrays ... | col | val] in one pinned buffer, same layout on every device
@@ -704,10 +705,11 @@ int enqueue_band(Part* p, size_t idx) {
   PART_CUDA(p, cudaEventRecord(sl.k0, s));
   if (sh.exact) {
     if (sh.unsorted_l)
-      launches += launch_unsorted_pairs(p->d_list_ptr, p->d_list_id, p->d_list_val, p->dtree.length, b.first, b.count,
-                                        sl.dev64, s);
+      launches += launch_unsorted_pairs(p->d_list_ptr, p->d_list_id, p->d_list_val, p->dtree.length, b.first, sh.geo,
+                                        b.count, sl.dev64, s);
     else
-      launches += launch_exact_pairs(p->d_E, p->dtree.length, sh.B, sh.np, sh.weighted, b.first, b.count, sl.dev64, s);
+      launches += launch_exact_pairs(p->d_E, p->dtree.length, sh.B, sh.np, sh.weighted, b.first, sh.geo, b.count,
+                                     sl.dev64, s);
     PART_CUDA(p, cudaEventRecord(sl.k1, s));
   } else {
     // no copy-engine work between the kernels: a memset or an 8-byte D2H would queue behind the
@@ -717,18 +719,18 @@ int enqueue_band(Part* p, size_t idx) {
     *sl.ex.count = 0;  // (the slot's previous band has been delivered)
     if (sh.weighted) {
       launches += launch_weighted_tiles(p->pm, sh.np, sh.kp, p->d_lenf, sh.prescale, p->d_W, p->d_tiles + b.tile_off,
-                                        b.n_tiles, sh.N, b.first, sl.dev32, kFlagBelowW, sl.flagged, cnt, dc->num_sms, s,
-                                        p->d_K);
+                                        b.n_tiles, sh.N, b.first, sh.geo, sl.dev32, kFlagBelowW, sl.flagged, cnt,
+                                        dc->num_sms, s, p->d_K);
       PART_CUDA(p, cudaEventRecord(sl.k1, s));
       // (one workspace per compute stream: consecutive bands run their fix-ups concurrently)
       launches += launch_weighted_fixup(p->dcsr, p->dtree, sh.opts.normalize == 1 ? p->d_total : nullptr, p->d_W,
-                                        sl.flagged, cnt, sl.n_flagged_host, b.first, p->d_fix_ws[si], kFixupCtas,
+                                        sl.flagged, cnt, sl.n_flagged_host, b.first, sh.geo, p->d_fix_ws[si], kFixupCtas,
                                         sl.dev32, sl.ex, s, p->d_K, sh.kp);
     } else {
-      launches += launch_unweighted_tc(p->tc, p->d_r, p->d_tiles + b.tile_off, b.n_tiles, sh.N, b.first, sl.dev32,
-                                       kFlagBelow, sl.flagged, cnt, dc->num_sms, s);
+      launches += launch_unweighted_tc(p->tc, p->d_r, p->d_tiles + b.tile_off, b.n_tiles, sh.N, b.first, sh.geo,
+                                       sl.dev32, kFlagBelow, sl.flagged, cnt, dc->num_sms, s);
       PART_CUDA(p, cudaEventRecord(sl.k1, s));
-      launches += launch_unweighted_fixup(p->tc, sl.flagged, cnt, sl.n_flagged_host, b.first, sl.dev32, sl.ex,
+      launches += launch_unweighted_fixup(p->tc, sl.flagged, cnt, sl.n_flagged_host, b.first, sh.geo, sl.dev32, sl.ex,
                                           dc->num_sms, s);
     }
   }
@@ -799,11 +801,11 @@ int start_pairs_capacity(Part* p) {
       if (cb.shard < c) continue;
       const int32_t t0 = cb.coff[c], n = cb.coff[c + 1] - cb.coff[c];
       launches += launch_weighted_tiles(pm, sh.np, sh.kp, p->d_lenf, sh.prescale, p->d_W, p->d_tiles + cb.tile_off + t0, n,
-                                        sh.N, cb.first, cb.out, kFlagBelowW, cb.flagged, cb.cnt, dc->num_sms, s);
+                                        sh.N, cb.first, sh.geo, cb.out, kFlagBelowW, cb.flagged, cb.cnt, dc->num_sms, s);
       if (cb.shard == c) {
         launches += launch_weighted_fixup(p->dcsr, p->dtree, sh.opts.normalize == 1 ? p->d_total : nullptr, p->d_W,
-                                          cb.flagged, cb.cnt, cb.n_flagged_host, cb.first, p->d_fix_ws[0], kFixupCtas,
-                                          cb.out, cb.ex, s);
+                                          cb.flagged, cb.cnt, cb.n_flagged_host, cb.first, sh.geo, p->d_fix_ws[0],
+                                          kFixupCtas, cb.out, cb.ex, s);
         PART_CUDA(p, cudaEventRecord(cb.done, s));
       }
     }
@@ -1057,8 +1059,27 @@ int frc_ctx_comm_init(frc_ctx_t* ctx, const char* id, int32_t rank, int32_t worl
 namespace {
 
 // ------------------------------------------------------------------ frc_create, unit by unit
-// (1) options and table header; fills the sizes of `sh`.  No CUDA call.
-int validate_header(frc_job* j, const frc_tree_t* tree, const frc_csr_t* abnd, const frc_opts_t* opts) {
+// The shape checks of one table; `name` is null for frc_create's table, "reference" / "query" for the two tables of
+// frc_create_cross (their messages then name the table and the row within it).
+int check_table(frc_job* j, const frc_csr_t* t, const char* name) {
+  const std::string pre = name ? std::string(name) + " table: " : "";
+  const int64_t N = t->n_samples;
+  if (N < 0 || (N > 0 && !t->row_ptr)) return fail(j, FRC_ERR_ARG, pre + "bad abundance table");
+  if (N > (1LL << 31) - 256) return fail(j, FRC_ERR_UNSUPPORTED, pre + "too many samples");
+  const int64_t nnz = N > 0 ? t->row_ptr[N] : 0;
+  if (N > 0 && t->row_ptr[0] != 0) return fail(j, FRC_ERR_ARG, pre + "row_ptr[0] != 0");
+  if (nnz < 0 || (nnz > 0 && (!t->col || !t->val))) return fail(j, FRC_ERR_ARG, pre + "bad abundance table");
+  for (int64_t s = 0; s < N; ++s)
+    if (t->row_ptr[s + 1] < t->row_ptr[s] || t->row_ptr[s + 1] > nnz)
+      return fail(j, FRC_ERR_ARG, name ? pre + "row_ptr is not monotone at " + name + " sample #" + std::to_string(s + 1)
+                                       : std::string("row_ptr is not monotone"));
+  return FRC_OK;
+}
+
+// (1) options and table header; fills the sizes of `sh`.  No CUDA call.  query != null: frc_create_cross, abnd is
+// the reference table and the job stages [reference rows; empty rows up to q0; query rows] (Geometry).
+int validate_header(frc_job* j, const frc_tree_t* tree, const frc_csr_t* abnd, const frc_csr_t* query,
+                    const frc_opts_t* opts) {
   Shared& sh = j->sh;
   if (opts->mode != FRC_UNWEIGHTED && opts->mode != FRC_WEIGHTED) return fail(j, FRC_ERR_ARG, "bad mode");
   if (opts->path < FRC_PATH_AUTO || opts->path > FRC_PATH_EXACT) return fail(j, FRC_ERR_ARG, "bad path");
@@ -1076,26 +1097,42 @@ int validate_header(frc_job* j, const frc_tree_t* tree, const frc_csr_t* abnd, c
   const int rank = opts->world <= 0 ? 0 : opts->rank;
   if (rank < 0 || rank >= world) return fail(j, FRC_ERR_ARG, "rank outside [0, world)");
   if (opts->band_rows < 0) return fail(j, FRC_ERR_ARG, "band_rows < 0");
+  if (query) {
+    // one process, one ordered stream of the block: the multi-process forms (band sharding over ranks, the sharded
+    // embedding) are triangle-only
+    if (opts->world > 1)
+      return fail(j, FRC_ERR_UNSUPPORTED, "frc_create_cross runs in one process (world <= 1); opts.n_devices spreads "
+                                          "it over several GPUs");
+    if (opts->flags & FRC_FLAG_SHARD_EMBED)
+      return fail(j, FRC_ERR_UNSUPPORTED, "FRC_FLAG_SHARD_EMBED (one process per GPU) is not supported by "
+                                          "frc_create_cross");
+  }
   const int32_t B = tree->n_nodes;
   if (B < 1 || !tree->parent || !tree->length) return fail(j, FRC_ERR_ARG, "empty tree");
   if (tree->parent[0] != -1) return fail(j, FRC_ERR_ARG, "parent[0] must be -1 (root has pre-order id 0)");
-  const int64_t N = abnd->n_samples;
-  if (N < 0 || (N > 0 && !abnd->row_ptr)) return fail(j, FRC_ERR_ARG, "bad abundance table");
-  if (N > (1LL << 31) - 256) return fail(j, FRC_ERR_UNSUPPORTED, "too many samples");
-  const int64_t nnz = N > 0 ? abnd->row_ptr[N] : 0;
-  if (N > 0 && abnd->row_ptr[0] != 0) return fail(j, FRC_ERR_ARG, "row_ptr[0] != 0");
-  if (nnz < 0 || (nnz > 0 && (!abnd->col || !abnd->val))) return fail(j, FRC_ERR_ARG, "bad abundance table");
-  for (int64_t s = 0; s < N; ++s)
-    if (abnd->row_ptr[s + 1] < abnd->row_ptr[s] || abnd->row_ptr[s + 1] > nnz)
-      return fail(j, FRC_ERR_ARG, "row_ptr is not monotone");
+  if (int rc = check_table(j, abnd, query ? "reference" : nullptr)) return rc;
+  if (query)
+    if (int rc = check_table(j, query, "query")) return rc;
   // (entries are validated while they are copied into the pinned staging buffer)
+  int64_t N = abnd->n_samples;
+  int64_t nnz = N > 0 ? abnd->row_ptr[N] : 0;
+  int64_t n_pairs = N >= 2 ? tri(N) : 0;
+  if (query) {
+    const int64_t n_ref = N, n_q = query->n_samples;
+    sh.geo.rect = true;
+    sh.geo.n_ref = n_ref;
+    sh.geo.q0 = round_up(n_ref, 2 * kTile);
+    N = sh.geo.q0 + n_q;
+    if (N > (1LL << 31) - 256) return fail(j, FRC_ERR_UNSUPPORTED, "too many samples");
+    nnz += n_q > 0 ? query->row_ptr[n_q] : 0;
+    n_pairs = n_q * n_ref;
+  }
   sh.opts = *opts;
   sh.opts.devices = nullptr;  // (borrowed pointer: not kept)
   sh.weighted = opts->mode == FRC_WEIGHTED;
   sh.N = N; sh.B = B; sh.nnz = nnz;
   sh.world = world; sh.rank0 = rank;
   sh.d2h = !(opts->flags & FRC_FLAG_NO_D2H);
-  const int64_t n_pairs = N >= 2 ? tri(N) : 0;
   if (opts->path == FRC_PATH_EXACT || (opts->normalize == 0 && !l_tiles)) sh.exact = true;
   else if (opts->path == FRC_PATH_FAST) sh.exact = false;
   else sh.exact = n_pairs == 0 || (static_cast<double>(n_pairs) * B <= static_cast<double>(kExactWorkLimit));
@@ -1162,6 +1199,10 @@ int plan_job(frc_job* j, const frc_tree_t* tree, bool neg_len) {
         cudaGetLastError();
       }
     }
+    if (want && sh.geo.rect)
+      return fail(j, FRC_ERR_UNSUPPORTED, "frc_create_cross keeps the weighted panels of all samples on every device; the "
+                                          "capacity mode, which shards them over the devices when they exceed about half "
+                                          "of one device's free HBM (or with FRC_CAPACITY=1), only runs triangle jobs");
     if (want && sh.keyed)
       return fail(j, FRC_ERR_UNSUPPORTED, "the key-matched tiles of -l as coded (FRC_FLAG_L_TILES) keep the value and key "
                                           "panels of all samples on every device; the capacity mode, which shards them "
@@ -1193,8 +1234,12 @@ int plan_job(frc_job* j, const frc_tree_t* tree, bool neg_len) {
       }
     }
   }
-  sh.bands = sh.capacity ? make_bands_capacity(sh.N, sh.shards, sh.opts.band_rows, sh.d2h)
-                         : make_bands(sh.N, sh.opts.band_rows, owners, sh.d2h, sh.knobs.bands_per_rank, 8);
+  if (sh.geo.rect)
+    sh.bands = make_bands_cross(sh.geo.q0, sh.N - sh.geo.q0, sh.geo.n_ref, sh.opts.band_rows, owners, sh.d2h,
+                                sh.knobs.bands_per_rank, 8);
+  else
+    sh.bands = sh.capacity ? make_bands_capacity(sh.N, sh.shards, sh.opts.band_rows, sh.d2h)
+                           : make_bands(sh.N, sh.opts.band_rows, owners, sh.d2h, sh.knobs.bands_per_rank, 8);
   for (const Band& b : sh.bands)
     if (b.count >= (1LL << 32)) return fail(j, FRC_ERR_UNSUPPORTED, "band too large; lower band_rows");
   return FRC_OK;
@@ -1263,7 +1308,8 @@ int prepare_part(Part* p) {
       p->cap.push_back(g);
     }
   } else if (!sh.exact) {
-    for (Band& b : p->bands) append_band_tiles(b, fast_uw, p->tiles);
+    const int32_t col_tiles = sh.geo.rect ? static_cast<int32_t>((sh.geo.n_ref + kTile - 1) / kTile) : 0;
+    for (Band& b : p->bands) append_band_tiles(b, fast_uw, p->tiles, col_tiles);
   }
   std::vector<uint8_t> need;
   if (fast_uw && sh.shards.ranges.size() > 1 && sh.fused_embed) need = operand_need_blocks(p->tiles, sh.np, true);
@@ -1516,7 +1562,7 @@ void aggregate_info(frc_job* j) {
   a.path_taken = sh.exact ? FRC_PATH_EXACT : FRC_PATH_FAST;
   a.n_bands_total = static_cast<int32_t>(sh.bands.size());
   a.tree_height = sh.tree_height;
-  a.n_pairs_total = sh.N >= 2 ? tri(sh.N) : 0;
+  a.n_pairs_total = sh.geo.rect ? (sh.N - sh.geo.q0) * sh.geo.n_ref : sh.N >= 2 ? tri(sh.N) : 0;
   a.n_nodes_padded = sh.exact ? sh.B : sh.kp;
   a.operand_kind = (!sh.exact && !sh.weighted) ? (sh.cols.i8 ? (sh.bits_feed ? 3 : 2) : 1) : 0;
   a.n_devices = static_cast<int32_t>(j->parts.size());
@@ -1541,16 +1587,11 @@ void aggregate_info(frc_job* j) {
   }
 }
 
-}  // namespace
-
-extern "C" {
-
-int frc_create(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, const frc_opts_t* opts,
-               frc_job_t** out) {
-  g_create_error.clear();
-  if (!out) { g_create_error = "frc_create: out is NULL"; return FRC_ERR_ARG; }
-  *out = nullptr;
-  if (!tree || !abnd || !opts) { g_create_error = "frc_create: NULL argument"; return FRC_ERR_ARG; }
+// frc_create (query == null) and frc_create_cross (abnd = the reference table).  A cross job stages ONE table of
+// q0 + n_q rows -- the reference rows, empty rows up to q0, the query rows (Shared::geo) -- and everything up to the
+// pair stage runs on it as on any table; only the bands, the tiles and the pair kernels' geometry differ.
+int create_job(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, const frc_csr_t* query,
+               const frc_opts_t* opts, frc_job_t** out) {
   DeviceGuard guard;
   const auto t_create0 = std::chrono::steady_clock::now();
   frc_job* j = new frc_job();
@@ -1571,7 +1612,7 @@ int frc_create(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
   };
 
   // ------------------------------------------------------------ (1) options, table header
-  int rc = validate_header(j, tree, abnd, opts);
+  int rc = validate_header(j, tree, abnd, query, opts);
   if (rc) return bail(rc);
   const int32_t B0 = sh.B;  // the caller's tree (FRC_FLAG_PRUNE: B = the pruned one)
   const int64_t N = sh.N, nnz = sh.nnz;
@@ -1611,12 +1652,14 @@ int frc_create(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
     if (check_preorder(tree0->parent, B0, depth.data(), &bad_parent, &bad_order)) {
       // the leaves listed in ANY row: every rank of a sharded multi-process job derives the same tree (out-of-range
       // entries are left to the staging checks)
+      // (frc_create_cross: the leaves of both tables)
       std::vector<uint8_t> marks(B0, 0);
       const int T = nnz >= 65536 ? c->pool->size() : 1;
+      const int64_t nnz_a = abnd->n_samples > 0 ? abnd->row_ptr[abnd->n_samples] : 0;
       const std::function<void(int)> mark_leaves = [&](int t) {
         const int64_t k1 = nnz * (t + 1) / T;
         for (int64_t k = nnz * t / T; k < k1; ++k) {
-          const int32_t cc = abnd->col[k];
+          const int32_t cc = k < nnz_a ? abnd->col[k] : query->col[k - nnz_a];
           // (read first: storing into lines that are already marked would bounce them between the cores)
           if (cc >= 0 && cc < B0 && !__atomic_load_n(&marks[cc], __ATOMIC_RELAXED))
             __atomic_store_n(&marks[cc], uint8_t{1}, __ATOMIC_RELAXED);
@@ -1641,9 +1684,27 @@ int frc_create(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
     sh.stage_in = static_cast<char*>(c->pin.alloc(sh.in_bytes, &e));
     if (!sh.stage_in) return bail(fail(j, FRC_ERR_OOM, std::string("pinned staging of the inputs: ") + cudaGetErrorString(e)));
     int64_t* rp = reinterpret_cast<int64_t*>(sh.stage_in + sh.in_rowptr.off);
-    if (N > 0) memcpy(rp, abnd->row_ptr, sizeof(int64_t) * (N + 1)); else rp[0] = 0;
+    const int64_t n_a = abnd->n_samples;
+    if (n_a > 0) memcpy(rp, abnd->row_ptr, sizeof(int64_t) * (n_a + 1)); else rp[0] = 0;
+    if (query) {  // empty rows up to q0, then the query rows after the reference entries
+      const int64_t q0 = sh.geo.q0, nnz_a = rp[n_a];
+      for (int64_t s = n_a + 1; s <= q0; ++s) rp[s] = nnz_a;
+      for (int64_t s = 1; s <= N - q0; ++s) rp[q0 + s] = nnz_a + query->row_ptr[s];
+    }
   }
   char* const stage_in = sh.stage_in;
+  const int64_t* const staged_rp = reinterpret_cast<const int64_t*>(stage_in + sh.in_rowptr.off);
+  // the caller's entries of staged row s (not called for empty rows) and the row's name in messages
+  auto source_row = [&](int64_t s, const int32_t** cp, const double** vp) {
+    const frc_csr_t* t = query && s >= sh.geo.q0 ? query : abnd;
+    const int64_t r = t == query ? s - sh.geo.q0 : s;
+    *cp = t->col + t->row_ptr[r];
+    *vp = t->val + t->row_ptr[r];
+  };
+  auto row_name = [&](int64_t s) {
+    if (!query) return "sample #" + std::to_string(s + 1);
+    return s < sh.geo.q0 ? "reference sample #" + std::to_string(s + 1) : "query sample #" + std::to_string(s - sh.geo.q0 + 1);
+  };
 
   // One task list for the pool: the tree walks, the preparation of devices 1.. (they wait for the plan),
   // then the CSR entries in chunks, all handed out through one counter; the calling thread plans, prepares
@@ -1695,7 +1756,7 @@ int frc_create(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
     const bool check_dup = sh.need_val;
     const int32_t* parent = tree0->parent;  // (checked against the caller's tree, staged with new_of_old ids)
     auto row_at = [&](int64_t target) {
-      return static_cast<int64_t>(std::lower_bound(abnd->row_ptr, abnd->row_ptr + N, target) - abnd->row_ptr);
+      return static_cast<int64_t>(std::lower_bound(staged_rp, staged_rp + N, target) - staged_rp);
     };
     std::vector<int64_t>& stamp = c->stamps[t];
     if (check_dup && static_cast<int32_t>(stamp.size()) < B0) stamp.assign(B0, -1);
@@ -1714,11 +1775,15 @@ int frc_create(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
       const int64_t s0 = row_at(stage_k0 + span * ch / TS), s1 = ch == TS - 1 ? row_at(stage_k1) : row_at(stage_k0 + span * (ch + 1) / TS);
       bool failed = false;
       for (int64_t s = s0; s < s1 && !failed; ++s) {
-        const int64_t b = abnd->row_ptr[s], e = abnd->row_ptr[s + 1];
+        const int64_t b = staged_rp[s], e = staged_rp[s + 1];
+        if (b == e) continue;
         const int64_t mark_s = stamp_tag + s;
+        const int32_t* scol;
+        const double* sval;
+        source_row(s, &scol, &sval);
         for (int64_t k = b; k < e; ++k) {
-          const int32_t cc = abnd->col[k];
-          const double v = abnd->val[k];
+          const int32_t cc = scol[k - b];
+          const double v = sval[k - b];
           const char* what = nullptr;
           if (cc < 0 || cc >= B0) what = "node id out of range";
           // pre-order ids: the first child of a node is the next id (the numbering itself is being
@@ -1727,8 +1792,8 @@ int frc_create(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
           else if (!(v > 0) || std::isinf(v)) what = "bad value";
           else if (check_dup && stamp[cc] == mark_s) what = "leaf listed twice";
           if (what) {
-            csr_errs[ch] = "sample #" + std::to_string(s + 1) + ": entry " + std::to_string(k - b + 1) + " (node " +
-                           std::to_string(cc) + "): " + what;
+            csr_errs[ch] = row_name(s) + ": entry " + std::to_string(k - b + 1) + " (node " + std::to_string(cc) + "): " +
+                           what;
             failed = true;
             break;
           }
@@ -1754,7 +1819,7 @@ int frc_create(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
   // shard plan that plan_job will make)
   if (!sh.exact && !sh.weighted && sh.n_parts == 1 && sh.world > 1 && (opts->flags & FRC_FLAG_SHARD_EMBED) && N > 0) {
     const Range own = plan_shards(N, sh.world, ShardPlan::kSharded).ranges[sh.rank0][0];
-    stage_k0 = abnd->row_ptr[std::min(N, own.s0)]; stage_k1 = abnd->row_ptr[std::min(N, own.s1)];
+    stage_k0 = staged_rp[std::min(N, own.s0)]; stage_k1 = staged_rp[std::min(N, own.s1)];
   }
   const int n_workers = c->pool->size() - 1;
   if (n_workers > 0) {
@@ -1818,6 +1883,29 @@ int frc_create(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
   j->create_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_create0).count();
   *out = j;
   return FRC_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int frc_create(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, const frc_opts_t* opts,
+               frc_job_t** out) {
+  g_create_error.clear();
+  if (!out) { g_create_error = "frc_create: out is NULL"; return FRC_ERR_ARG; }
+  *out = nullptr;
+  if (!tree || !abnd || !opts) { g_create_error = "frc_create: NULL argument"; return FRC_ERR_ARG; }
+  return create_job(ctx, tree, abnd, nullptr, opts, out);
+}
+
+int frc_create_cross(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* ref, const frc_csr_t* query,
+                     const frc_opts_t* opts, frc_job_t** out) {
+  g_create_error.clear();
+  if (!out) { g_create_error = "frc_create_cross: out is NULL"; return FRC_ERR_ARG; }
+  *out = nullptr;
+  if (!tree || !ref || !opts) { g_create_error = "frc_create_cross: NULL argument"; return FRC_ERR_ARG; }
+  if (!query) { g_create_error = "frc_create_cross: the query table is NULL"; return FRC_ERR_ARG; }
+  return create_job(ctx, tree, ref, query, opts, out);
 }
 
 }  // extern "C"

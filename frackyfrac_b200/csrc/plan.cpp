@@ -9,15 +9,11 @@
 namespace frc {
 
 // Largest-first onto the least loaded owner: the best balance, any order.
-static std::vector<int> band_owners_lpt(const std::vector<int64_t>& rows, int world) {
-  const size_t n = rows.size() > 0 ? rows.size() - 1 : 0;
+static std::vector<int> band_owners_lpt(const std::vector<int64_t>& cnt, int world) {
+  const size_t n = cnt.size();
   std::vector<int> owner(n, 0);
   std::vector<size_t> order(n);
-  std::vector<int64_t> cnt(n);
-  for (size_t k = 0; k < n; ++k) {
-    order[k] = k;
-    cnt[k] = tri(rows[k + 1]) - (rows[k] >= 2 ? tri(rows[k]) : 0);
-  }
+  for (size_t k = 0; k < n; ++k) order[k] = k;
   std::stable_sort(order.begin(), order.end(), [&](size_t a, size_t b) { return cnt[a] > cnt[b]; });
   std::vector<int64_t> load(world, 0);
   for (size_t k : order) {
@@ -30,18 +26,18 @@ static std::vector<int> band_owners_lpt(const std::vector<int64_t>& rows, int wo
   return owner;
 }
 
-std::vector<int> band_owners(const std::vector<int64_t>& rows, int world) {
+std::vector<int> band_owners(const std::vector<int64_t>& counts, int world) {
   // Few bands (at most 8 per owner: the automatic plan of a triangle that fits the rings): every owner queues
   // ALL its bands at once, so the order in which the consumer reads them cannot stall anybody and the
   // assignment only has to balance: largest first onto the least loaded owner (within ~1 %).
-  if (world > 1 && rows.size() >= 1 && rows.size() - 1 <= 8 * static_cast<size_t>(world)) return band_owners_lpt(rows, world);
+  if (world > 1 && counts.size() <= 8 * static_cast<size_t>(world)) return band_owners_lpt(counts, world);
   // More bands than the rings hold: dealt in ROUNDS of G consecutive bands, every owner exactly one band per round: a consumer reading the
   // stream in flat-index order then drains every owner's ring (and PCIe link) at the same pace, whatever the
   // ring size (a largest-first assignment over all bands balances better but hands one owner runs of
   // consecutive bands: the others' rings fill up and their GPUs idle until the consumer gets to them).
   // Inside a round the largest band goes to the owner with the smallest load so far (tile-row rounding makes
   // band sizes differ by ~10 % on small triangles; the greedy match keeps the owners within ~2 %).
-  const size_t n = rows.size() > 0 ? rows.size() - 1 : 0;
+  const size_t n = counts.size();
   std::vector<int> owner(n, 0);
   if (world <= 1) return owner;
   std::vector<int64_t> load(world, 0);
@@ -51,7 +47,7 @@ std::vector<int> band_owners(const std::vector<int64_t>& rows, int world) {
     const size_t k1 = std::min(n, k0 + world);
     idx.clear();
     for (size_t k = k0; k < k1; ++k) idx.push_back(k);
-    auto cnt = [&](size_t k) { return tri(rows[k + 1]) - (rows[k] >= 2 ? tri(rows[k]) : 0); };
+    auto cnt = [&](size_t k) { return counts[k]; };
     std::stable_sort(idx.begin(), idx.end(), [&](size_t a, size_t b) { return cnt(a) > cnt(b); });
     for (int r = 0; r < world; ++r) who[r] = r;
     std::stable_sort(who.begin(), who.end(), [&](int a, int b) { return load[a] < load[b]; });
@@ -102,7 +98,9 @@ std::vector<int64_t> band_boundaries(int64_t N, int64_t requested, int world, bo
 
 std::vector<Band> make_bands(int64_t N, int64_t requested, int world, bool d2h, int per_rank, int value_bytes) {
   const std::vector<int64_t> rows = band_boundaries(N, requested, world, d2h, per_rank, value_bytes);
-  const std::vector<int> owners = band_owners(rows, world);
+  std::vector<int64_t> counts;
+  for (size_t k = 0; k + 1 < rows.size(); ++k) counts.push_back(tri(rows[k + 1]) - (rows[k] >= 2 ? tri(rows[k]) : 0));
+  const std::vector<int> owners = band_owners(counts, world);
   std::vector<Band> bands;
   for (size_t k = 0; k + 1 < rows.size(); ++k) {
     Band b;
@@ -111,6 +109,54 @@ std::vector<Band> make_bands(int64_t N, int64_t requested, int world, bool d2h, 
     b.count = tri(b.row1) - b.first;
     b.owner = owners[k];
     if (b.count > 0) bands.push_back(b);
+  }
+  return bands;
+}
+
+std::vector<Band> make_bands_cross(int64_t q0, int64_t n_q, int64_t n_ref, int64_t requested, int world, bool d2h,
+                                   int per_rank, int value_bytes) {
+  // query rows [0, n_q) relative to q0; every row holds n_ref pairs, so equal pair counts are equal row counts
+  std::vector<int64_t> rows{0};
+  if (n_q > 0 && n_ref > 0) {
+    if (world < 1) world = 1;
+    if (requested > 0) {
+      const int64_t step = round_up(requested, kTile);
+      for (int64_t r = step; r < n_q; r += step) rows.push_back(r);
+    } else {
+      // the policy of band_boundaries: band count per owner, the same byte caps per band, whole tiles
+      const int64_t tile_rows = (n_q + kTile - 1) / kTile;
+      int64_t n = d2h ? 8LL * world : (world == 1 ? 1 : 2LL * world);
+      if (d2h && per_rank > 0) n = static_cast<int64_t>(per_rank) * world;
+      const double total_bytes = static_cast<double>(value_bytes) * static_cast<double>(n_q) * static_cast<double>(n_ref);
+      const double band_cap = d2h ? 96.0 * 1024 * 1024 : 1536.0 * 1024 * 1024;
+      const int64_t by_size = static_cast<int64_t>(std::ceil(total_bytes / band_cap));
+      if (by_size > n) n = round_up(by_size, 2LL * world);
+      n = std::max<int64_t>(1, std::min(n, tile_rows));
+      for (int64_t k = 1; k < n; ++k) {
+        int64_t r = static_cast<int64_t>(std::llround(static_cast<double>(n_q) * k / n / kTile)) * kTile;
+        r = std::max(r, rows.back() + kTile);
+        if (r >= n_q) break;
+        rows.push_back(r);
+      }
+      if (d2h && world == 1 && rows.size() > 1) {
+        // (as for the triangle: the first band is cut again so that the D2H chain starts early)
+        const int64_t r = static_cast<int64_t>(std::llround(static_cast<double>(n_q) * 0.25 / n / kTile)) * kTile;
+        if (r >= kTile && r < rows[1]) rows.insert(rows.begin() + 1, r);
+      }
+    }
+    rows.push_back(n_q);
+  }
+  std::vector<int64_t> counts;
+  for (size_t k = 0; k + 1 < rows.size(); ++k) counts.push_back((rows[k + 1] - rows[k]) * n_ref);
+  const std::vector<int> owners = band_owners(counts, world);
+  std::vector<Band> bands;
+  for (size_t k = 0; k + 1 < rows.size(); ++k) {
+    Band b;
+    b.row0 = q0 + rows[k]; b.row1 = q0 + rows[k + 1];
+    b.first = rows[k] * n_ref;
+    b.count = counts[k];
+    b.owner = owners[k];
+    bands.push_back(b);
   }
   return bands;
 }
@@ -308,27 +354,29 @@ ColumnPlan plan_columns(const double* length, int32_t B, bool want_i8, int gb, b
   return p;
 }
 
-void append_band_tiles(Band& b, bool pair_tiles, std::vector<Tile>& tiles) {
+void append_band_tiles(Band& b, bool pair_tiles, std::vector<Tile>& tiles, int32_t col_tiles) {
   b.tile_off = static_cast<int32_t>(tiles.size());
   const int32_t t0 = static_cast<int32_t>(b.row0 / kTile), t1 = static_cast<int32_t>((b.row1 - 1) / kTile);
+  const bool rect = col_tiles > 0;
   if (pair_tiles) {
-    // pair tiles: (ti, tj) and (ti, tj+1) with tj even; needed when tj <= ti.  The clusters
-    // that run together (74 on a B200) take consecutive list entries, so the list walks
+    // pair tiles: (ti, tj) and (ti, tj+1) with tj even; needed when tj <= ti (rectangle: tj < col_tiles).
+    // The clusters that run together (74 on a B200) take consecutive list entries, so the list walks
     // compact super-tiles of ~9 tile rows x ~8 tile-pair columns: the wave then shares
     // 9 + 8 operand panels instead of 2 + 37 and its working set fits the 126 MB L2.
     const int32_t rows_blk = std::min<int32_t>(9, t1 - t0 + 1);
     const int32_t cols_blk = std::max<int32_t>(1, 74 / rows_blk);  // in tile pairs
     for (int32_t tb = t0; tb <= t1; tb += rows_blk) {
       const int32_t te = std::min(t1, tb + rows_blk - 1);
-      for (int32_t pb = 0; 2 * pb <= te; pb += cols_blk)
-        for (int32_t tp = pb; tp < pb + cols_blk && 2 * tp <= te; ++tp)
-          for (int32_t ti = std::max(2 * tp, tb); ti <= te; ++ti) tiles.push_back({ti, 2 * tp});
+      const int32_t tp_end = rect ? (col_tiles + 1) / 2 : te / 2 + 1;  // tile pairs of the super-tile row
+      for (int32_t pb = 0; pb < tp_end; pb += cols_blk)
+        for (int32_t tp = pb; tp < pb + cols_blk && tp < tp_end; ++tp)
+          for (int32_t ti = rect ? tb : std::max(2 * tp, tb); ti <= te; ++ti) tiles.push_back({ti, 2 * tp});
     }
   } else {
     // column-major inside the band: CTAs running together share the few i-tiles of the band and
     // neighbouring j-tiles (L2 reuse of both operands)
-    for (int32_t tj = 0; tj <= t1; ++tj)
-      for (int32_t ti = std::max(tj, t0); ti <= t1; ++ti) tiles.push_back({ti, tj});
+    for (int32_t tj = 0; tj < (rect ? col_tiles : t1 + 1); ++tj)
+      for (int32_t ti = rect ? t0 : std::max(tj, t0); ti <= t1; ++ti) tiles.push_back({ti, tj});
   }
   b.n_tiles = static_cast<int32_t>(tiles.size()) - b.tile_off;
 }
@@ -507,6 +555,24 @@ int64_t frc_debug_capacity_groups(int64_t n_samples, int64_t np, int32_t n_dev, 
   }
   for (size_t k = 0; k < tiles.size(); ++k) { out_tiles[2 * k] = tiles[k].ti; out_tiles[2 * k + 1] = tiles[k].tj; }
   return static_cast<int64_t>(g.size());
+}
+
+// Bands of the query x reference block (frc_create_cross; q0 = n_ref rounded up to 256): same output layout as
+// frc_debug_bands, rows in the staged table (the query rows start at q0).
+int64_t frc_debug_cross_bands(int64_t n_ref, int64_t n_q, int64_t band_rows, int32_t world, int32_t d2h, int32_t per_rank,
+                              int32_t value_bytes, int64_t* out5, int64_t cap) {
+  return write_bands(frc::make_bands_cross(frc::round_up(n_ref, 2 * frc::kTile), n_q, n_ref, band_rows, world, d2h != 0,
+                                           per_rank, value_bytes), out5, cap);
+}
+
+// Tiles of the cross band [row0, row1) (staged rows) against n_ref reference samples: as frc_debug_band_tiles.
+int64_t frc_debug_cross_tiles(int64_t row0, int64_t row1, int64_t n_ref, int32_t pair_tiles, int32_t* out2, int64_t cap) {
+  frc::Band b;
+  b.row0 = row0; b.row1 = row1;
+  std::vector<frc::Tile> tiles;
+  frc::append_band_tiles(b, pair_tiles != 0, tiles, static_cast<int32_t>((n_ref + frc::kTile - 1) / frc::kTile));
+  for (size_t k = 0; k < tiles.size() && static_cast<int64_t>(k) < cap; ++k) { out2[2 * k] = tiles[k].ti; out2[2 * k + 1] = tiles[k].tj; }
+  return static_cast<int64_t>(tiles.size());
 }
 
 // Tiles of the band [row0, row1): writes up to `cap` (ti, tj) pairs; returns the count.

@@ -30,11 +30,17 @@ struct Band {
 //                   one or two per rank when the distances stay in HBM; more when a band would exceed
 //                   96 MB (streamed) / 1.5 GB (kept in HBM).
 std::vector<int64_t> band_boundaries(int64_t N, int64_t requested, int world, bool d2h, int per_rank, int value_bytes);
-// One band per owner in every round of G consecutive bands, greedily balanced (deterministic; the same in
-// every process).
-std::vector<int> band_owners(const std::vector<int64_t>& rows, int world);
+// Owners of bands with these pair counts: one band per owner in every round of G consecutive bands, greedily
+// balanced (deterministic; the same in every process).
+std::vector<int> band_owners(const std::vector<int64_t>& counts, int world);
 // Every non-empty band of the triangle, in flat-index order, with its owner.
 std::vector<Band> make_bands(int64_t N, int64_t requested, int world, bool d2h, int per_rank, int value_bytes);
+// The query x reference block (Geometry in frc_internal.h): bands of whole 128-row query tiles, rows [row0, row1)
+// of the staged table (query rows from q0 on) and flat range [(row0 - q0) * n_ref, (row1 - q0) * n_ref).
+// `requested` counts query rows; the band count and byte caps follow band_boundaries, the owners band_owners.
+// Empty when n_q or n_ref is 0.
+std::vector<Band> make_bands_cross(int64_t q0, int64_t n_q, int64_t n_ref, int64_t requested, int world, bool d2h,
+                                   int per_rank, int value_bytes);
 
 // Sample shards of the embedding: the padded samples [0, np) in n_shards shards of shard_rows samples (whole tiles).
 // A shard sits in its owner's per-sample arrays at [slot * shard_rows, +shard_rows).
@@ -88,8 +94,9 @@ ColumnPlan plan_columns(const double* length, int32_t n_nodes, bool want_i8, int
 
 // Tiles of one band, appended to `tiles`: pair tiles (ti, tj) + (ti, tj + 1), tj even, walked in
 // super-tiles of ~9 tile rows x ~8 tile-pair columns when `pair_tiles` (tensor-core kernel), plain
-// column-major 128 x 128 tiles otherwise (FP32 tile kernel).
-void append_band_tiles(Band& b, bool pair_tiles, std::vector<Tile>& tiles);
+// column-major 128 x 128 tiles otherwise (FP32 tile kernel).  Triangle (col_tiles == 0): tj <= ti;
+// rectangle: every tj < col_tiles (the reference tiles), no diagonal.
+void append_band_tiles(Band& b, bool pair_tiles, std::vector<Tile>& tiles, int32_t col_tiles = 0);
 // Per block of 256 samples: bit 0 = some tile reads its A rows (column samples), bit 1 = its Bh / Bl rows.
 std::vector<uint8_t> operand_need_blocks(const std::vector<Tile>& tiles, int64_t np, bool pair_tiles);
 

@@ -142,10 +142,11 @@ __device__ __forceinline__ void drain_int(uint32_t taddr, uint32_t shift, unsign
 
 // The exact ratios of column sample j (this thread's TMEM lane) and row samples i0 + [0, EPI2_COLS) (its
 // registers), stored from out[off] on (off: band offset of (i0, j)); pairs with U below flag_u_int are flagged.
+template <bool kRect>
 __device__ __forceinline__ void ratio_int(const unsigned long long (&acc)[EPI2_COLS], const long long* __restrict__ r_int,
                                           int64_t i0, int64_t j, int lane, int64_t n_samples, int64_t off,
                                           long long flag_u_int, float* __restrict__ out, uint32_t* __restrict__ flagged,
-                                          unsigned long long* __restrict__ n_flagged) {
+                                          unsigned long long* __restrict__ n_flagged, const Geometry& geo) {
   const long long rj = j < n_samples ? r_int[j] : 0;
   const long long ri_lane = r_int[i0 + lane];
 #pragma unroll
@@ -169,7 +170,7 @@ __device__ __forceinline__ void ratio_int(const unsigned long long (&acc)[EPI2_C
 #pragma unroll
     for (int x = 0; x < 8; ++x) {
       const int64_t i = i0 + n0 + x;
-      if (i < n_samples && j < i) {
+      if (i < n_samples && (kRect ? j < geo.n_ref : j < i)) {
         out[off] = dv[x];  // fp32 is what the ratio is; the host widens (wire.cu)
         // U and V are exact integer sums of the quantised lengths: no cancellation error, so a small d
         // needs no recompute here (identical samples give U = 0 exactly); only the absolute-error rule of
@@ -179,7 +180,7 @@ __device__ __forceinline__ void ratio_int(const unsigned long long (&acc)[EPI2_C
           flagged[slot] = static_cast<uint32_t>(off);
         }
       }
-      off += i;  // row i+1 starts i entries later
+      off += kRect ? geo.n_ref : i;  // row i+1 starts i (rectangle: n_ref) entries later
     }
   }
 }
@@ -188,7 +189,7 @@ __device__ __forceinline__ void ratio_int(const unsigned long long (&acc)[EPI2_C
 // spanning more than 2^16), 2 = u8 planes with 64-bit INTEGER accumulation and an integer / fp32 ratio
 // epilogue: no fp64 instruction at all (every DADD/DFMA stalls its warp for tens of cycles on B200:
 // ncu showed half of the epilogue warps' samples in stall_math on them at 4.5 % fp64-pipe utilisation).
-template <int kMode>
+template <int kMode, bool kRect>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS2, 1)
 k_unweighted_tc2(const __grid_constant__ CUtensorMap mapP, const __grid_constant__ CUtensorMap mapBh,
                  const __grid_constant__ CUtensorMap mapBl, const int32_t* __restrict__ chunk_end,
@@ -197,7 +198,7 @@ k_unweighted_tc2(const __grid_constant__ CUtensorMap mapP, const __grid_constant
                  const long long* __restrict__ r_int, double unit, const Tile* __restrict__ tiles, int32_t n_tiles,
                  int64_t n_samples, int64_t first, float* __restrict__ out, double flag_below,
                  const double* __restrict__ flag_u_ptr, uint32_t* __restrict__ flagged,
-                 unsigned long long* __restrict__ n_flagged, int dbg) {
+                 unsigned long long* __restrict__ n_flagged, int dbg, const Geometry geo) {
   (void)dbg;
   constexpr bool kI8 = kMode != 0;
   constexpr bool kInt = kMode == 2;
@@ -403,13 +404,14 @@ k_unweighted_tc2(const __grid_constant__ CUtensorMap mapP, const __grid_constant
       static_assert(EPI2_COLS == 32, "r[i] is broadcast from lane n");
       if (TL_ON(4)) {
         if (acc[0] == static_cast<Acc>(-1.5)) out[0] = 0.f;
-      } else if (static_cast<int64_t>(tile.tj + static_cast<int>(cta)) * BM + q * 32 < i0 + EPI2_COLS) {  // warp-uniform
-        int64_t off = i0 * (i0 - 1) / 2 - first + j;  // flat index of (i0, j) relative to the band
+      } else if (kRect || static_cast<int64_t>(tile.tj + static_cast<int>(cta)) * BM + q * 32 < i0 + EPI2_COLS) {  // warp-uniform
+        // flat index of (i0, j) relative to the band
+        int64_t off = kRect ? (i0 - geo.q0) * geo.n_ref - first + j : i0 * (i0 - 1) / 2 - first + j;
         // r is padded to a multiple of the tile size: the loads are in range and coalesced.
         // Batches of 8 row samples: first the arithmetic of all 8 (independent chains the scheduler can
         // interleave), then the stores and the (rare) fix-up flags.
         if constexpr (kInt) {
-          ratio_int(acc, r_int, i0, j, lane, n_samples, off, flag_u_int, out, flagged, n_flagged);
+          ratio_int<kRect>(acc, r_int, i0, j, lane, n_samples, off, flag_u_int, out, flagged, n_flagged, geo);
         } else {
           const double rj = j < n_samples ? r[j] : 0.0;
           const double ri_lane = r[i0 + lane];
@@ -428,14 +430,14 @@ k_unweighted_tc2(const __grid_constant__ CUtensorMap mapP, const __grid_constant
 #pragma unroll
             for (int x = 0; x < 8; ++x) {
               const int64_t i = i0 + n0 + x;
-              if (i < n_samples && j < i) {
+              if (i < n_samples && (kRect ? j < geo.n_ref : j < i)) {
                 out[off] = dv[x];  // fp32 is what the ratio is; the host widens (wire.cu)
                 if (dv[x] < flag_d || uv[x] < flag_u) {
                   unsigned long long slot = atomicAdd(n_flagged, 1ULL);
                   flagged[slot] = static_cast<uint32_t>(off);
                 }
               }
-              off += i;  // row i+1 starts i entries later
+              off += kRect ? geo.n_ref : i;  // row i+1 starts i (rectangle: n_ref) entries later
             }
           }
         }
@@ -494,6 +496,7 @@ __device__ __forceinline__ uint32_t mask4(uint32_t nib) {
 }
 }  // namespace bits
 
+template <bool kRect>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(bits::THREADS, 1)
 k_unweighted_bits2(const __grid_constant__ CUtensorMap mapBits, const uint8_t* __restrict__ qa,
                    const uint8_t* __restrict__ qh, const uint8_t* __restrict__ ql,
@@ -501,7 +504,7 @@ k_unweighted_bits2(const __grid_constant__ CUtensorMap mapBits, const uint8_t* _
                    int32_t n_chunks, const long long* __restrict__ r_int, double unit,
                    const Tile* __restrict__ tiles, int32_t n_tiles, int64_t n_samples, int64_t first,
                    float* __restrict__ out, const double* __restrict__ flag_u_ptr,
-                   uint32_t* __restrict__ flagged, unsigned long long* __restrict__ n_flagged) {
+                   uint32_t* __restrict__ flagged, unsigned long long* __restrict__ n_flagged, const Geometry geo) {
   using namespace bits;  // (EPI_WARP0 is written bits::EPI_WARP0: k_unweighted_tc2 has its own)
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw = ptx::smem_u32(smem_raw);
@@ -711,9 +714,10 @@ k_unweighted_bits2(const __grid_constant__ CUtensorMap mapBits, const uint8_t* _
       }
       const int64_t j = static_cast<int64_t>(tile.tj + static_cast<int>(cta)) * BM + q * 32 + lane;
       const int64_t i0 = static_cast<int64_t>(tile.ti) * BN + cg * EPI2_COLS;
-      if (static_cast<int64_t>(tile.tj + static_cast<int>(cta)) * BM + q * 32 < i0 + EPI2_COLS)  // warp-uniform
-        ratio_int(acc, r_int, i0, j, lane, n_samples, i0 * (i0 - 1) / 2 - first + j, flag_u_int, out, flagged,
-                  n_flagged);
+      if (kRect || static_cast<int64_t>(tile.tj + static_cast<int>(cta)) * BM + q * 32 < i0 + EPI2_COLS)  // warp-uniform
+        ratio_int<kRect>(acc, r_int, i0, j, lane, n_samples,
+                         kRect ? (i0 - geo.q0) * geo.n_ref - first + j : i0 * (i0 - 1) / 2 - first + j, flag_u_int,
+                         out, flagged, n_flagged, geo);
     }
   }
 
@@ -734,12 +738,12 @@ enum class Rows {
           // and has a non-zero length
   kBits,  // the bit rows bitsS[np][kp / 32] of the bits feed
 };
-template <Rows kRows>
+template <Rows kRows, bool kRect>
 __global__ void __launch_bounds__(256)
 k_unweighted_fixup(const void* __restrict__ rows, int32_t kp, const double* __restrict__ len_col,
                    const uint32_t* __restrict__ flagged, const unsigned long long* __restrict__ n_flagged,
                    unsigned long long* __restrict__ count_host, int64_t first, float* __restrict__ out,
-                   const Exceptions ex) {
+                   const Exceptions ex, const Geometry geo) {
   const unsigned long long total = *n_flagged;
   if (blockIdx.x == 0 && threadIdx.x == 0) *count_host = total;  // mapped pinned memory
   const int lane = threadIdx.x & 31;
@@ -749,7 +753,7 @@ k_unweighted_fixup(const void* __restrict__ rows, int32_t kp, const double* __re
        w < total; w += warps) {
     const uint32_t off = flagged[w];
     int64_t i, j;
-    pair_of(first + off, i, j);
+    pair_at<kRect>(first + off, geo, i, j);
     double uniq = 0.0, comm = 0.0;
     if constexpr (kRows == Rows::kBits) {
       const uint32_t* bi = static_cast<const uint32_t*>(rows) + i * words;
@@ -850,16 +854,16 @@ bool tc_setup(std::string* err) {
     g_encode = reinterpret_cast<PFN_tmapEncodeTiled>(fn);
   }
   // per device (function attributes live in the device's context): called once per device context
-  cudaError_t e = cudaFuncSetAttribute(k_unweighted_tc2<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM2_BYTES);
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(k_unweighted_tc2<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM2_BYTES);
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(k_unweighted_tc2<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM2_BYTES);
+  cudaError_t e = cudaSuccess;
+  for (auto kernel : {k_unweighted_tc2<0, false>, k_unweighted_tc2<1, false>, k_unweighted_tc2<2, false>,
+                      k_unweighted_tc2<0, true>, k_unweighted_tc2<1, true>, k_unweighted_tc2<2, true>})
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM2_BYTES);
   if (e != cudaSuccess) {
     if (err) *err = std::string("cudaFuncSetAttribute(k_unweighted_tc2): ") + cudaGetErrorString(e);
     return false;
   }
-  e = cudaFuncSetAttribute(k_unweighted_bits2, cudaFuncAttributeMaxDynamicSharedMemorySize, bits::SMEM_BYTES);
+  for (auto kernel : {k_unweighted_bits2<false>, k_unweighted_bits2<true>})
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bits::SMEM_BYTES);
   if (e != cudaSuccess) {
     if (err) *err = std::string("cudaFuncSetAttribute(k_unweighted_bits2): ") + cudaGetErrorString(e);
     return false;
@@ -946,7 +950,7 @@ int tc_chunk_kblocks() {
 }
 
 int launch_unweighted_tc(const TcOperands* ops, const double* r, const Tile* tiles, int32_t n_tiles,
-                         int64_t n_samples, int64_t first, float* out, double flag_below,
+                         int64_t n_samples, int64_t first, const Geometry& geo, float* out, double flag_below,
                          uint32_t* flagged, unsigned long long* n_flagged, int num_sms, cudaStream_t s) {
   if (n_tiles <= 0) return 0;
   // `tiles` lists pair tiles (tj even): one cluster of two CTAs each
@@ -954,28 +958,31 @@ int launch_unweighted_tc(const TcOperands* ops, const double* r, const Tile* til
   const int grid = 2 * (n_tiles < pairs ? n_tiles : pairs);
   const TcChunks& c = ops->chunks;
   if (ops->from_bits) {  // integer mode: U and V are exact, so r and flag_below play no part
-    k_unweighted_bits2<<<grid, bits::THREADS, bits::SMEM_BYTES, s>>>(
+    const auto kernel = geo.rect ? k_unweighted_bits2<true> : k_unweighted_bits2<false>;
+    kernel<<<grid, bits::THREADS, bits::SMEM_BYTES, s>>>(
         ops->mapBits, ops->qa, ops->qh, ops->ql, c.end, c.shift, c.n, ops->r_int, ops->unit, tiles, n_tiles, n_samples,
-        first, out, ops->flag_u, flagged, n_flagged);
+        first, out, ops->flag_u, flagged, n_flagged, geo);
     return 1;
   }
-#define FRC_TC2_ARGS ops->mapP, ops->mapBh, ops->mapBl, c.end, c.scale, c.shift, c.n, c.biased ? 1 : 0, r, ops->r_int, \
-                     ops->unit, tiles, n_tiles, n_samples, first, out, flag_below, ops->flag_u, flagged, n_flagged, ops->dbg
-  if (ops->i8 && ops->r_int) k_unweighted_tc2<2><<<grid, THREADS2, SMEM2_BYTES, s>>>(FRC_TC2_ARGS);
-  else if (ops->i8) k_unweighted_tc2<1><<<grid, THREADS2, SMEM2_BYTES, s>>>(FRC_TC2_ARGS);
-  else k_unweighted_tc2<0><<<grid, THREADS2, SMEM2_BYTES, s>>>(FRC_TC2_ARGS);
-#undef FRC_TC2_ARGS
+  const int mode = ops->i8 && ops->r_int ? 2 : ops->i8 ? 1 : 0;
+  const auto kernel = geo.rect ? (mode == 2 ? k_unweighted_tc2<2, true> : mode == 1 ? k_unweighted_tc2<1, true>
+                                                                                   : k_unweighted_tc2<0, true>)
+                               : (mode == 2 ? k_unweighted_tc2<2, false> : mode == 1 ? k_unweighted_tc2<1, false>
+                                                                                    : k_unweighted_tc2<0, false>);
+  kernel<<<grid, THREADS2, SMEM2_BYTES, s>>>(ops->mapP, ops->mapBh, ops->mapBl, c.end, c.scale, c.shift, c.n,
+                                             c.biased ? 1 : 0, r, ops->r_int, ops->unit, tiles, n_tiles, n_samples, first,
+                                             out, flag_below, ops->flag_u, flagged, n_flagged, ops->dbg, geo);
   return 1;
 }
 
 int launch_unweighted_fixup(const TcOperands* ops, const uint32_t* flagged, const unsigned long long* n_flagged,
-                            unsigned long long* count_host, int64_t first, float* out, const Exceptions& ex,
-                            int num_sms, cudaStream_t s) {
-  const auto kernel = ops->from_bits ? k_unweighted_fixup<Rows::kBits>
-                      : ops->i8      ? k_unweighted_fixup<Rows::kU8>
-                                     : k_unweighted_fixup<Rows::kBf16>;
+                            unsigned long long* count_host, int64_t first, const Geometry& geo, float* out,
+                            const Exceptions& ex, int num_sms, cudaStream_t s) {
+  const auto kernel = ops->from_bits ? (geo.rect ? k_unweighted_fixup<Rows::kBits, true> : k_unweighted_fixup<Rows::kBits, false>)
+                      : ops->i8      ? (geo.rect ? k_unweighted_fixup<Rows::kU8, true> : k_unweighted_fixup<Rows::kU8, false>)
+                                     : (geo.rect ? k_unweighted_fixup<Rows::kBf16, true> : k_unweighted_fixup<Rows::kBf16, false>);
   const void* rows = ops->from_bits ? static_cast<const void*>(ops->bitsS) : ops->P;
-  kernel<<<num_sms * 4, 256, 0, s>>>(rows, ops->kp, ops->len_col, flagged, n_flagged, count_host, first, out, ex);
+  kernel<<<num_sms * 4, 256, 0, s>>>(rows, ops->kp, ops->len_col, flagged, n_flagged, count_host, first, out, ex, geo);
   return 1;
 }
 

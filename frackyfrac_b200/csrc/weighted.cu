@@ -28,6 +28,8 @@
 // the L1 loop -- and forms numer = W_i + W_j - 2 S in fp64.  The int32 key panels K[np/128][kp][128] ride in the
 // same TMA ring as the values, which doubles a stage to 64 KB: the ring is 3 stages deep (192 KB; 6 would need
 // 384 KB).  Keyed panels are always resident in local HBM (no capacity mode), where 2 slabs in flight suffice.
+#include <type_traits>
+
 #include "frc_internal.h"
 #include "ptx.cuh"
 #include "wire.cuh"
@@ -56,12 +58,12 @@ __device__ __forceinline__ const float* panel_of(const PanelMap& m, int32_t t, i
 // Operand staging: one thread issues TMA bulk copies (cp.async.bulk, 16 KB per operand slab: the tile-panel
 // layout makes a slab of 32 nodes x 128 samples contiguous) that complete on an mbarrier per stage.  The
 // FP32-issue-bound inner loop spends no slot on copies and the copy engine keeps the whole ring in flight.
-template <bool kPrescaled, bool kKeyed>
+template <bool kPrescaled, bool kKeyed, bool kRect>
 __global__ void __launch_bounds__(256, 1)
 k_weighted_tiles(const PanelMap A, int64_t ld, int32_t kp, const float* __restrict__ lenf,
                  const double* __restrict__ W, const Tile* __restrict__ tiles, int64_t n_samples,
                  int64_t first, float* __restrict__ out, double flag_below, uint32_t* __restrict__ flagged,
-                 unsigned long long* __restrict__ n_flagged, const int32_t* __restrict__ K) {
+                 unsigned long long* __restrict__ n_flagged, const int32_t* __restrict__ K, const Geometry geo) {
   constexpr int STAGES = kStages<kKeyed>;
   constexpr int STAGE_FLOATS = kStageFloats<kKeyed>;
   extern __shared__ __align__(128) float smem[];
@@ -170,11 +172,11 @@ k_weighted_tiles(const PanelMap A, int64_t ld, int32_t kp, const float* __restri
     const int64_t i = i0 + (a < 4 ? ty * 4 + a : 64 + ty * 4 + (a - 4));
     if (i >= n_samples) continue;
     const double wi = W[i];
-    float* orow = out + (i * (i - 1) / 2 - first);
+    float* orow = kRect ? out + ((i - geo.q0) * geo.n_ref - first) : out + (i * (i - 1) / 2 - first);
 #pragma unroll
     for (int b = 0; b < 8; ++b) {
       const int64_t j = j0 + (b < 4 ? tx * 4 + b : 64 + tx * 4 + (b - 4));
-      if (j < i) {
+      if (kRect ? j < geo.n_ref : j < i) {
         // keyed: the accumulator holds S = sum over matched nodes of len * min(a, b)
         const double num = kKeyed ? (wi + W[j]) - 2.0 * static_cast<double>(tot[a][b] + acc[a][b])
                                   : static_cast<double>(tot[a][b] + acc[a][b]);
@@ -199,7 +201,7 @@ k_weighted_tiles(const PanelMap A, int64_t ld, int32_t kp, const float* __restri
 // ws is one zeroed int64 array of n_nodes entries per CTA.
 // Keyed (-l as coded): a second array per CTA accumulates sum[v] = a_i(v) + a_j(v) the same way, and a touched
 // node adds len * |diff| where the key panels say the two samples match at v, len * sum where they do not.
-template <bool kKeyed>
+template <bool kKeyed, bool kRect>
 __global__ void __launch_bounds__(256)
 k_weighted_fixup(const int64_t* __restrict__ row_ptr, const int32_t* __restrict__ col,
                  const double* __restrict__ val, const int32_t* __restrict__ parent,
@@ -207,7 +209,7 @@ k_weighted_fixup(const int64_t* __restrict__ row_ptr, const int32_t* __restrict_
                  const double* __restrict__ W, const uint32_t* __restrict__ flagged,
                  const unsigned long long* __restrict__ n_flagged, unsigned long long* __restrict__ count_host,
                  int64_t first, long long* __restrict__ ws, float* __restrict__ out, const Exceptions ex,
-                 const int32_t* __restrict__ K, int32_t kp) {
+                 const int32_t* __restrict__ K, int32_t kp, const Geometry geo) {
   __shared__ double red[8];
   const unsigned long long n = *n_flagged;
   if (blockIdx.x == 0 && threadIdx.x == 0) *count_host = n;  // mapped pinned memory
@@ -217,7 +219,7 @@ k_weighted_fixup(const int64_t* __restrict__ row_ptr, const int32_t* __restrict_
   for (unsigned long long w = blockIdx.x; w < n; w += gridDim.x) {
     const uint32_t off = flagged[w];
     int64_t i, j;
-    pair_of(first + off, i, j);
+    pair_at<kRect>(first + off, geo, i, j);
     const int64_t smp[2] = {i, j};
     // without normalisation (-l) raw values are summed: scale them into the fixed-point range
     double inv[2];
@@ -285,39 +287,49 @@ k_weighted_fixup(const int64_t* __restrict__ row_ptr, const int32_t* __restrict_
 
 int launch_weighted_fixup(const DevCsr& a, const DevTree& t, const double* total, const double* W,
                           const uint32_t* flagged, const unsigned long long* n_flagged,
-                          unsigned long long* count_host, int64_t first, long long* ws, int ws_ctas, float* out,
-                          const Exceptions& ex, cudaStream_t s, const int32_t* K, int32_t kp) {
-  if (K)
-    k_weighted_fixup<true><<<ws_ctas, 256, 0, s>>>(a.row_ptr, a.col, a.val, t.parent, t.length, t.n_nodes, total, W,
-                                                   flagged, n_flagged, count_host, first, ws, out, ex, K, kp);
-  else
-    k_weighted_fixup<false><<<ws_ctas, 256, 0, s>>>(a.row_ptr, a.col, a.val, t.parent, t.length, t.n_nodes, total, W,
-                                                    flagged, n_flagged, count_host, first, ws, out, ex, nullptr, 0);
+                          unsigned long long* count_host, int64_t first, const Geometry& geo, long long* ws,
+                          int ws_ctas, float* out, const Exceptions& ex, cudaStream_t s, const int32_t* K, int32_t kp) {
+  const auto kernel = K ? (geo.rect ? k_weighted_fixup<true, true> : k_weighted_fixup<true, false>)
+                        : (geo.rect ? k_weighted_fixup<false, true> : k_weighted_fixup<false, false>);
+  kernel<<<ws_ctas, 256, 0, s>>>(a.row_ptr, a.col, a.val, t.parent, t.length, t.n_nodes, total, W, flagged, n_flagged,
+                                 count_host, first, ws, out, ex, K, K ? kp : 0, geo);
   return 1;
 }
 
 void weighted_setup() {
-  cudaFuncSetAttribute(k_weighted_tiles<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes<false>);
-  cudaFuncSetAttribute(k_weighted_tiles<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes<false>);
-  cudaFuncSetAttribute(k_weighted_tiles<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes<true>);
-  cudaFuncSetAttribute(k_weighted_tiles<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes<true>);
+  auto smem = [](auto kernel, int bytes) { cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes); };
+  smem(k_weighted_tiles<true, false, false>, kSmemBytes<false>);
+  smem(k_weighted_tiles<false, false, false>, kSmemBytes<false>);
+  smem(k_weighted_tiles<true, true, false>, kSmemBytes<true>);
+  smem(k_weighted_tiles<false, true, false>, kSmemBytes<true>);
+  smem(k_weighted_tiles<true, false, true>, kSmemBytes<false>);
+  smem(k_weighted_tiles<false, false, true>, kSmemBytes<false>);
+  smem(k_weighted_tiles<true, true, true>, kSmemBytes<true>);
+  smem(k_weighted_tiles<false, true, true>, kSmemBytes<true>);
 }
 
 int launch_weighted_tiles(const PanelMap& A, int64_t ld, int32_t kp, const float* lenf, bool prescaled,
                           const double* W, const Tile* tiles, int32_t n_tiles, int64_t n_samples,
-                          int64_t first, float* out, double flag_below, uint32_t* flagged,
+                          int64_t first, const Geometry& geo, float* out, double flag_below, uint32_t* flagged,
                           unsigned long long* n_flagged, int num_sms, cudaStream_t s, const int32_t* K) {
   (void)num_sms;
   if (n_tiles <= 0) return 0;
   auto go = [&](auto kernel, int smem) {
-    kernel<<<n_tiles, 256, smem, s>>>(A, ld, kp, lenf, W, tiles, n_samples, first, out, flag_below, flagged, n_flagged, K);
+    kernel<<<n_tiles, 256, smem, s>>>(A, ld, kp, lenf, W, tiles, n_samples, first, out, flag_below, flagged, n_flagged, K,
+                                      geo);
+  };
+  // (the capacity mode, which shards the panels, only runs triangle jobs)
+  auto pick = [&](auto prescaled_c, auto keyed_c) {
+    constexpr bool kP = decltype(prescaled_c)::value, kK = decltype(keyed_c)::value;
+    if (geo.rect) go(k_weighted_tiles<kP, kK, true>, kSmemBytes<kK>);
+    else go(k_weighted_tiles<kP, kK, false>, kSmemBytes<kK>);
   };
   if (K) {
-    if (prescaled) go(k_weighted_tiles<true, true>, kSmemBytes<true>);
-    else go(k_weighted_tiles<false, true>, kSmemBytes<true>);
+    if (prescaled) pick(std::true_type{}, std::true_type{});
+    else pick(std::false_type{}, std::true_type{});
   } else {
-    if (prescaled) go(k_weighted_tiles<true, false>, kSmemBytes<false>);
-    else go(k_weighted_tiles<false, false>, kSmemBytes<false>);
+    if (prescaled) pick(std::true_type{}, std::false_type{});
+    else pick(std::false_type{}, std::false_type{});
   }
   return 1;
 }

@@ -1,4 +1,4 @@
-// Device side of the flat lower triangle and of the fp32 output format (see wire.cu): how a pair kernel
+// Device side of the flat pair index and of the fp32 output format (see wire.cu): how a pair kernel
 // finds the samples of a flat pair index, and how the exact fix-up kernels store a recomputed distance
 // into an fp32 band.
 #pragma once
@@ -15,6 +15,19 @@ __device__ __forceinline__ void pair_of(int64_t p, int64_t& i, int64_t& j) {
   while ((g + 1) * g / 2 <= p) ++g;
   i = g;
   j = p - g * (g - 1) / 2;
+}
+
+// Flat pair index p -> samples (i, j) in the job's geometry (Geometry in frc_internal.h): the triangle's pair_of, or
+// the query x reference block, p = (i - q0) * n_ref + j (query-major).
+template <bool kRect>
+__device__ __forceinline__ void pair_at(int64_t p, const Geometry& g, int64_t& i, int64_t& j) {
+  if constexpr (kRect) {
+    const int64_t q = p / g.n_ref;
+    i = g.q0 + q;
+    j = p - q * g.n_ref;
+  } else {
+    pair_of(p, i, j);
+  }
 }
 
 // out[off] = float(d).  A value fp32 cannot carry to 2^-23 relative (underflow: |d| < 1.2e-38) is also

@@ -29,7 +29,8 @@ COMM_ID_BYTES = 128
 
 NORM_L_AS_CODED, NORM_DEFAULT, NORM_L_DOCUMENTED = 0, 1, 2  # frc_opts_t.normalize
 
-EXPORTS = ["frc_abi_version", "frc_ctx_create", "frc_ctx_create_multi", "frc_ctx_destroy", "frc_create", "frc_next",
+EXPORTS = ["frc_abi_version", "frc_ctx_create", "frc_ctx_create_multi", "frc_ctx_destroy", "frc_create",
+           "frc_create_cross", "frc_next",
            "frc_next_f32", "frc_chunk_exceptions", "frc_restart", "frc_job_info", "frc_destroy", "frc_last_error",
            "frc_plan_bands", "frc_comm_unique_id", "frc_ctx_comm_init"]
 
@@ -112,6 +113,8 @@ def lib():
         L.frc_ctx_destroy.restype = None
         L.frc_create.argtypes = [C.c_void_p, C.POINTER(_Tree), C.POINTER(_Csr), C.POINTER(_Opts),
                                  C.POINTER(C.c_void_p)]
+        L.frc_create_cross.argtypes = [C.c_void_p, C.POINTER(_Tree), C.POINTER(_Csr), C.POINTER(_Csr),
+                                       C.POINTER(_Opts), C.POINTER(C.c_void_p)]
         L.frc_next.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
         L.frc_next_f32.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
         L.frc_chunk_exceptions.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_int64)]
@@ -185,26 +188,35 @@ def comm_unique_id() -> bytes:
     return buf.raw
 
 
+def _csr(keep, row_ptr, col, val):
+    """A _Csr over contiguous copies of the arrays (appended to `keep` so that they outlive the call)."""
+    rp, c, v = (np.ascontiguousarray(row_ptr, np.int64), np.ascontiguousarray(col, np.int32),
+                np.ascontiguousarray(val, np.float64))
+    if len(c) != len(v) or (len(rp) and rp[-1] != len(c)):
+        raise ValueError("CSR arrays are inconsistent")
+    keep += [rp, c, v]
+    return _Csr(max(len(rp) - 1, 0), rp.ctypes.data if len(rp) else None, c.ctypes.data, v.ctypes.data)
+
+
 class Job:
     """One unifrac() call.  Iterate `chunks()` for (first_index, ndarray) runs."""
 
     def __init__(self, parent, length, row_ptr, col, val, *, weighted: bool, normalize=True,
                  path: int = PATH_AUTO, ctx: Context | None = None, device: int = -1, rank: int = 0,
-                 world: int = 1, band_rows: int = 0, flags: int = 0, devices=None):
+                 world: int = 1, band_rows: int = 0, flags: int = 0, devices=None, query=None):
         """normalize: True / 1 = default; False / 0 = flag -l as CODED in the reference (unsorted merge-join:
         the bit-exact list walk, or with flags=FLAG_L_TILES the key-matched FP32 tiles wherever `path` picks the
         fast kernels); 2 = flag -l as documented.  devices: None = one GPU (`device` or the context's);
-        a list of ordinals or -1 (all) = this process drives several GPUs, one ordered stream."""
-        self._keep = [np.ascontiguousarray(parent, np.int32), np.ascontiguousarray(length, np.float64),
-                      np.ascontiguousarray(row_ptr, np.int64), np.ascontiguousarray(col, np.int32),
-                      np.ascontiguousarray(val, np.float64)]
-        p, l, rp, c, v = self._keep
+        a list of ordinals or -1 (all) = this process drives several GPUs, one ordered stream.
+        query: (row_ptr, col, val) of a second table = frc_create_cross: the table above is the reference and the
+        stream is the query-major n_q x n_ref block, flat index q * n_ref + r (band_rows counts query rows)."""
+        self._keep = [np.ascontiguousarray(parent, np.int32), np.ascontiguousarray(length, np.float64)]
+        p, l = self._keep
         if len(p) != len(l):
             raise ValueError("parent and length differ in size")
-        if len(c) != len(v) or (len(rp) and rp[-1] != len(c)):
-            raise ValueError("CSR arrays are inconsistent")
         t = _Tree(len(p), p.ctypes.data, l.ctypes.data)
-        a = _Csr(max(len(rp) - 1, 0), rp.ctypes.data if len(rp) else None, c.ctypes.data, v.ctypes.data)
+        a = _csr(self._keep, row_ptr, col, val)
+        q = None if query is None else _csr(self._keep, *query)
         norm = int(normalize) if not isinstance(normalize, bool) else (1 if normalize else 0)
         ids = None
         if devices is None:
@@ -218,7 +230,11 @@ class Job:
         self.h = C.c_void_p()
         self.flags = flags
         self.ctx = ctx
-        rc = lib().frc_create(ctx.h if ctx else None, C.byref(t), C.byref(a), C.byref(o), C.byref(self.h))
+        if q is None:
+            rc = lib().frc_create(ctx.h if ctx else None, C.byref(t), C.byref(a), C.byref(o), C.byref(self.h))
+        else:
+            rc = lib().frc_create_cross(ctx.h if ctx else None, C.byref(t), C.byref(a), C.byref(q), C.byref(o),
+                                        C.byref(self.h))
         if rc:
             self.h = None
             raise FrcError(rc, lib().frc_last_error(None).decode())
@@ -332,3 +348,14 @@ def unifrac(parent, length, row_ptr, col, val, weighted: bool, normalize=True, *
         for first, a in job.chunks(copy=False):
             out[first:first + len(a)] = a
     return out
+
+
+def unifrac_cross(parent, length, ref, query, weighted: bool, normalize=True, **kw) -> np.ndarray:
+    """The (n_q, n_ref) distances between every query sample and every reference sample (frc_create_cross);
+    ref and query are (row_ptr, col, val) tables over the same tree."""
+    n_ref, n_q = max(len(ref[0]) - 1, 0), max(len(query[0]) - 1, 0)
+    out = np.zeros(n_q * n_ref, np.float64)
+    with Job(parent, length, *ref, weighted=weighted, normalize=normalize, query=query, **kw) as job:
+        for first, a in job.chunks(copy=False):
+            out[first:first + len(a)] = a
+    return out.reshape(n_q, n_ref)

@@ -118,8 +118,19 @@ int main(int argc, char** argv) {
     lap("read table file");
     frchost::Table tab = frchost::parse_table(it.data(), it.size(), fl.sparse, static_cast<int>(fl.nt));  // -p workers (frcfrc.go:42-50)
     lap("parse table");
+    // FRCFRC_QUERY=<table> (stand-in only, like FRCFRC_PRUNE): -i is the reference table and the output is the
+    // query x reference block, (q1,r1) ... (q1,rR), (q2,r1) ... (frc_create_cross); -s applies to both tables
+    const char* fquery = getenv("FRCFRC_QUERY");
+    frchost::Table qtab;
+    if (fquery) {
+      std::string qt = frchost::read_file(fquery);
+      qtab = frchost::parse_table(qt.data(), qt.size(), fl.sparse, static_cast<int>(fl.nt));
+      lap("read + parse query table");
+    }
     fputs("Validating\n", stderr);
     frchost::Csr csr = frchost::resolve(tab, tree, static_cast<int>(fl.nt));
+    frchost::Csr qcsr;
+    if (fquery) qcsr = frchost::resolve(qtab, tree, static_cast<int>(fl.nt));
     lap("validate + resolve");
 
     frchost::Writer w(fl.fout, static_cast<int>(fl.nt));  // aio.Create (frcfrc.go:100-106): ".gz" / ".zst" by suffix
@@ -127,6 +138,7 @@ int main(int argc, char** argv) {
     fputs("Converting abundances\n", stderr);
     frc_tree_t ft{static_cast<int32_t>(tree.parent.size()), tree.parent.data(), tree.length.data()};
     frc_csr_t fc{tab.n_samples(), csr.row_ptr.data(), csr.col.data(), csr.val.data()};
+    frc_csr_t fq{qtab.n_samples(), qcsr.row_ptr.data(), qcsr.col.data(), qcsr.val.data()};
     frc_opts_t fo{};
     fo.mode = fl.wgt ? FRC_WEIGHTED : FRC_UNWEIGHTED;
     // -l: the reference's behaviour as coded (normalize = 0: unifrac.go:108-110 skips the id-sort together with
@@ -147,10 +159,12 @@ int main(int argc, char** argv) {
     // (FRCFRC_DEVICES=n limits it to the first n; tiny inputs are not worth more than one context)
     fo.n_devices = -1;
     if (const char* e = getenv("FRCFRC_DEVICES")) fo.n_devices = std::max(1, atoi(e));
-    else if (static_cast<double>(tab.n_samples()) * static_cast<double>(tab.n_samples()) * static_cast<double>(tree.parent.size()) < 4e12)
+    else if (static_cast<double>(tab.n_samples()) * static_cast<double>(fquery ? qtab.n_samples() : tab.n_samples()) *
+                 static_cast<double>(tree.parent.size()) < 4e12)
       fo.n_devices = 1;
     frc_job_t* job = nullptr;
-    if (frc_create(nullptr, &ft, &fc, &fo, &job) != FRC_OK) die(frc_last_error(nullptr));
+    const int crc = fquery ? frc_create_cross(nullptr, &ft, &fc, &fq, &fo, &job) : frc_create(nullptr, &ft, &fc, &fo, &job);
+    if (crc != FRC_OK) die(frc_last_error(nullptr));
     lap("frc_create (+ CUDA init)");
     fputs("Calculating distances\n", stderr);
     frc_info_t info;

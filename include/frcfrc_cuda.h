@@ -164,7 +164,7 @@ typedef struct {
   int32_t n_bands_total;   /* bands of the whole triangle                       */
   int32_t n_bands_mine;    /* bands this rank yields                            */
   int32_t tree_height;     /* level-synchronous passes of the embedding         */
-  int64_t n_pairs_total;   /* n(n-1)/2                                          */
+  int64_t n_pairs_total;   /* n(n-1)/2 (frc_create_cross: n_q * n_ref)           */
   int64_t n_pairs_mine;
   int64_t n_nodes_padded;  /* contraction length the pair kernel runs over      */
   int64_t kernel_launches; /* kernels of this library launched so far           */
@@ -213,10 +213,33 @@ int frc_ctx_comm_init(frc_ctx_t *ctx, const char *id, int32_t rank, int32_t worl
 int frc_create(frc_ctx_t *ctx, const frc_tree_t *tree, const frc_csr_t *abnd,
                const frc_opts_t *opts, frc_job_t **out);
 
+/* Query x reference distances (an extension: the reference CLI has no such mode).  The job yields the
+ * n_q x n_ref block of distances between every query sample and every reference sample, and nothing else
+ * (no reference x reference or query x query pairs).
+ *   distance  d(q, r) is exactly what frc_create over the concatenated table [ref rows; query rows] gives for
+ *             the pair (i, j) = (n_ref + q, r): the query sample is the FIRST sample of the pair (row i,
+ *             common.go:25), which matters for normalize = 0, whose merge-join is not symmetric in fp.
+ *   stream    frc_next / frc_next_f32 / frc_chunk_exceptions use the flat index q * n_ref + r (query-major),
+ *             contiguous runs in strictly increasing order, one band of whole 128-row query tiles per run;
+ *             frc_restart and FRC_FLAG_NO_D2H work as for frc_create.  frc_job_info: n_pairs_total =
+ *             n_q * n_ref.  n_ref == 0 or n_q == 0 is an empty stream; an empty sample gives NaN.
+ *   options   mode, normalize 0 / 1 / 2, path (AUTO applies its rule to the block's pair count), device,
+ *             n_devices / devices (one ordered stream), band_rows (counted in QUERY rows), and the flags
+ *             FRC_FLAG_NO_D2H, FRC_FLAG_UW_BF16, FRC_FLAG_UW_BITS, FRC_FLAG_L_TILES and FRC_FLAG_PRUNE (the
+ *             support is the union of the leaves both tables list).
+ *   refused   FRC_ERR_UNSUPPORTED for world > 1, FRC_FLAG_SHARD_EMBED, and the capacity mode of the fast
+ *             weighted path over several devices (FRC_CAPACITY=1, or panels beyond about half of one device's
+ *             free HBM).
+ * Both tables get every check of frc_create; the messages name the table and the row within it.  The
+ * argument checks (also the refusals above except the capacity mode) come before any CUDA call. */
+int frc_create_cross(frc_ctx_t *ctx, const frc_tree_t *tree, const frc_csr_t *ref, const frc_csr_t *query,
+                     const frc_opts_t *opts, frc_job_t **out);
+
 /* Replaces ranging over the iter.Seq[float64] that unifrac() returns
  * (frcfrc/frcfrc.go:58-62, unifrac.go:209-228).  Yields contiguous runs of the
  * flat lower-triangle vector, index(i,j) = i(i-1)/2 + j for j < i
- * (common/common.go:21-31), in strictly increasing index order.  `*data` is
+ * (common/common.go:21-31), in strictly increasing index order (frc_create_cross:
+ * the query-major block, index q * n_ref + r).  `*data` is
  * engine-owned pinned host memory (device memory with FRC_FLAG_NO_D2H), valid
  * until the next call on this job.  *count == 0 means the stream has ended.
  * A run is one tile band of the plan (frc_plan_bands) or, for the fast paths on
