@@ -14,20 +14,23 @@
 //
 // Tiling: CTA = 128 x 128 pairs, 256 threads, each an 8 x 8 register block
 // (two 4-wide groups per side, so every shared-memory read is a conflict-free
-// LDS.128).  The contraction is staged through shared memory in 32-node slabs
-// with a 6-deep ring of TMA bulk copies (one 16 KB copy per operand slab).  Accumulation is two-level (flush the 64
-// running sums into 64 totals every 256 nodes) to keep fp32 summation error
-// well under the 1e-5 budget for contractions of 10^5..10^6 nodes.
+// LDS.128).  The contraction is staged through shared memory in slabs of 32 nodes (16 keyed)
+// with a 3-deep ring of TMA bulk copies (one copy per operand slab).  Accumulation is two-level: fp32 running
+// sums over 256 nodes, flushed into fp64 per-pair totals that live in shared memory (128 KB per CTA:
+// they would not fit the registers beside the running sums).  Only the 256-term fp32 level rounds the way a
+// regular input (equal lengths and counts) drives every rounding in one direction: at most 4e-6 relative
+// for constant terms, against the 1e-5 budget, whatever the number of nodes (tests/test_weighted_accuracy.py
+// models this arithmetic).  An fp32 total grew that error with every flush (1.45e-5 at 2^18 nodes).
 //
 // Keyed variant (normalize = 0, flag -l as the reference codes it, FRC_FLAG_L_TILES).  Without the id-sort the
 // reference's merge-join walks post-order lists and pairs nodes up by accident; the outcome has a closed form
 // (DESIGN.md, "-l as coded"): with key_s(v) = the largest present leaf id under v (-1 when v is absent),
 //   numer = sum_v len_v * (key_i(v) == key_j(v) ? |a - b| : a + b),   denom = W_i + W_j.
-// Since |a - b| = a + b - 2 min(a, b) for a, b >= 0, the kernel accumulates S = sum over matched v of
-// len_v * min(a, b) -- ISETP + FMNMX + predicated FADD (FFMA), 3 instructions per (pair, node) against the 2 of
-// the L1 loop -- and forms numer = W_i + W_j - 2 S in fp64.  The int32 key panels K[np/128][kp][128] ride in the
-// same TMA ring as the values, which doubles a stage to 64 KB: the ring is 3 stages deep (192 KB; 6 would need
-// 384 KB).  Keyed panels are always resident in local HBM (no capacity mode), where 2 slabs in flight suffice.
+// Since a, b >= 0, both branches are |a - (match ? b : -b)|: the kernel sums that term directly -- ISETP + FSEL
+// + FADD + FADD, 4 instructions per (pair, node) against the 2 of the L1 loop -- so the numerator never comes from
+// a cancellation (W_i + W_j - 2 * sum of the matched min(a, b) multiplied the error of the sum by (1 - d) / d,
+// about 30 just above the fix-up threshold).  The int32 key panels K[np/128][kp][128] ride in the same TMA ring as
+// the values; a keyed slab is 16 nodes so that its stage (32 KB) leaves room for the fp64 totals.
 #include <type_traits>
 
 #include "frc_internal.h"
@@ -37,15 +40,17 @@
 namespace frc {
 namespace {
 
-constexpr int KT = 32;        // nodes per smem slab
-constexpr int FLUSH = 8;      // slabs between flushes (256 nodes)
-constexpr int SLAB_FLOATS = KT * kTile;             // one operand side: 16 KB
-// ring depth: 5 slabs (160 KB) in flight per CTA, enough to cover NVLink latency in capacity mode; keyed: 3
-// stages of values + keys (64 KB each)
-template <bool kKeyed> constexpr int kStages = kKeyed ? 3 : 6;
-// per stage: the two value slabs, per-node lengths (128 B), keyed: the two key slabs
-template <bool kKeyed> constexpr int kStageFloats = (kKeyed ? 4 : 2) * SLAB_FLOATS + KT;
-template <bool kKeyed> constexpr int kSmemBytes = kStages<kKeyed> * kStageFloats<kKeyed> * 4 + kStages<kKeyed> * 8 + 128;
+constexpr int kFlushNodes = 256;  // nodes per fp32 running sum, between two flushes into the fp64 totals
+template <bool kKeyed> constexpr int kKT = kKeyed ? 16 : 32;       // nodes per smem slab
+template <bool kKeyed> constexpr int kSlabFloats = kKT<kKeyed> * kTile;
+// ring depth: 2 slabs in flight cover the HBM latency (every panel the kernel reads is in local HBM: the
+// capacity mode rotates the remote shards in with the copy engines)
+constexpr int kStages = 3;
+// per stage: the two value slabs, per-node lengths, keyed: the two key slabs
+template <bool kKeyed> constexpr int kStageFloats = (kKeyed ? 4 : 2) * kSlabFloats<kKeyed> + kKT<kKeyed>;
+constexpr int kTotBytes = 64 * 256 * 8;  // fp64 totals: 64 pairs per thread
+template <bool kKeyed> constexpr int kSmemBytes = kTotBytes + kStages * kStageFloats<kKeyed> * 4 + kStages * 8 + 128;
+static_assert(kSmemBytes<false> <= 227 * 1024 && kSmemBytes<true> <= 227 * 1024, "shared memory per CTA");
 
 // Panel of sample tile t (PanelMap in frc_internal.h): the one local array, or the place its shard currently
 // occupies in this device's HBM.
@@ -64,16 +69,23 @@ k_weighted_tiles(const PanelMap A, int64_t ld, int32_t kp, const float* __restri
                  const double* __restrict__ W, const Tile* __restrict__ tiles, int64_t n_samples,
                  int64_t first, float* __restrict__ out, double flag_below, uint32_t* __restrict__ flagged,
                  unsigned long long* __restrict__ n_flagged, const int32_t* __restrict__ K, const Geometry geo) {
-  constexpr int STAGES = kStages<kKeyed>;
+  constexpr int STAGES = kStages;
   constexpr int STAGE_FLOATS = kStageFloats<kKeyed>;
+  constexpr int KT = kKT<kKeyed>;
+  constexpr int SLAB_FLOATS = kSlabFloats<kKeyed>;
+  constexpr int FLUSH = kFlushNodes / KT;  // slabs between flushes
   extern __shared__ __align__(128) float smem[];
+  // the fp64 totals of this thread's 64 pairs: tot[e * 256 + tid] (a warp's loads and stores are contiguous),
+  // then the ring
+  double* const tot = reinterpret_cast<double*>(smem);
+  float* const ring = smem + kTotBytes / 4;
   const Tile tile = tiles[blockIdx.x];
   const int64_t i0 = static_cast<int64_t>(tile.ti) * kTile;
   const int64_t j0 = static_cast<int64_t>(tile.tj) * kTile;
   const int tid = threadIdx.x;
   const int tx = tid & 15, ty = tid >> 4;
   const int n_slabs = kp / KT;
-  const uint32_t bar0 = ptx::smem_u32(smem + STAGES * STAGE_FLOATS);
+  const uint32_t bar0 = ptx::smem_u32(ring + STAGES * STAGE_FLOATS);
   (void)ld;
 
   // tile-panel layout [kp][128] per sample tile
@@ -84,7 +96,7 @@ k_weighted_tiles(const PanelMap A, int64_t ld, int32_t kp, const float* __restri
   const int32_t* const kb_g = kKeyed ? K + static_cast<int64_t>(tile.tj) * kp * kTile : nullptr;
   auto issue = [&](int slab) {  // thread 0 only
     const int stage = slab % STAGES;
-    float* sa = smem + stage * STAGE_FLOATS;
+    float* sa = ring + stage * STAGE_FLOATS;
     const uint32_t bar = bar0 + 8u * stage;
     constexpr uint32_t kSlabBytes = SLAB_FLOATS * 4;
     ptx::mbar_expect_tx(bar, (kKeyed ? 4 : 2) * kSlabBytes + (kPrescaled ? 0u : KT * 4u));
@@ -105,18 +117,18 @@ k_weighted_tiles(const PanelMap A, int64_t ld, int32_t kp, const float* __restri
   if (tid == 0)
     for (int p = 0; p < STAGES - 1 && p < n_slabs; ++p) issue(p);
 
-  float acc[8][8], tot[8][8];
+  float acc[8][8];
 #pragma unroll
   for (int a = 0; a < 8; ++a)
 #pragma unroll
-    for (int b = 0; b < 8; ++b) { acc[a][b] = 0.f; tot[a][b] = 0.f; }
+    for (int b = 0; b < 8; ++b) { acc[a][b] = 0.f; tot[(a * 8 + b) * 256 + tid] = 0.0; }
 
   for (int slab = 0; slab < n_slabs; ++slab) {
     // the stage that slab + STAGES - 1 goes to was read in the previous iteration (barrier at its end)
     if (tid == 0 && slab + STAGES - 1 < n_slabs) issue(slab + STAGES - 1);
     const int stage = slab % STAGES;
     ptx::mbar_wait(bar0 + 8u * stage, static_cast<uint32_t>((slab / STAGES) & 1));
-    const float* sa = smem + stage * STAGE_FLOATS;
+    const float* sa = ring + stage * STAGE_FLOATS;
     const float* sb = sa + SLAB_FLOATS;
     const float* sl = sb + SLAB_FLOATS;
     const int32_t* ska = reinterpret_cast<const int32_t*>(sl + KT);
@@ -140,11 +152,12 @@ k_weighted_tiles(const PanelMap A, int64_t ld, int32_t kp, const float* __restri
 #pragma unroll
         for (int a = 0; a < 8; ++a)
 #pragma unroll
-          for (int b = 0; b < 8; ++b)
-            if (ka[a] == kb[b]) {
-              if (kPrescaled) acc[a][b] += fminf(av[a], bv[b]);
-              else acc[a][b] = fmaf(l, fminf(av[a], bv[b]), acc[a][b]);
-            }
+          for (int b = 0; b < 8; ++b) {
+            // matched: |a - b|; otherwise a + b = |a - (-b)| (a, b >= 0)
+            const float t = fabsf(av[a] - (ka[a] == kb[b] ? bv[b] : -bv[b]));
+            if (kPrescaled) acc[a][b] += t;
+            else acc[a][b] = fmaf(l, t, acc[a][b]);
+          }
       } else if (kPrescaled) {
 #pragma unroll
         for (int a = 0; a < 8; ++a)
@@ -162,7 +175,10 @@ k_weighted_tiles(const PanelMap A, int64_t ld, int32_t kp, const float* __restri
 #pragma unroll
       for (int a = 0; a < 8; ++a)
 #pragma unroll
-        for (int b = 0; b < 8; ++b) { tot[a][b] += acc[a][b]; acc[a][b] = 0.f; }
+        for (int b = 0; b < 8; ++b) {
+          tot[(a * 8 + b) * 256 + tid] += static_cast<double>(acc[a][b]);
+          acc[a][b] = 0.f;
+        }
     }
     __syncthreads();  // every thread is done with this stage: it may be refilled
   }
@@ -177,12 +193,10 @@ k_weighted_tiles(const PanelMap A, int64_t ld, int32_t kp, const float* __restri
     for (int b = 0; b < 8; ++b) {
       const int64_t j = j0 + (b < 4 ? tx * 4 + b : 64 + tx * 4 + (b - 4));
       if (kRect ? j < geo.n_ref : j < i) {
-        // keyed: the accumulator holds S = sum over matched nodes of len * min(a, b)
-        const double num = kKeyed ? (wi + W[j]) - 2.0 * static_cast<double>(tot[a][b] + acc[a][b])
-                                  : static_cast<double>(tot[a][b] + acc[a][b]);
+        const double num = tot[(a * 8 + b) * 256 + tid] + static_cast<double>(acc[a][b]);
         const double d = num / (wi + W[j]);
         orow[j] = static_cast<float>(d);  // fp32 numerator: fp32 is what the value carries (wire.cu)
-        // fp32 operands carry 6e-8 relative error each, so the L1 numerator is off by up to
+        // fp32 operands carry 6e-8 relative error each, so the numerator (L1 or keyed) is off by up to
         // 6e-8 * (W_i + W_j) = 6e-8 / d relative: small distances are recomputed (k_weighted_fixup)
         if (d < flag_below) {
           unsigned long long slot = atomicAdd(n_flagged, 1ULL);
