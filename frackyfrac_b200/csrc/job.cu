@@ -175,16 +175,25 @@ struct frc_ctx {
 
 namespace {
 
+// What the pair stage of a fast path writes: fp32 distances, the pairs flagged for the fix-up, their count (mapped
+// pinned, published by the fix-up) and the distances fp32 cannot carry.  A ring slot owns one for its band; in
+// capacity mode a row-shard group owns one for all of its bands.
+struct PairOut {
+  float* dev32 = nullptr;
+  uint32_t* flagged = nullptr;
+  unsigned long long* n_flagged_host = nullptr;
+  Exceptions ex;          // mapped pinned
+  bool counted = false;   // its counts have been added to the part's info on this pass
+};
+
 struct Slot {
   double* dev64 = nullptr;   // exact path: the band in HBM / its pinned landing buffer
   double* host64 = nullptr;
-  float* dev32 = nullptr;    // fast paths
-  float* host32 = nullptr;
-  uint32_t* flagged = nullptr;
-  unsigned long long* n_flagged_host = nullptr;
-  Exceptions ex;             // mapped pinned
+  float* host32 = nullptr;   // fast paths: the pinned landing buffer
+  PairOut own;               // fast paths outside capacity mode
+  PairOut* out = nullptr;    // fast paths: the record the slot's band lives in (`own` or its group's), from out_off on
+  int64_t out_off = 0;
   cudaEvent_t k0 = nullptr, k1 = nullptr, k2 = nullptr, done = nullptr;
-  int band = -1;  // index into mine[]
 };
 
 struct Seg { size_t off = 0, bytes = 0; };
@@ -261,13 +270,8 @@ struct Part {
     int64_t first = 0, count = 0;  // flat range of the group's rows
     int32_t tile_off = 0;          // into the part's tile list
     std::vector<int32_t> coff;     // tile offset (inside the group's list) of every column shard, + end
-    float* out = nullptr;
-    uint32_t* flagged = nullptr;
-    unsigned long long* cnt = nullptr;  // device counter of flagged pairs
-    unsigned long long* n_flagged_host = nullptr;
-    Exceptions ex;
+    PairOut out;
     cudaEvent_t done = nullptr;
-    bool counted = false;          // its flagged / exception counts have been added to the job's info
   };
   std::vector<CapGroup> cap;
   std::vector<int> band_group;     // per band of this part: index into cap
@@ -281,7 +285,7 @@ struct Part {
   Tile* d_tiles = nullptr;
   int32_t* d_level_ptr = nullptr;
   int32_t* d_post = nullptr;
-  unsigned long long* d_flag_counts = nullptr;  // one per band of this part
+  unsigned long long* d_flag_counts = nullptr;  // one per band of this part (capacity mode: per group)
   int64_t ws_slab = 0;
   bool peer_push = false;     // multi-process sharding: the bits kernel stores into every rank's bitsT over IPC mappings
   uint32_t* d_bits2[2] = {nullptr, nullptr};  // (double-buffered by run parity: a rank may be one pass ahead)
@@ -379,6 +383,20 @@ T* pin_alloc(Part* p, size_t n) {
     p->rc = FRC_ERR_OOM;
   }
   return static_cast<T*>(q);
+}
+
+// A PairOut for n pairs.
+int alloc_pair_out(Part* p, PairOut& o, int64_t n) {
+  if (!(o.dev32 = dev_alloc<float>(p, n))) return p->rc;
+  if (!(o.flagged = dev_alloc<uint32_t>(p, n))) return p->rc;
+  if (!(o.n_flagged_host = pin_alloc<unsigned long long>(p, 1))) return p->rc;
+  *o.n_flagged_host = 0;
+  if (!(o.ex.count = pin_alloc<unsigned long long>(p, 1))) return p->rc;
+  if (!(o.ex.index = pin_alloc<int64_t>(p, kMaxExceptions))) return p->rc;
+  if (!(o.ex.value = pin_alloc<double>(p, kMaxExceptions))) return p->rc;
+  o.ex.cap = kMaxExceptions;
+  *o.ex.count = 0;
+  return FRC_OK;
 }
 
 // Runs fn(part index) for every part: on the pool when there are several (each task binds its own
@@ -668,6 +686,51 @@ int embed_stage2(Part* p) {
   return FRC_OK;
 }
 
+// Fast paths: the tile kernel over n tiles into record o, whose first pair has flat index `first`; *cnt counts the
+// flagged pairs.  (pm: where the weighted panels are; the capacity mode passes the visiting shards.)
+int launch_tiles(Part* p, const PanelMap& pm, const Tile* tiles, int32_t n, int64_t first, const PairOut& o,
+                 unsigned long long* cnt, cudaStream_t s) {
+  const Shared& sh = *p->sh;
+  if (sh.weighted)
+    return launch_weighted_tiles(pm, sh.np, sh.kp, p->d_lenf, sh.prescale, p->d_W, tiles, n, sh.N, first, sh.geo, o.dev32,
+                                 kFlagBelowW, o.flagged, cnt, p->dc->num_sms, s, p->d_K);
+  return launch_unweighted_tc(p->tc, p->d_r, tiles, n, sh.N, first, sh.geo, o.dev32, kFlagBelow, o.flagged, cnt,
+                              p->dc->num_sms, s);
+}
+
+// ... and the fix-up of the pairs it flagged (ws: the weighted fix-up's workspace).
+int launch_fixup(Part* p, const PairOut& o, const unsigned long long* cnt, int64_t first, long long* ws, cudaStream_t s) {
+  const Shared& sh = *p->sh;
+  if (sh.weighted)
+    return launch_weighted_fixup(p->dcsr, p->dtree, sh.opts.normalize == 1 ? p->d_total : nullptr, p->d_W, o.flagged, cnt,
+                                 o.n_flagged_host, first, sh.geo, ws, kFixupCtas, o.dev32, o.ex, s, p->d_K, sh.kp);
+  return launch_unweighted_fixup(p->tc, o.flagged, cnt, o.n_flagged_host, first, sh.geo, o.dev32, o.ex, p->dc->num_sms, s);
+}
+
+// Queue the way of band mine[idx] to the host on stream s, after `ready` unless that is null: the D2H into its slot,
+// the slot's `done` event and, after the part's last band, the join of the streams and the end-of-run stamp.
+int hand_off_band(Part* p, size_t idx, cudaEvent_t ready, cudaStream_t s) {
+  const Shared& sh = *p->sh;
+  DevCtx* dc = p->dc;
+  const Slot& sl = p->slots[idx % p->n_slots];
+  if (ready) PART_CUDA(p, cudaStreamWaitEvent(s, ready, 0));
+  if (sh.d2h) {
+    const int64_t bytes = (sh.exact ? sizeof(double) : sizeof(float)) * p->bands[idx].count;
+    if (sh.exact) PART_CUDA(p, cudaMemcpyAsync(sl.host64, sl.dev64, bytes, cudaMemcpyDeviceToHost, s));
+    else PART_CUDA(p, cudaMemcpyAsync(sl.host32, sl.out->dev32 + sl.out_off, bytes, cudaMemcpyDeviceToHost, s));
+    p->info.d2h_bytes += bytes;
+  }
+  PART_CUDA(p, cudaEventRecord(sl.done, s));
+  if (idx + 1 == p->mine.size()) {
+    // last band queued: join all streams and stamp the end of the run on stream 0
+    PART_CUDA(p, cudaEventRecord(p->ev_join, dc->stream[1]));
+    PART_CUDA(p, cudaStreamWaitEvent(dc->stream[0], p->ev_join, 0));
+    PART_CUDA(p, cudaStreamWaitEvent(dc->stream[0], sl.done, 0));
+    PART_CUDA(p, cudaEventRecord(p->ev_run1, dc->stream[0]));
+  }
+  return FRC_OK;
+}
+
 // Queue band mine[idx] of the part into its slot.
 int enqueue_band(Part* p, size_t idx) {
   const Shared& sh = *p->sh;
@@ -679,28 +742,13 @@ int enqueue_band(Part* p, size_t idx) {
   Slot& sl = p->slots[idx % p->n_slots];
   const int si = static_cast<int>(idx % 2);
   cudaStream_t s = dc->stream[si];
-  sl.band = static_cast<int>(idx);
   int launches = 0;
   if (sh.capacity) {
-    // the band was (or is being) computed by the rotation; what is queued here is its way to the host
+    // the band was (or is being) computed by the rotation into its group's record
     Part::CapGroup& cb = p->cap[p->band_group[idx]];
-    cudaStream_t cs = dc->stream[2];
-    float* band_out = cb.out + (b.first - cb.first);
-    sl.dev32 = band_out; sl.flagged = cb.flagged; sl.ex = cb.ex;
-    sl.n_flagged_host = cb.counted ? nullptr : cb.n_flagged_host;  // (a group's count is reported once)
-    cb.counted = true;
-    PART_CUDA(p, cudaStreamWaitEvent(cs, cb.done, 0));
-    for (cudaEvent_t e : {sl.k0, sl.k1, sl.k2}) PART_CUDA(p, cudaEventRecord(e, cs));
-    if (sh.d2h) {
-      PART_CUDA(p, cudaMemcpyAsync(sl.host32, band_out, sizeof(float) * b.count, cudaMemcpyDeviceToHost, cs));
-      p->info.d2h_bytes += static_cast<int64_t>(sizeof(float)) * b.count;
-    }
-    PART_CUDA(p, cudaEventRecord(sl.done, cs));
-    if (idx + 1 == p->mine.size()) {
-      PART_CUDA(p, cudaStreamWaitEvent(dc->stream[0], sl.done, 0));
-      PART_CUDA(p, cudaEventRecord(p->ev_run1, dc->stream[0]));
-    }
-    return FRC_OK;
+    sl.out = &cb.out;
+    sl.out_off = b.first - cb.first;
+    return hand_off_band(p, idx, cb.done, dc->stream[2]);
   }
   PART_CUDA(p, cudaEventRecord(sl.k0, s));
   if (sh.exact) {
@@ -716,51 +764,20 @@ int enqueue_band(Part* p, size_t idx) {
     // previous band's bulk D2H and stall this band (measured).  Counters are per band, zeroed once
     // per run; the fix-up kernel publishes the count through mapped pinned memory.
     unsigned long long* cnt = p->d_flag_counts + idx;
-    *sl.ex.count = 0;  // (the slot's previous band has been delivered)
-    if (sh.weighted) {
-      launches += launch_weighted_tiles(p->pm, sh.np, sh.kp, p->d_lenf, sh.prescale, p->d_W, p->d_tiles + b.tile_off,
-                                        b.n_tiles, sh.N, b.first, sh.geo, sl.dev32, kFlagBelowW, sl.flagged, cnt,
-                                        dc->num_sms, s, p->d_K);
-      PART_CUDA(p, cudaEventRecord(sl.k1, s));
-      // (one workspace per compute stream: consecutive bands run their fix-ups concurrently)
-      launches += launch_weighted_fixup(p->dcsr, p->dtree, sh.opts.normalize == 1 ? p->d_total : nullptr, p->d_W,
-                                        sl.flagged, cnt, sl.n_flagged_host, b.first, sh.geo, p->d_fix_ws[si], kFixupCtas,
-                                        sl.dev32, sl.ex, s, p->d_K, sh.kp);
-    } else {
-      launches += launch_unweighted_tc(p->tc, p->d_r, p->d_tiles + b.tile_off, b.n_tiles, sh.N, b.first, sh.geo,
-                                       sl.dev32, kFlagBelow, sl.flagged, cnt, dc->num_sms, s);
-      PART_CUDA(p, cudaEventRecord(sl.k1, s));
-      launches += launch_unweighted_fixup(p->tc, sl.flagged, cnt, sl.n_flagged_host, b.first, sh.geo, sl.dev32, sl.ex,
-                                          dc->num_sms, s);
-    }
+    sl.out = &sl.own;      // (at offset 0)
+    *sl.own.ex.count = 0;  // (the slot's previous band has been delivered)
+    sl.own.counted = false;
+    launches += launch_tiles(p, p->pm, p->d_tiles + b.tile_off, b.n_tiles, b.first, sl.own, cnt, s);
+    PART_CUDA(p, cudaEventRecord(sl.k1, s));
+    // (one weighted workspace per compute stream: consecutive bands run their fix-ups concurrently)
+    launches += launch_fixup(p, sl.own, cnt, b.first, p->d_fix_ws[si], s);
   }
   PART_CUDA(p, cudaGetLastError());
   PART_CUDA(p, cudaEventRecord(sl.k2, s));
+  p->info.kernel_launches += launches;
   // bulk D2H runs on its own stream so the compute streams never hold copy-engine work
   // (a kernel queued behind a copy in the same stream cannot overlap that copy)
-  if (sh.d2h) {
-    cudaStream_t cs = dc->stream[2];
-    PART_CUDA(p, cudaStreamWaitEvent(cs, sl.k2, 0));
-    if (sh.exact) {
-      PART_CUDA(p, cudaMemcpyAsync(sl.host64, sl.dev64, sizeof(double) * b.count, cudaMemcpyDeviceToHost, cs));
-      p->info.d2h_bytes += static_cast<int64_t>(sizeof(double)) * b.count;
-    } else {
-      PART_CUDA(p, cudaMemcpyAsync(sl.host32, sl.dev32, sizeof(float) * b.count, cudaMemcpyDeviceToHost, cs));
-      p->info.d2h_bytes += static_cast<int64_t>(sizeof(float)) * b.count;
-    }
-    PART_CUDA(p, cudaEventRecord(sl.done, cs));
-  } else {
-    PART_CUDA(p, cudaEventRecord(sl.done, s));
-  }
-  p->info.kernel_launches += launches;
-  if (idx + 1 == p->mine.size()) {
-    // last band queued: join all streams and stamp the end of the run on stream 0
-    PART_CUDA(p, cudaEventRecord(p->ev_join, dc->stream[1]));
-    PART_CUDA(p, cudaStreamWaitEvent(dc->stream[0], p->ev_join, 0));
-    PART_CUDA(p, cudaStreamWaitEvent(dc->stream[0], sl.done, 0));
-    PART_CUDA(p, cudaEventRecord(p->ev_run1, dc->stream[0]));
-  }
-  return FRC_OK;
+  return sh.d2h ? hand_off_band(p, idx, sl.k2, dc->stream[2]) : hand_off_band(p, idx, nullptr, s);
 }
 
 // Capacity mode of the fast weighted path: queue the WHOLE pair stage of this part.  The column shards
@@ -780,8 +797,7 @@ int start_pairs_capacity(Part* p) {
   PanelMap pm = p->pm;  // own shards set by the embedding stage
   int prev_user[2] = {-1, -1};
   int64_t fetched = 0;
-  for (Part::CapGroup& cb : p->cap) { *cb.ex.count = 0; cb.counted = false; }
-  PART_CUDA(p, cudaMemsetAsync(p->cap[0].cnt, 0, sizeof(unsigned long long) * p->cap.size(), s));
+  for (Part::CapGroup& cb : p->cap) { *cb.out.ex.count = 0; cb.out.counted = false; }
   for (int c = 0; c <= last_c; ++c) {
     const bool remote = sp.owner[c] != p->index;
     if (remote) {
@@ -797,15 +813,14 @@ int start_pairs_capacity(Part* p) {
       prev_user[buf] = c;
       fetched += static_cast<int64_t>(shard_floats * sizeof(float));
     }
-    for (Part::CapGroup& cb : p->cap) {
+    for (size_t k = 0; k < p->cap.size(); ++k) {
+      const Part::CapGroup& cb = p->cap[k];
       if (cb.shard < c) continue;
+      unsigned long long* cnt = p->d_flag_counts + k;  // (zeroed with the bands' counters: a part has no fewer bands)
       const int32_t t0 = cb.coff[c], n = cb.coff[c + 1] - cb.coff[c];
-      launches += launch_weighted_tiles(pm, sh.np, sh.kp, p->d_lenf, sh.prescale, p->d_W, p->d_tiles + cb.tile_off + t0, n,
-                                        sh.N, cb.first, sh.geo, cb.out, kFlagBelowW, cb.flagged, cb.cnt, dc->num_sms, s);
+      launches += launch_tiles(p, pm, p->d_tiles + cb.tile_off + t0, n, cb.first, cb.out, cnt, s);
       if (cb.shard == c) {
-        launches += launch_weighted_fixup(p->dcsr, p->dtree, sh.opts.normalize == 1 ? p->d_total : nullptr, p->d_W,
-                                          cb.flagged, cb.cnt, cb.n_flagged_host, cb.first, sh.geo, p->d_fix_ws[0],
-                                          kFixupCtas, cb.out, cb.ex, s);
+        launches += launch_fixup(p, cb.out, cnt, cb.first, p->d_fix_ws[0], s);
         PART_CUDA(p, cudaEventRecord(cb.done, s));
       }
     }
@@ -1404,21 +1419,8 @@ int prepare_part(Part* p) {
           PART_CUDA(p, cudaEventCreateWithFlags(&p->ev_fetch[k], cudaEventDisableTiming));
           PART_CUDA(p, cudaEventCreateWithFlags(&p->ev_used[k], cudaEventDisableTiming));
         }
-        unsigned long long* cnts = dev_alloc<unsigned long long>(p, p->cap.size() + 1);
-        if (!cnts) return p->rc;
-        for (size_t k = 0; k < p->cap.size(); ++k) {
-          Part::CapGroup& cb = p->cap[k];
-          const size_t cnt = static_cast<size_t>(cb.count);
-          cb.cnt = cnts + k;
-          if (!(cb.out = dev_alloc<float>(p, cnt))) return p->rc;
-          if (!(cb.flagged = dev_alloc<uint32_t>(p, cnt))) return p->rc;
-          if (!(cb.n_flagged_host = pin_alloc<unsigned long long>(p, 1))) return p->rc;
-          *cb.n_flagged_host = 0;
-          if (!(cb.ex.count = pin_alloc<unsigned long long>(p, 1))) return p->rc;
-          if (!(cb.ex.index = pin_alloc<int64_t>(p, kMaxExceptions))) return p->rc;
-          if (!(cb.ex.value = pin_alloc<double>(p, kMaxExceptions))) return p->rc;
-          cb.ex.cap = kMaxExceptions;
-          *cb.ex.count = 0;
+        for (Part::CapGroup& cb : p->cap) {
+          if (alloc_pair_out(p, cb.out, cb.count)) return p->rc;
           PART_CUDA(p, cudaEventCreateWithFlags(&cb.done, cudaEventDisableTiming));
         }
       }
@@ -1505,20 +1507,10 @@ int prepare_part(Part* p) {
     if (sh.exact) {
       if (!(sl.dev64 = dev_alloc<double>(p, p->max_band))) return p->rc;
       if (sh.d2h && !(sl.host64 = pin_alloc<double>(p, p->max_band))) return p->rc;
-    } else if (sh.capacity) {
-      // (device buffers, flag lists and exception lists belong to the row-shard groups: Part::CapGroup)
-      if (sh.d2h && !(sl.host32 = pin_alloc<float>(p, p->max_band))) return p->rc;
     } else {
-      if (!(sl.dev32 = dev_alloc<float>(p, p->max_band))) return p->rc;
       if (sh.d2h && !(sl.host32 = pin_alloc<float>(p, p->max_band))) return p->rc;
-      if (!(sl.flagged = dev_alloc<uint32_t>(p, p->max_band))) return p->rc;
-      if (!(sl.n_flagged_host = pin_alloc<unsigned long long>(p, 1))) return p->rc;
-      *sl.n_flagged_host = 0;
-      if (!(sl.ex.count = pin_alloc<unsigned long long>(p, 1))) return p->rc;
-      if (!(sl.ex.index = pin_alloc<int64_t>(p, kMaxExceptions))) return p->rc;
-      if (!(sl.ex.value = pin_alloc<double>(p, kMaxExceptions))) return p->rc;
-      sl.ex.cap = kMaxExceptions;
-      *sl.ex.count = 0;
+      // (capacity mode: a band lives in its row-shard group's record, Part::CapGroup)
+      if (!sh.capacity && alloc_pair_out(p, sl.own, p->max_band)) return p->rc;
     }
     for (cudaEvent_t* e : {&sl.k0, &sl.k1, &sl.k2, &sl.done}) PART_CUDA(p, cudaEventCreate(e));
   }
@@ -1924,7 +1916,8 @@ int part_wait_band(Part* p, size_t idx, Slot** out) {
   const auto tn0 = std::chrono::steady_clock::now();
   PART_CUDA(p, cudaEventSynchronize(sl.done));
   float ms = 0.f;
-  if (p->mine.size() <= 2 || sh.knobs.trace) {
+  const bool spans = !sh.capacity;  // (capacity mode: a group's kernels serve all of its bands; no per-band span)
+  if (spans && (p->mine.size() <= 2 || sh.knobs.trace)) {
     // per-band kernel spans (info.pairs_ms / fixup_ms): meaningful for a job of one or two bands (bench.py's
     // roofline leg); a many-band stream skips the four driver calls per band on the consumer's thread
     PART_CUDA(p, cudaEventElapsedTime(&ms, sl.k0, sl.k1));
@@ -1938,19 +1931,23 @@ int part_wait_band(Part* p, size_t idx, Slot** out) {
     p->info.run_ms = ms;
     p->run_timed = true;
   }
-  if (sl.n_flagged_host) p->info.flagged_pairs += static_cast<int64_t>(*sl.n_flagged_host);
-  if (sl.ex.count) {
-    const unsigned long long n = *sl.ex.count;
-    if (n > static_cast<unsigned long long>(sl.ex.cap))
-      return pfail(p, FRC_ERR_UNSUPPORTED, "more than " + std::to_string(sl.ex.cap) + " distances of one band lie below "
+  if (sl.out && !sl.out->counted) {  // (the record's work has completed; a group's record holds several bands)
+    PairOut& o = *sl.out;
+    o.counted = true;
+    p->info.flagged_pairs += static_cast<int64_t>(*o.n_flagged_host);
+    const unsigned long long n = *o.ex.count;
+    if (n > static_cast<unsigned long long>(o.ex.cap))
+      return pfail(p, FRC_ERR_UNSUPPORTED, "more than " + std::to_string(o.ex.cap) + " distances of one band lie below "
                                            "fp32's range (|d| < 1.2e-38): run this input with path = FRC_PATH_EXACT");
-    if (!sh.capacity || sl.n_flagged_host) p->info.exceptions += static_cast<int64_t>(n);  // (capacity: once per group)
+    p->info.exceptions += static_cast<int64_t>(n);
   }
   if (sh.knobs.trace) {
     float a = 0, b = 0, c2 = 0, d = 0;
-    cudaEventElapsedTime(&a, p->ev_embed0, sl.k0);
-    cudaEventElapsedTime(&b, p->ev_embed0, sl.k1);
-    cudaEventElapsedTime(&c2, p->ev_embed0, sl.k2);
+    if (spans) {
+      cudaEventElapsedTime(&a, p->ev_embed0, sl.k0);
+      cudaEventElapsedTime(&b, p->ev_embed0, sl.k1);
+      cudaEventElapsedTime(&c2, p->ev_embed0, sl.k2);
+    }
     cudaEventElapsedTime(&d, p->ev_embed0, sl.done);
     fprintf(stderr, "[dev %d band %3zu] host: deliver at %.3f ms after waiting %.1f us; device: start %.3f kernel_end %.3f "
                     "fixup_end %.3f d2h_end %.3f ms (pairs %lld)\n", p->dc->device, idx,
@@ -1985,10 +1982,11 @@ void widen_piece(frc_job* j, const Slot& sl, int64_t band_first, int64_t off, in
       ch = T + nx->fetch_add(1, std::memory_order_relaxed);
     }
   });
-  const int64_t n_ex = std::min<int64_t>(static_cast<int64_t>(*sl.ex.count), sl.ex.cap);
+  const Exceptions& ex = sl.out->ex;
+  const int64_t n_ex = std::min<int64_t>(static_cast<int64_t>(*ex.count), ex.cap);
   for (int64_t k = 0; k < n_ex; ++k) {
-    const int64_t at = sl.ex.index[k] - band_first - off;
-    if (at >= 0 && at < n) dst[at] = sl.ex.value[k];
+    const int64_t at = ex.index[k] - band_first - off;
+    if (at >= 0 && at < n) dst[at] = ex.value[k];
   }
   if (trace)
     fprintf(stderr, "[host] widened %lld pairs on %d threads in %.0f us\n", static_cast<long long>(n), T,
@@ -2036,7 +2034,7 @@ int next_chunk(frc_job* j, int mode, const void** data, int64_t* first_index, in
   if (sh.exact) {
     *data = sh.d2h ? sl->host64 : sl->dev64;
   } else if (mode == 2) {
-    *data = sh.d2h ? sl->host32 : sl->dev32;
+    *data = sh.d2h ? sl->host32 : sl->out->dev32 + sl->out_off;
   } else {
     deliver_n = std::min(kWidePiece, b.count);
     j->piece_first = b.first; j->piece_off = deliver_n; j->piece_end = b.count;
@@ -2077,15 +2075,15 @@ int frc_chunk_exceptions(frc_job_t* j, const int64_t** index, const double** val
   if (!j || !index || !value || !count) return FRC_ERR_ARG;
   *index = nullptr; *value = nullptr; *count = 0;
   if (j->held_part < 0 || j->sh.exact) return FRC_OK;
-  const Slot& sl = j->parts[j->held_part]->slots[j->held_slot];
-  const int64_t n = std::min<int64_t>(static_cast<int64_t>(*sl.ex.count), sl.ex.cap);
+  const Exceptions& ex = j->parts[j->held_part]->slots[j->held_slot].out->ex;
+  const int64_t n = std::min<int64_t>(static_cast<int64_t>(*ex.count), ex.cap);
   if (n == 0) return FRC_OK;
   // (a list may cover more than this run: the capacity mode keeps one per row shard)
   j->ex_index.clear(); j->ex_value.clear();
   for (int64_t k = 0; k < n; ++k)
-    if (sl.ex.index[k] >= j->held_first && sl.ex.index[k] < j->held_first + j->held_count) {
-      j->ex_index.push_back(sl.ex.index[k]);
-      j->ex_value.push_back(sl.ex.value[k]);
+    if (ex.index[k] >= j->held_first && ex.index[k] < j->held_first + j->held_count) {
+      j->ex_index.push_back(ex.index[k]);
+      j->ex_value.push_back(ex.value[k]);
     }
   *index = j->ex_index.data();
   *value = j->ex_value.data();

@@ -139,6 +139,78 @@ def test_weighted_capacity_mode_reads_panels_from_peers(built, monkeypatch):
         ctx.close()
 
 
+def test_weighted_capacity_mode_counts_each_group_once(built, monkeypatch):
+    """In capacity mode one fix-up output serves all the bands of a row-shard group: its flagged pairs and its
+    distances below fp32's range must reach frc_job_info once per pass, and frc_chunk_exceptions must hand each of
+    those distances out with the band it lies in -- exactly as the resident path does, and again after a restart."""
+    import numpy as np
+    import torch
+
+    from frackyfrac_b200 import engine, synth
+
+    n_gpu = torch.cuda.device_count()
+    if n_gpu < 2:
+        pytest.skip("needs at least 2 GPUs")
+    tree = synth.random_tree(900, 411)
+    tree.length = tree.length.copy()
+    # two sibling leaves a, b on branches of 1e-60: samples that differ only in which of them they hold lie ~1e-60
+    # apart, below fp32's range
+    kids = {}
+    for v in range(1, tree.n_nodes):
+        kids.setdefault(int(tree.parent[v]), []).append(v)
+    leaves = set(tree.leaf_ids.tolist())
+    a, b = next(c for c in kids.values() if len(c) == 2 and set(c) <= leaves)
+    tree.length[[a, b]] = 1e-60
+    n = 2100  # with band_rows = 128: at least two bands in every row-shard group on up to 8 devices
+    rp, col, val = synth.random_table(tree, n, 0.04, 412, integer_counts=False)
+    rows = []
+    for s in range(n):
+        c, v = col[rp[s]:rp[s + 1]], val[rp[s]:rp[s + 1]]
+        keep = (c != a) & (c != b)
+        rows.append((c[keep], v[keep]))
+    c0, v0 = rows[0]
+    rows[9] = (c0, v0 * (1 + 1e-4 * (np.arange(len(v0)) % 3 == 0)))  # a near duplicate of sample 0: fix-up territory
+    variants = list(range(40, n, 100))  # sample 0 plus leaf a or leaf b, spread over many bands
+    for k, s in enumerate(variants):
+        rows[s] = (np.append(c0, a if k % 2 else b), np.append(v0, 1.0))
+    rp = np.concatenate([[0], np.cumsum([len(c) for c, _ in rows])]).astype(np.int64)
+    col = np.concatenate([c for c, _ in rows]).astype(np.int32)
+    val = np.concatenate([v for _, v in rows])
+    n_ab = (len(variants) // 2) * ((len(variants) + 1) // 2)
+
+    def drain(job):
+        got, ex, expect = [], [], 0
+        for first, d in job.chunks_f32():
+            assert first == expect, (first, expect)
+            xi, xv = job.exceptions()
+            assert ((xi >= first) & (xi < first + len(d))).all(), (first, len(d), xi)
+            ex += zip(xi.tolist(), xv.tolist())
+            got.append(d)
+            expect += len(d)
+        i = job.info()
+        return np.concatenate(got), sorted(ex), (i.n_pairs_total, i.flagged_pairs, i.exceptions, i.d2h_bytes)
+
+    for nd in [k for k in (2, 4, 8) if k <= n_gpu]:
+        ctx = engine.Context(devices=list(range(nd)))
+        passes = {}
+        for cap in ("0", "1"):
+            monkeypatch.setenv("FRC_CAPACITY", cap)
+            with engine.Job(tree.parent, tree.length, rp, col, val, weighted=True, path=engine.PATH_FAST, ctx=ctx,
+                            band_rows=128) as job:
+                passes[cap] = [drain(job)]
+                job.restart()
+                passes[cap].append(drain(job))
+        got, ex, counts = passes["0"][0]
+        assert len(ex) == n_ab and all(0 < x < 1e-38 for _, x in ex)
+        assert counts == (n * (n - 1) // 2, counts[1], n_ab, 4 * n * (n - 1) // 2) and counts[1] > n_ab
+        for cap in ("0", "1"):
+            for k, (g, e, c) in enumerate(passes[cap]):
+                assert g.tobytes() == got.tobytes(), (nd, cap, k)
+                assert e == ex, (nd, cap, k)
+                assert c == counts, (nd, cap, k, c, counts)
+        ctx.close()
+
+
 def test_cli_on_all_gpus_reproduces_the_reference_fixtures(built, tmp_path):
     """The CLI stand-in with every visible GPU behind it: the six testdata/*.want files, byte for byte."""
     import torch
