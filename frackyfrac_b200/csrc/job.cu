@@ -233,6 +233,12 @@ struct Shared {
   char* stage_plan = nullptr;
   Seg pl_q0, pl_hi, pl_lo, pl_lenq, pl_order, pl_cexp, pl_lcol, pl_cend, pl_cscale, pl_cshift;
   size_t plan_bytes = 0;
+
+  int owners() const { return n_parts > 1 ? n_parts : world; }
+  // rows of the staged table whose CSR entries owner `owner` reads (set once `exchange` is)
+  std::pair<int64_t, int64_t> rows_read(int owner) const {
+    return frc::rows_read(N, owners(), owner, exchange != kNone && !exact && !weighted);
+  }
 };
 
 }  // namespace
@@ -1178,26 +1184,94 @@ void layout_inputs(Shared& sh) {
   sh.in_bytes = seg.total;
 }
 
+// FRC_FLAG_PRUNE: the subtree the staged table observes, from the leaves listed in ANY of its rows, so that every
+// rank of a sharded multi-process job derives the same tree.  Everything from the layout on runs on the pruned tree;
+// the entries are still checked against the caller's tree (same checks, same node ids in the messages) and staged
+// with their new ids.  A tree that fails the pre-order check is not pruned (false): the tree walks report it as they
+// do without the flag.
+bool prune_to_table(Shared& sh, Pool& pool, const frc_tree_t* tree, const StagedTable& table, PrunedTree* out) {
+  const int32_t B = tree->n_nodes;
+  std::vector<int32_t> depth(B);
+  int32_t bad_parent = 0, bad_order = 0;
+  if (!check_preorder(tree->parent, B, depth.data(), &bad_parent, &bad_order)) return false;
+  std::vector<uint8_t> marks(B, 0);
+  const int64_t nnz = sh.nnz;
+  const int T = nnz >= 65536 ? pool.size() : 1;
+  pool.run(T, [&](int t) { mark_table_leaves(table, nnz * t / T, nnz * (t + 1) / T, B, marks.data()); });
+  // merging reorders the fp64 sums of the exact path: it is only pruned
+  *out = prune_tree(tree->parent, tree->length, B, marks.data(), !sh.exact);
+  sh.B = out->n_nodes;
+  sh.node_mult = !sh.exact && sh.weighted && sh.opts.normalize == 1;
+  return true;
+}
+
+// The two tree tasks of the staging (pool workers, while the entries are staged), on the tree the kernels use.
+// Level order and level_ptr.
+TreeLevels stage_tree_levels(const Shared& sh, const frc_tree_t* tree) {
+  char* const st = sh.stage_in;
+  TreeLevels levels = tree_levels(tree->parent, sh.B, reinterpret_cast<int32_t*>(st + sh.in_lvl.off),
+                                  reinterpret_cast<int32_t*>(st + sh.in_lpar.off));
+  if (levels.height >= 0) memcpy(st + sh.in_lptr.off, levels.level_ptr.data(), sizeof(int32_t) * (levels.height + 2));
+  return levels;
+}
+// Children lists, parent / length, fp32 lengths, post-order (-l as coded), node multiplicities (mult: FRC_FLAG_PRUNE).
+// false when a parent id is out of range.
+bool stage_tree_children(const Shared& sh, const frc_tree_t* tree, const int32_t* mult) {
+  char* const st = sh.stage_in;
+  const int32_t B = sh.B;
+  if (!tree_children(tree->parent, B, reinterpret_cast<int32_t*>(st + sh.in_cptr.off),
+                     reinterpret_cast<int32_t*>(st + sh.in_cidx.off))) return false;
+  memcpy(st + sh.in_parent.off, tree->parent, sizeof(int32_t) * B);
+  memcpy(st + sh.in_len.off, tree->length, sizeof(double) * B);
+  float* lf = reinterpret_cast<float*>(st + sh.in_lenf.off);
+  const int32_t kp_pad = static_cast<int32_t>(round_up(B, kKBlock));
+  for (int32_t v = 0; v < kp_pad; ++v) lf[v] = v < B ? static_cast<float>(tree->length[v]) : 0.f;
+  if (sh.unsorted_l) tree_post_order(tree->parent, B, reinterpret_cast<int32_t*>(st + sh.in_post.off));
+  if (sh.node_mult) {
+    double* m = reinterpret_cast<double*>(st + sh.in_mult.off);
+    for (int32_t v = 0; v < B; ++v) m[v] = mult[v];
+  }
+  return true;
+}
+
+// Branch lengths: bad = a non-finite one in the caller's tree (only the exact path handles it), neg = a negative
+// finite one in the tree the kernels use.
+void scan_lengths(const frc_tree_t* caller, const frc_tree_t* tree, bool* bad, bool* neg) {
+  bool b = false, n = false;
+  for (int32_t v = 0; v < caller->n_nodes; ++v) {
+    const double l = caller->length[v];
+    if (!(l == l) || std::isinf(l)) b = true;
+  }
+  for (int32_t v = 0; v < tree->n_nodes; ++v) {
+    const double l = tree->length[v];
+    if (l < 0 && !std::isinf(l)) n = true;
+  }
+  *bad = b; *neg = n;
+}
+
+// How the sample shards of the embedding meet.  It depends on nothing the staging produces, so it is decided before
+// the staging starts, which then knows the rows a sharded rank reads (Shared::rows_read).
+void plan_exchange(Shared& sh, const frc_ctx* c) {
+  sh.fused_embed = !sh.knobs.embed_levels;
+  sh.exchange = Shared::kNone;
+  if (sh.exact) return;
+  if (sh.n_parts > 1 && c->peer_ok && sh.knobs.shard != 0 && (sh.weighted || sh.fused_embed)) sh.exchange = Shared::kInProcess;
+  if (sh.n_parts == 1 && sh.world > 1 && (sh.opts.flags & FRC_FLAG_SHARD_EMBED)) sh.exchange = Shared::kNccl;
+}
+
 // (3) the plan that does not depend on the table: operand columns; then bands + owners.
 int plan_job(frc_job* j, const frc_tree_t* tree, bool neg_len) {
   Shared& sh = j->sh;
   frc_ctx* c = j->ctx;
   const int n_parts = sh.n_parts;
   const bool fast_uw = !sh.exact && !sh.weighted;
-  sh.fused_embed = !sh.knobs.embed_levels;
-  // how the sample shards of the embedding meet
-  sh.exchange = Shared::kNone;
-  if (!sh.exact) {
-    if (n_parts > 1 && c->peer_ok && sh.knobs.shard != 0 && (sh.weighted || sh.fused_embed)) sh.exchange = Shared::kInProcess;
-    if (n_parts == 1 && sh.world > 1 && (sh.opts.flags & FRC_FLAG_SHARD_EMBED)) {
-      if (!c->comm || comm_world(c->comm) != sh.world || comm_rank(c->comm) != sh.rank0)
-        return fail(j, FRC_ERR_STATE, "FRC_FLAG_SHARD_EMBED needs a context whose communicator "
-                                      "(frc_ctx_comm_init) matches opts->rank / opts->world");
-      if (fast_uw && !sh.fused_embed) return fail(j, FRC_ERR_UNSUPPORTED, "FRC_EMBED_LEVELS=1 cannot build a sample shard");
-      sh.exchange = Shared::kNccl;
-    }
+  if (sh.exchange == Shared::kNccl) {
+    if (!c->comm || comm_world(c->comm) != sh.world || comm_rank(c->comm) != sh.rank0)
+      return fail(j, FRC_ERR_STATE, "FRC_FLAG_SHARD_EMBED needs a context whose communicator "
+                                    "(frc_ctx_comm_init) matches opts->rank / opts->world");
+    if (fast_uw && !sh.fused_embed) return fail(j, FRC_ERR_UNSUPPORTED, "FRC_EMBED_LEVELS=1 cannot build a sample shard");
   }
-  const int owners = sh.n_parts > 1 ? sh.n_parts : sh.world;
+  const int owners = sh.owners();
   ShardPlan::Mode mode = sh.exchange == Shared::kNone ? ShardPlan::kWhole : ShardPlan::kSharded;
   // Capacity mode of the fast weighted path: the fp32 panels of ALL samples (kp x np x 4 bytes: 320 GB at
   // BASELINE config 5) would not fit one device -> they stay sharded where they are built (two shards per
@@ -1332,13 +1406,11 @@ int prepare_part(Part* p) {
   const Range& own = sh.shards.ranges[p->owner][0];
   p->shard_w0 = static_cast<int32_t>(own.s0 / 32);
   p->shard_nw = static_cast<int32_t>((own.s1 - own.s0) / 32);
-  // CSR entries this part uploads: its own rows when only the embedding reads the table (the weighted
-  // fix-up walks the rows of any flagged pair, so weighted parts keep the whole table)
-  p->csr_k0 = 0; p->csr_k1 = sh.nnz;
-  if (sh.exchange != Shared::kNone && fast_uw && sh.N > 0) {
+  // CSR entries this part uploads (row_ptr is copied into the staging buffer before any task starts)
+  {
     const int64_t* rp = reinterpret_cast<const int64_t*>(sh.stage_in + sh.in_rowptr.off);
-    // (row_ptr is copied into the staging buffer before any task starts)
-    p->csr_k0 = rp[std::min(sh.N, own.s0)]; p->csr_k1 = rp[std::min(sh.N, own.s1)];
+    const std::pair<int64_t, int64_t> rows = sh.rows_read(p->owner);
+    p->csr_k0 = rp[rows.first]; p->csr_k1 = rp[rows.second];
   }
   // ---- per-part staging: tiles + need blocks
   SegAlloc seg;
@@ -1579,6 +1651,35 @@ void aggregate_info(frc_job* j) {
   }
 }
 
+// The job's context (the caller's, or one of its own from opts), one part per device, and how the parts' sample
+// shards meet.
+int attach_context(frc_job* j, frc_ctx_t* ctx, const frc_opts_t* opts) {
+  Shared& sh = j->sh;
+  if (ctx) {
+    if (ctx->in_use) return fail(j, FRC_ERR_STATE, "context already has a live job");
+    j->ctx = ctx;
+  } else {
+    const int rc = opts->n_devices > 1 || opts->n_devices < 0
+                       ? frc_ctx_create_multi(opts->n_devices, opts->devices, &j->ctx)
+                       : frc_ctx_create(opts->n_devices == 1 && opts->devices ? opts->devices[0] : opts->device, &j->ctx);
+    if (rc) { j->err = g_create_error; j->ctx = nullptr; return rc; }
+    j->own_ctx = true;
+  }
+  frc_ctx* c = j->ctx;
+  c->in_use = true;
+  sh.n_parts = static_cast<int>(c->devs.size());
+  if (sh.n_parts > 1 && sh.world > 1)
+    return fail(j, FRC_ERR_UNSUPPORTED, "a multi-device job cannot also be a rank of a multi-process run (world > 1)");
+  for (int k = 0; k < sh.n_parts; ++k) {
+    j->parts.emplace_back(new Part());
+    Part* p = j->parts.back().get();
+    p->job = j; p->sh = &sh; p->dc = c->devs[k]; p->index = k;
+    p->owner = sh.n_parts > 1 ? k : sh.rank0;
+  }
+  plan_exchange(sh, c);
+  return FRC_OK;
+}
+
 // frc_create (query == null) and frc_create_cross (abnd = the reference table).  A cross job stages ONE table of
 // q0 + n_q rows -- the reference rows, empty rows up to q0, the query rows (Shared::geo) -- and everything up to the
 // pair stage runs on it as on any table; only the bands, the tiles and the pair kernels' geometry differ.
@@ -1606,68 +1707,20 @@ int create_job(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
   // ------------------------------------------------------------ (1) options, table header
   int rc = validate_header(j, tree, abnd, query, opts);
   if (rc) return bail(rc);
-  const int32_t B0 = sh.B;  // the caller's tree (FRC_FLAG_PRUNE: B = the pruned one)
+  const frc_tree_t* const tree0 = tree;  // the caller's tree (FRC_FLAG_PRUNE: `tree` becomes the pruned one)
+  const StagedTable table{abnd, query, sh.geo.q0};
   const int64_t N = sh.N, nnz = sh.nnz;
 
   // ------------------------------------------------------------ context
-  if (ctx) {
-    if (ctx->in_use) return bail(fail(j, FRC_ERR_STATE, "context already has a live job"));
-    j->ctx = ctx;
-  } else {
-    if (opts->n_devices > 1 || opts->n_devices < 0) rc = frc_ctx_create_multi(opts->n_devices, opts->devices, &j->ctx);
-    else rc = frc_ctx_create(opts->n_devices == 1 && opts->devices ? opts->devices[0] : opts->device, &j->ctx);
-    if (rc) { j->err = g_create_error; j->ctx = nullptr; return bail(rc); }
-    j->own_ctx = true;
-  }
+  if ((rc = attach_context(j, ctx, opts)) != FRC_OK) return bail(rc);
   frc_ctx* c = j->ctx;
-  c->in_use = true;
-  sh.n_parts = static_cast<int>(c->devs.size());
-  if (sh.n_parts > 1 && sh.world > 1)
-    return bail(fail(j, FRC_ERR_UNSUPPORTED, "a multi-device job cannot also be a rank of a multi-process run (world > 1)"));
-  for (int k = 0; k < sh.n_parts; ++k) {
-    j->parts.emplace_back(new Part());
-    Part* p = j->parts.back().get();
-    p->job = j; p->sh = &sh; p->dc = c->devs[k]; p->index = k;
-    p->owner = sh.n_parts > 1 ? k : sh.rank0;
-  }
 
-  // ------------------------------------------------------------ FRC_FLAG_PRUNE: the subtree the table observes
-  // Everything from the layout on runs on the pruned tree; the entries are still checked against the caller's tree
-  // (same checks, same node ids in the messages) and staged with their new ids.
-  const frc_tree_t* const tree0 = tree;
   PrunedTree pruned;
   frc_tree_t ptree{};
-  if (opts->flags & FRC_FLAG_PRUNE) {
-    std::vector<int32_t> depth(B0);
-    int32_t bad_parent = 0, bad_order = 0;
-    // (a tree that fails the check is not pruned: the tree walks below report it as they do without the flag)
-    if (check_preorder(tree0->parent, B0, depth.data(), &bad_parent, &bad_order)) {
-      // the leaves listed in ANY row: every rank of a sharded multi-process job derives the same tree (out-of-range
-      // entries are left to the staging checks)
-      // (frc_create_cross: the leaves of both tables)
-      std::vector<uint8_t> marks(B0, 0);
-      const int T = nnz >= 65536 ? c->pool->size() : 1;
-      const int64_t nnz_a = abnd->n_samples > 0 ? abnd->row_ptr[abnd->n_samples] : 0;
-      const std::function<void(int)> mark_leaves = [&](int t) {
-        const int64_t k1 = nnz * (t + 1) / T;
-        for (int64_t k = nnz * t / T; k < k1; ++k) {
-          const int32_t cc = k < nnz_a ? abnd->col[k] : query->col[k - nnz_a];
-          // (read first: storing into lines that are already marked would bounce them between the cores)
-          if (cc >= 0 && cc < B0 && !__atomic_load_n(&marks[cc], __ATOMIC_RELAXED))
-            __atomic_store_n(&marks[cc], uint8_t{1}, __ATOMIC_RELAXED);
-        }
-      };
-      c->pool->run(T, mark_leaves);
-      // merging reorders the fp64 sums of the exact path: it is only pruned
-      pruned = prune_tree(tree0->parent, tree0->length, B0, marks.data(), !sh.exact);
-      ptree = frc_tree_t{pruned.n_nodes, pruned.parent.data(), pruned.length.data()};
-      tree = &ptree;
-      sh.B = pruned.n_nodes;
-      sh.node_mult = !sh.exact && sh.weighted && opts->normalize == 1;
-    }
+  if ((opts->flags & FRC_FLAG_PRUNE) && prune_to_table(sh, *c->pool, tree0, table, &pruned)) {
+    ptree = frc_tree_t{pruned.n_nodes, pruned.parent.data(), pruned.length.data()};
+    tree = &ptree;
   }
-  const int32_t B = sh.B;
-  const int32_t* const new_of_old = pruned.new_of_old.empty() ? nullptr : pruned.new_of_old.data();
 
   // ------------------------------------------------------------ (2) staging buffer; row_ptr right away
   layout_inputs(sh);
@@ -1675,28 +1728,9 @@ int create_job(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
     cudaError_t e = cudaSuccess;
     sh.stage_in = static_cast<char*>(c->pin.alloc(sh.in_bytes, &e));
     if (!sh.stage_in) return bail(fail(j, FRC_ERR_OOM, std::string("pinned staging of the inputs: ") + cudaGetErrorString(e)));
-    int64_t* rp = reinterpret_cast<int64_t*>(sh.stage_in + sh.in_rowptr.off);
-    const int64_t n_a = abnd->n_samples;
-    if (n_a > 0) memcpy(rp, abnd->row_ptr, sizeof(int64_t) * (n_a + 1)); else rp[0] = 0;
-    if (query) {  // empty rows up to q0, then the query rows after the reference entries
-      const int64_t q0 = sh.geo.q0, nnz_a = rp[n_a];
-      for (int64_t s = n_a + 1; s <= q0; ++s) rp[s] = nnz_a;
-      for (int64_t s = 1; s <= N - q0; ++s) rp[q0 + s] = nnz_a + query->row_ptr[s];
-    }
   }
-  char* const stage_in = sh.stage_in;
-  const int64_t* const staged_rp = reinterpret_cast<const int64_t*>(stage_in + sh.in_rowptr.off);
-  // the caller's entries of staged row s (not called for empty rows) and the row's name in messages
-  auto source_row = [&](int64_t s, const int32_t** cp, const double** vp) {
-    const frc_csr_t* t = query && s >= sh.geo.q0 ? query : abnd;
-    const int64_t r = t == query ? s - sh.geo.q0 : s;
-    *cp = t->col + t->row_ptr[r];
-    *vp = t->val + t->row_ptr[r];
-  };
-  auto row_name = [&](int64_t s) {
-    if (!query) return "sample #" + std::to_string(s + 1);
-    return s < sh.geo.q0 ? "reference sample #" + std::to_string(s + 1) : "query sample #" + std::to_string(s - sh.geo.q0 + 1);
-  };
+  int64_t* const staged_rp = reinterpret_cast<int64_t*>(sh.stage_in + sh.in_rowptr.off);
+  table.fill_row_ptr(staged_rp);
 
   // One task list for the pool: the tree walks, the preparation of devices 1.. (they wait for the plan),
   // then the CSR entries in chunks, all handed out through one counter; the calling thread plans, prepares
@@ -1704,31 +1738,11 @@ int create_job(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
   TreeLevels levels;
   bool children_ok = false;
   std::atomic<int> plan_ready{0};  // 1 = planned, -1 = planning failed
-  auto tree_children_share = [&]() {
-    if (!tree_children(tree->parent, B, reinterpret_cast<int32_t*>(stage_in + sh.in_cptr.off),
-                       reinterpret_cast<int32_t*>(stage_in + sh.in_cidx.off))) return;
-    memcpy(stage_in + sh.in_parent.off, tree->parent, sizeof(int32_t) * B);
-    memcpy(stage_in + sh.in_len.off, tree->length, sizeof(double) * B);
-    float* lf = reinterpret_cast<float*>(stage_in + sh.in_lenf.off);
-    const int32_t kp_pad = static_cast<int32_t>(round_up(B, kKBlock));
-    for (int32_t v = 0; v < kp_pad; ++v) lf[v] = v < B ? static_cast<float>(tree->length[v]) : 0.f;
-    if (sh.unsorted_l) tree_post_order(tree->parent, B, reinterpret_cast<int32_t*>(stage_in + sh.in_post.off));
-    if (sh.node_mult) {
-      double* m = reinterpret_cast<double*>(stage_in + sh.in_mult.off);
-      for (int32_t v = 0; v < B; ++v) m[v] = pruned.mult[v];
-    }
-    children_ok = true;
-  };
-  auto tree_levels_share = [&]() {
-    levels = tree_levels(tree->parent, B, reinterpret_cast<int32_t*>(stage_in + sh.in_lvl.off),
-                         reinterpret_cast<int32_t*>(stage_in + sh.in_lpar.off));
-    if (levels.height >= 0)
-      memcpy(stage_in + sh.in_lptr.off, levels.level_ptr.data(), sizeof(int32_t) * (levels.height + 2));
-  };
   // The entries are cut into many more chunks than workers and handed out through a counter: a worker
   // on a busy or slow core (the slowest static share took 1.5-2.4x the median) just takes fewer.
-  // A rank of a multi-process sharded unweighted job only reads its own rows: only those are checked and staged.
-  int64_t stage_k0 = 0, stage_k1 = nnz;
+  // The one part of a process stages the rows it reads; several parts of one process stage every row once.
+  const std::pair<int64_t, int64_t> rows = sh.n_parts == 1 ? sh.rows_read(sh.rank0) : std::pair<int64_t, int64_t>{0, N};
+  const int64_t stage_k0 = staged_rp[rows.first], stage_k1 = staged_rp[rows.second];
   const int csr_chunks = nnz >= 65536 ? static_cast<int>(std::max<int64_t>(1, std::min<int64_t>(c->pool->size() * 8LL, nnz / 8192))) : 1;
   const int n_prep = sh.n_parts - 1;
   const int n_tasks = 2 + n_prep + csr_chunks;
@@ -1739,23 +1753,17 @@ int create_job(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
   // context, so nothing is cleared between jobs
   const int64_t stamp_tag = c->stamp_epoch;
   c->stamp_epoch += N + 1;
+  int32_t* const dcol = reinterpret_cast<int32_t*>(sh.stage_in + sh.in_col.off);
+  double* const dval = sh.need_val ? reinterpret_cast<double*>(sh.stage_in + sh.in_val.off) : nullptr;
+  const int32_t* const new_of_old = pruned.new_of_old.empty() ? nullptr : pruned.new_of_old.data();
   const std::function<void(int)> work = [&](int t) {
     const auto w0 = std::chrono::steady_clock::now();
-    int32_t* dcol = reinterpret_cast<int32_t*>(stage_in + sh.in_col.off);
-    double* dval = sh.need_val ? reinterpret_cast<double*>(stage_in + sh.in_val.off) : nullptr;
-    const int TS = csr_chunks;
-    // a leaf listed twice in a row only matters when values are used (presence is an OR)
-    const bool check_dup = sh.need_val;
-    const int32_t* parent = tree0->parent;  // (checked against the caller's tree, staged with new_of_old ids)
-    auto row_at = [&](int64_t target) {
-      return static_cast<int64_t>(std::lower_bound(staged_rp, staged_rp + N, target) - staged_rp);
-    };
     std::vector<int64_t>& stamp = c->stamps[t];
-    if (check_dup && static_cast<int32_t>(stamp.size()) < B0) stamp.assign(B0, -1);
+    if (dval && static_cast<int32_t>(stamp.size()) < tree0->n_nodes) stamp.assign(tree0->n_nodes, -1);
     for (int task = task_next.fetch_add(1, std::memory_order_relaxed); task < n_tasks;
          task = task_next.fetch_add(1, std::memory_order_relaxed)) {
-      if (task == 0) { tree_levels_share(); continue; }
-      if (task == 1) { tree_children_share(); continue; }
+      if (task == 0) { levels = stage_tree_levels(sh, tree); continue; }
+      if (task == 1) { children_ok = stage_tree_children(sh, tree, pruned.mult.data()); continue; }
       if (task < 2 + n_prep) {
         int ready;
         while ((ready = plan_ready.load(std::memory_order_acquire)) == 0) std::this_thread::yield();
@@ -1763,56 +1771,13 @@ int create_job(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
         continue;
       }
       const int ch = task - 2 - n_prep;
-      const int64_t span = stage_k1 - stage_k0;
-      const int64_t s0 = row_at(stage_k0 + span * ch / TS), s1 = ch == TS - 1 ? row_at(stage_k1) : row_at(stage_k0 + span * (ch + 1) / TS);
-      bool failed = false;
-      for (int64_t s = s0; s < s1 && !failed; ++s) {
-        const int64_t b = staged_rp[s], e = staged_rp[s + 1];
-        if (b == e) continue;
-        const int64_t mark_s = stamp_tag + s;
-        const int32_t* scol;
-        const double* sval;
-        source_row(s, &scol, &sval);
-        for (int64_t k = b; k < e; ++k) {
-          const int32_t cc = scol[k - b];
-          const double v = sval[k - b];
-          const char* what = nullptr;
-          if (cc < 0 || cc >= B0) what = "node id out of range";
-          // pre-order ids: the first child of a node is the next id (the numbering itself is being
-          // checked by another task at this moment; a bad tree fails the call before this result counts)
-          else if (cc + 1 < B0 && parent[cc + 1] == cc) what = "node is not a leaf";
-          else if (!(v > 0) || std::isinf(v)) what = "bad value";
-          else if (check_dup && stamp[cc] == mark_s) what = "leaf listed twice";
-          if (what) {
-            csr_errs[ch] = row_name(s) + ": entry " + std::to_string(k - b + 1) + " (node " + std::to_string(cc) + "): " +
-                           what;
-            failed = true;
-            break;
-          }
-          if (check_dup) stamp[cc] = mark_s;
-          const int32_t id = new_of_old ? new_of_old[cc] : cc;
-#if defined(__x86_64__)
-          // streaming stores: the staging buffer is read next by the DMA engines, not by a core
-          _mm_stream_si32(dcol + k, id);
-          if (dval) _mm_stream_si64(reinterpret_cast<long long*>(dval + k), static_cast<long long>(__builtin_bit_cast(int64_t, v)));
-#else
-          dcol[k] = id;
-          if (dval) dval[k] = v;
-#endif
-        }
-      }
+      const std::pair<int64_t, int64_t> r = chunk_rows(staged_rp, N, stage_k0, stage_k1, ch, csr_chunks);
+      // (checked against the caller's tree, staged with the pruned tree's ids)
+      csr_errs[ch] = stage_entries(table, staged_rp, r.first, r.second, tree0->parent, tree0->n_nodes, new_of_old,
+                                   stamp.data(), stamp_tag, dcol, dval);
     }
-#if defined(__x86_64__)
-    _mm_sfence();
-#endif
     csr_us[t] += std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - w0).count();
   };
-  // multi-process sharded unweighted: the rows of this rank's shard only (decided before the tasks start, from the
-  // shard plan that plan_job will make)
-  if (!sh.exact && !sh.weighted && sh.n_parts == 1 && sh.world > 1 && (opts->flags & FRC_FLAG_SHARD_EMBED) && N > 0) {
-    const Range own = plan_shards(N, sh.world, ShardPlan::kSharded).ranges[sh.rank0][0];
-    stage_k0 = staged_rp[std::min(N, own.s0)]; stage_k1 = staged_rp[std::min(N, own.s1)];
-  }
   const int n_workers = c->pool->size() - 1;
   if (n_workers > 0) {
     workers_busy = true;
@@ -1822,15 +1787,8 @@ int create_job(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
 
   // ------------------------------------------------------------ (3) plan (the walks and the staging run in the pool)
   // (refused on the caller's lengths; the sign test is on the lengths the kernels use)
-  bool neg_len = false, bad_len = false;
-  for (int32_t v = 0; v < B0; ++v) {
-    const double l = tree0->length[v];
-    if (!(l == l) || std::isinf(l)) bad_len = true;
-  }
-  for (int32_t v = 0; v < B; ++v) {
-    const double l = tree->length[v];
-    if (l < 0 && !std::isinf(l)) neg_len = true;
-  }
+  bool bad_len = false, neg_len = false;
+  scan_lengths(tree0, tree, &bad_len, &neg_len);
   auto plan_failed = [&](int code) { plan_ready.store(-1, std::memory_order_release); return bail(code); };
   if (!sh.exact && bad_len)
     return plan_failed(fail(j, FRC_ERR_UNSUPPORTED, "non-finite branch length: only the exact path handles it"));
@@ -1846,8 +1804,8 @@ int create_job(frc_ctx_t* ctx, const frc_tree_t* tree, const frc_csr_t* abnd, co
   if (trace) { fprintf(stderr, "[frc_create] share times (us):"); for (double u : csr_us) fprintf(stderr, " %.0f", u); fprintf(stderr, "\n"); }
   if (levels.bad_parent) return bail(fail(j, FRC_ERR_ARG, "parent[" + std::to_string(levels.bad_parent) + "] is not a smaller node id"));
   if (levels.bad_order) return bail(fail(j, FRC_ERR_ARG, "node ids are not a pre-order numbering (node " + std::to_string(levels.bad_order) + ")"));
-  for (auto& e : csr_errs)
-    if (!e.empty()) return bail(fail(j, FRC_ERR_ARG, e));
+  const std::string& csr_err = first_error(csr_errs);
+  if (!csr_err.empty()) return bail(fail(j, FRC_ERR_ARG, csr_err));
   if (levels.height < 0 || !children_ok) return bail(fail(j, FRC_ERR_ARG, "tree topology could not be prepared"));  // (unreachable)
   for (auto& p : j->parts)
     if (p->rc) { j->err = p->err; return bail(p->rc); }

@@ -4,7 +4,12 @@
 #include <algorithm>
 #include <climits>
 #include <cmath>
+#include <cstdio>
 #include <cstring>
+
+#if defined(__x86_64__)
+#include <immintrin.h>
+#endif
 
 namespace frc {
 
@@ -178,6 +183,12 @@ ShardPlan plan_shards(int64_t N, int owners, ShardPlan::Mode mode) {
     else for (std::vector<Range>& r : sp.ranges) r.push_back(rg);
   }
   return sp;
+}
+
+std::pair<int64_t, int64_t> rows_read(int64_t N, int owners, int owner, bool sharded_fast_uw) {
+  if (!sharded_fast_uw || N <= 0) return {0, N};
+  const Range own = plan_shards(N, owners, ShardPlan::kSharded).ranges[owner][0];
+  return {std::min(N, own.s0), std::min(N, own.s1)};
 }
 
 std::vector<Band> make_bands_capacity(int64_t N, const ShardPlan& sp, int64_t requested, bool d2h) {
@@ -484,11 +495,96 @@ PrunedTree prune_tree(const int32_t* parent, const double* length, int32_t B, co
   return t;
 }
 
+std::string StagedTable::row_name(int64_t s) const {
+  if (!query) return "sample #" + std::to_string(s + 1);
+  return s < q0 ? "reference sample #" + std::to_string(s + 1) : "query sample #" + std::to_string(s - q0 + 1);
+}
+
+void StagedTable::fill_row_ptr(int64_t* rp) const {
+  const int64_t n_a = ref->n_samples;
+  if (n_a > 0) memcpy(rp, ref->row_ptr, sizeof(int64_t) * (n_a + 1)); else rp[0] = 0;
+  if (!query) return;
+  const int64_t nnz_a = rp[n_a];
+  for (int64_t s = n_a + 1; s <= q0; ++s) rp[s] = nnz_a;
+  for (int64_t s = 1; s <= query->n_samples; ++s) rp[q0 + s] = nnz_a + query->row_ptr[s];
+}
+
+std::string stage_entries(const StagedTable& t, const int64_t* rp, int64_t s0, int64_t s1, const int32_t* parent,
+                          int32_t B, const int32_t* new_of_old, int64_t* stamp, int64_t stamp_tag, int32_t* dcol,
+                          double* dval) {
+  // a leaf listed twice in a row only matters when values are used (presence is an OR)
+  const bool check_dup = dval != nullptr;
+  std::string err;
+  for (int64_t s = s0; s < s1 && err.empty(); ++s) {
+    const int64_t b = rp[s], e = rp[s + 1];
+    if (b == e) continue;
+    const int64_t mark_s = stamp_tag + s;
+    const int32_t* scol = t.col(s);
+    const double* sval = t.val(s);
+    for (int64_t k = b; k < e; ++k) {
+      const int32_t cc = scol[k - b];
+      const double v = sval[k - b];
+      const char* what = nullptr;
+      if (cc < 0 || cc >= B) what = "node id out of range";
+      // pre-order ids: the first child of a node is the next id (in frc_create the numbering itself is being
+      // checked by another task at this moment; a bad tree fails the call before this result counts)
+      else if (cc + 1 < B && parent[cc + 1] == cc) what = "node is not a leaf";
+      else if (!(v > 0) || std::isinf(v)) what = "bad value";
+      else if (check_dup && stamp[cc] == mark_s) what = "leaf listed twice";
+      if (what) {
+        err = t.row_name(s) + ": entry " + std::to_string(k - b + 1) + " (node " + std::to_string(cc) + "): " + what;
+        break;
+      }
+      if (check_dup) stamp[cc] = mark_s;
+      const int32_t id = new_of_old ? new_of_old[cc] : cc;
+#if defined(__x86_64__)
+      // streaming stores: the staging buffer is read next by the DMA engines, not by a core
+      _mm_stream_si32(dcol + k, id);
+      if (dval) _mm_stream_si64(reinterpret_cast<long long*>(dval + k), static_cast<long long>(__builtin_bit_cast(int64_t, v)));
+#else
+      dcol[k] = id;
+      if (dval) dval[k] = v;
+#endif
+    }
+  }
+#if defined(__x86_64__)
+  _mm_sfence();
+#endif
+  return err;
+}
+
+std::pair<int64_t, int64_t> chunk_rows(const int64_t* rp, int64_t N, int64_t k0, int64_t k1, int ch, int n_chunks) {
+  auto row_at = [&](int64_t target) { return static_cast<int64_t>(std::lower_bound(rp, rp + N, target) - rp); };
+  const int64_t span = k1 - k0;
+  return {row_at(k0 + span * ch / n_chunks), row_at(k0 + span * (ch + 1) / n_chunks)};
+}
+
+const std::string& first_error(const std::vector<std::string>& chunk_errors) {
+  static const std::string none;
+  for (const std::string& e : chunk_errors)
+    if (!e.empty()) return e;
+  return none;
+}
+
+void mark_table_leaves(const StagedTable& t, int64_t k0, int64_t k1, int32_t B, uint8_t* marks) {
+  auto mark = [&](const int32_t* col, int64_t a, int64_t b) {
+    for (int64_t k = a; k < b; ++k) {
+      const int32_t cc = col[k];
+      // (read first: storing into lines that are already marked would bounce them between the cores)
+      if (cc >= 0 && cc < B && !__atomic_load_n(&marks[cc], __ATOMIC_RELAXED))
+        __atomic_store_n(&marks[cc], uint8_t{1}, __ATOMIC_RELAXED);
+    }
+  };
+  const int64_t nnz_a = t.ref_nnz();
+  if (k0 < nnz_a) mark(t.ref->col, k0, std::min(k1, nnz_a));
+  if (t.query && k1 > nnz_a) mark(t.query->col, std::max(k0, nnz_a) - nnz_a, k1 - nnz_a);
+}
+
 }  // namespace frc
 
 // ---------------------------------------------------------------- CPU test entry points
-// Not part of the C ABI (include/frcfrc_cuda.h): they let tests/test_plan.py exercise the planning
-// units on the CPU-only box.
+// Not part of the C ABI (include/frcfrc_cuda.h): they let tests/test_plan.py, test_prune.py and test_stage.py
+// exercise the planning and staging units on the CPU-only box.
 static int64_t write_bands(const std::vector<frc::Band>& bands, int64_t* out5, int64_t cap) {
   for (size_t k = 0; k < bands.size() && static_cast<int64_t>(k) < cap; ++k) {
     out5[5 * k] = bands[k].row0; out5[5 * k + 1] = bands[k].row1; out5[5 * k + 2] = bands[k].first;
@@ -631,6 +727,43 @@ int32_t frc_debug_prune(const int32_t* parent, const double* length, int32_t n_n
   for (int32_t v = 0; v < t.n_nodes; ++v) { out_parent[v] = t.parent[v]; out_length[v] = t.length[v]; out_mult[v] = t.mult[v]; }
   for (int32_t v = 0; v < n_nodes; ++v) new_of_old[v] = t.new_of_old[v];
   return t.n_nodes;
+}
+
+// Table staging as frc_create does it: the table (n_q < 0) or the reference + query pair of frc_create_cross
+// (q0 = n_ref rounded up to 256), checked against parent[n_nodes], its entries cut into n_chunks chunks.  out_rp holds
+// the staged rows + 1 entries, out_col / out_val (null: presence only) the entries; new_of_old may be null, stamp
+// [n_nodes] is needed with out_val.  Writes the reported message (NUL-terminated, cut to msg_cap) into msg; returns the
+// staged row count.  PRUNE marks of the same entries go to marks[n_nodes] unless it is null.
+int64_t frc_debug_stage(const int32_t* parent, int32_t n_nodes, int64_t n_ref, const int64_t* ref_rp,
+                        const int32_t* ref_col, const double* ref_val, int64_t n_q, const int64_t* q_rp,
+                        const int32_t* q_col, const double* q_val, const int32_t* new_of_old, int32_t n_chunks,
+                        int64_t* stamp, int64_t stamp_tag, int64_t* out_rp, int32_t* out_col, double* out_val,
+                        uint8_t* marks, char* msg, int64_t msg_cap) {
+  const frc_csr_t ref{n_ref, ref_rp, ref_col, ref_val}, query{n_q, q_rp, q_col, q_val};
+  frc::StagedTable t{&ref, n_q >= 0 ? &query : nullptr, 0};
+  int64_t N = n_ref;
+  if (t.query) {
+    t.q0 = frc::round_up(n_ref, 2 * frc::kTile);
+    N = t.q0 + n_q;
+  }
+  t.fill_row_ptr(out_rp);
+  const int64_t nnz = out_rp[N];
+  if (marks) frc::mark_table_leaves(t, 0, nnz, n_nodes, marks);
+  std::vector<std::string> errs(n_chunks);
+  for (int ch = n_chunks - 1; ch >= 0; --ch) {  // (backwards: the report must not depend on which chunk ends first)
+    const std::pair<int64_t, int64_t> rows = frc::chunk_rows(out_rp, N, 0, nnz, ch, n_chunks);
+    errs[ch] = frc::stage_entries(t, out_rp, rows.first, rows.second, parent, n_nodes, new_of_old, stamp, stamp_tag,
+                                  out_col, out_val);
+  }
+  const std::string& e = frc::first_error(errs);
+  snprintf(msg, static_cast<size_t>(msg_cap), "%s", e.c_str());
+  return N;
+}
+
+// Rows [out2[0], out2[1]) of the staged table whose entries `owner` reads (rows_read).
+void frc_debug_rows_read(int64_t n_samples, int32_t owners, int32_t owner, int32_t sharded_fast_uw, int64_t* out2) {
+  const std::pair<int64_t, int64_t> r = frc::rows_read(n_samples, owners, owner, sharded_fast_uw != 0);
+  out2[0] = r.first; out2[1] = r.second;
 }
 
 }  // extern "C"

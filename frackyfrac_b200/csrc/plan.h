@@ -7,11 +7,14 @@
 //   tile lists     per band: the 128 x 128 sample tiles (CTA-pair tiles for the tensor-core kernel)
 //   tree walk      pre-order check, children lists, level order (what enumerateNodes' numbering implies,
 //                  frcfrc/unifrac.go:127-133)
+//   table staging  the caller's CSR entries checked and copied into the staged table (tests/test_stage.py)
 #pragma once
 #include <cstdint>
 #include <string>
+#include <utility>
 #include <vector>
 
+#include "../../include/frcfrc_cuda.h"
 #include "frc_internal.h"
 
 namespace frc {
@@ -57,6 +60,10 @@ struct ShardPlan {
   std::vector<std::vector<Range>> ranges;  // per owner, in slot order
 };
 ShardPlan plan_shards(int64_t N, int owners, ShardPlan::Mode mode);
+// Rows [first, second) of the staged table whose CSR entries `owner` reads.  With a sharded embedding on the fast
+// unweighted path only the embedding reads the table, and an owner builds its own kSharded shard; otherwise every row
+// (the weighted fix-up walks the rows of any flagged pair, and the capacity mode is weighted only).
+std::pair<int64_t, int64_t> rows_read(int64_t N, int owners, int owner, bool sharded_fast_uw);
 
 // Capacity mode of the fast weighted path (PanelMap in frc_internal.h): the bands of every shard of `sp`, owned by
 // the shard's device.  Bands never straddle a shard.
@@ -130,5 +137,46 @@ struct PrunedTree {
   std::vector<int32_t> mult;
 };
 PrunedTree prune_tree(const int32_t* parent, const double* length, int32_t n_nodes, const uint8_t* marks, bool merge);
+
+// The table frc_create stages: the caller's table, or for frc_create_cross the reference rows, empty rows up to q0
+// (Geometry), then the query rows, whose entries follow the reference entries.  The one place that maps staged rows
+// and entries back to the caller's tables.  The tables' headers have been checked (validate_header).
+struct StagedTable {
+  const frc_csr_t* ref = nullptr;    // frc_create: the table; frc_create_cross: the reference table
+  const frc_csr_t* query = nullptr;  // frc_create_cross: the query table
+  int64_t q0 = 0;                    // staged row of query row 0
+
+  int64_t ref_nnz() const { return ref->n_samples > 0 ? ref->row_ptr[ref->n_samples] : 0; }
+  bool in_query(int64_t s) const { return query && s >= q0; }
+  // the caller's entries of staged row s (not for the empty rows below q0)
+  const int32_t* col(int64_t s) const {
+    return in_query(s) ? query->col + query->row_ptr[s - q0] : ref->col + ref->row_ptr[s];
+  }
+  const double* val(int64_t s) const {
+    return in_query(s) ? query->val + query->row_ptr[s - q0] : ref->val + ref->row_ptr[s];
+  }
+  // "sample #k", "reference sample #k" or "query sample #k" (k from 1, within the caller's table)
+  std::string row_name(int64_t s) const;
+  // the staged row_ptr: q0 + n_q + 1 entries (frc_create: n_samples + 1)
+  void fill_row_ptr(int64_t* rp) const;
+};
+
+// Checks the entries of staged rows [s0, s1) against the caller's tree parent[n_nodes] and copies them into the
+// staged col / val (rp: the staged row_ptr) with streaming stores, node ids mapped through new_of_old (null: kept).
+// The checks, in this order, on every entry: node id in range, a leaf (pre-order ids: a node's first child is the next
+// id), value positive and finite, and -- only when values are used (val != null) -- not listed twice in its row.  The
+// duplicate test marks stamp[node] = stamp_tag + row: stamp[n_nodes] persists across jobs, and each job's tag lies
+// past every mark of the previous ones.  Stops at the first bad entry and returns its message (empty: none).
+std::string stage_entries(const StagedTable& t, const int64_t* rp, int64_t s0, int64_t s1, const int32_t* parent,
+                          int32_t n_nodes, const int32_t* new_of_old, int64_t* stamp, int64_t stamp_tag, int32_t* col,
+                          double* val);
+// The staged entries [k0, k1) are checked and copied in n_chunks chunks of whole rows and about equal entry counts:
+// rows [first, second) of chunk ch (rp: the staged row_ptr of N rows).
+std::pair<int64_t, int64_t> chunk_rows(const int64_t* rp, int64_t N, int64_t k0, int64_t k1, int ch, int n_chunks);
+// The error frc_create reports from its chunks' messages: the first bad entry in row order (empty: none).
+const std::string& first_error(const std::vector<std::string>& chunk_errors);
+// FRC_FLAG_PRUNE: marks[node] = 1 for every node listed in the staged entries [k0, k1) of either table (ids outside
+// [0, n_nodes) are left to stage_entries).  Relaxed atomic stores: several threads mark disjoint entry ranges.
+void mark_table_leaves(const StagedTable& t, int64_t k0, int64_t k1, int32_t n_nodes, uint8_t* marks);
 
 }  // namespace frc
