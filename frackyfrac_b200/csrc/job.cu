@@ -107,41 +107,6 @@ constexpr int kMaxExceptions = 4096;            // per band: distances fp32 cann
 constexpr int kFixupCtas = 32;                  // weighted fix-up: CTAs (one int64[B] workspace each, per stream)
 constexpr int kMaxParts = 8;                    // devices per job (PeerPtrs holds 8)
 
-// Environment knobs (tests and experiments; DESIGN.md has the table).  Read ONCE per frc_create: nothing
-// on the per-band path calls getenv.
-struct Knobs {
-  bool trace = false;
-  int bands_per_rank = 0;     // FRC_BANDS
-  int widen_threads = 0;      // FRC_WIDEN_THREADS
-  int ws_slab = 0;            // FRC_WS_SLAB
-  bool uw_bf16 = false;       // FRC_UW_KERNEL=bf16
-  bool u8_acc_f64 = false;    // FRC_U8_ACC=f64
-  bool feed_bits = false;     // FRC_UW_FEED=bits
-  bool embed_levels = false;  // FRC_EMBED_LEVELS=1
-  int peer_push = -1;         // FRC_PEER_PUSH (multi-process sharding: 0 = NCCL all-gather of the bits)
-  int group_binades = 3;      // FRC_U8_GROUP_BINADES
-  int shard = -1;             // FRC_SHARD (in-process multi-GPU: 0 = every device rebuilds the embedding)
-  int capacity = -1;          // FRC_CAPACITY (in-process multi-GPU, fast weighted: 1 / 0 = force / forbid the sharded-panel mode)
-  static Knobs read() {
-    Knobs k;
-    auto num = [](const char* name, int dflt) { const char* e = getenv(name); return e && *e ? atoi(e) : dflt; };
-    auto is = [](const char* name, const char* v) { const char* e = getenv(name); return e && !strcmp(e, v); };
-    k.trace = getenv("FRC_TRACE") != nullptr;
-    k.bands_per_rank = std::max(0, num("FRC_BANDS", 0));
-    k.widen_threads = std::max(0, num("FRC_WIDEN_THREADS", 0));
-    k.ws_slab = std::max(0, num("FRC_WS_SLAB", 0));
-    k.uw_bf16 = is("FRC_UW_KERNEL", "bf16");
-    k.u8_acc_f64 = is("FRC_U8_ACC", "f64");
-    k.feed_bits = is("FRC_UW_FEED", "bits");
-    k.embed_levels = num("FRC_EMBED_LEVELS", 0) == 1;
-    k.peer_push = num("FRC_PEER_PUSH", -1);
-    k.group_binades = num("FRC_U8_GROUP_BINADES", 3);
-    k.shard = num("FRC_SHARD", -1);
-    k.capacity = num("FRC_CAPACITY", -1);
-    return k;
-  }
-};
-
 // The calling thread's current device is restored when an entry point returns (a job may drive several).
 struct DeviceGuard {
   int prev = -1;
@@ -217,9 +182,7 @@ struct Shared {
   Geometry geo;               // frc_create_cross: the query x reference block of the staged table (n_q = N - geo.q0)
   int n_parts = 1;
   int world = 1, rank0 = 0;   // band ownership: `world` owners; part p owns owner id rank0 + p
-  enum Exchange { kNone, kInProcess, kNccl } exchange = kNone;  // how the sample shards of the embedding meet
-  bool fused_embed = true, bits_feed = false;
-  bool capacity = false;      // fast weighted over several devices: panels stay sharded (PanelMap), tiles read peers' HBM
+  Variant variant;            // which variant of the fast path runs (csrc/plan.cpp)
   ShardPlan shards;           // which samples each owner builds (np = shards.np)
   ColumnPlan cols;
   std::vector<Band> bands;   // every band of the job (owners filled in)
@@ -235,9 +198,9 @@ struct Shared {
   size_t plan_bytes = 0;
 
   int owners() const { return n_parts > 1 ? n_parts : world; }
-  // rows of the staged table whose CSR entries owner `owner` reads (set once `exchange` is)
+  // rows of the staged table whose CSR entries owner `owner` reads (set once plan_exchange has run)
   std::pair<int64_t, int64_t> rows_read(int owner) const {
-    return frc::rows_read(N, owners(), owner, exchange != kNone && !exact && !weighted);
+    return frc::rows_read(N, owners(), owner, variant.sharded_fast_uw);
   }
 };
 
@@ -485,16 +448,16 @@ template <auto M> void* part_array(const Part* q) { return q->*M; }
 // r-th: the sharded plan puts shard r there), a barrier when nothing is copied; kInProcess: copies over NVLink.
 int exchange_shard(Part* p, const std::vector<ShardArray>& arrs, const Range& rg, cudaStream_t s) {
   const Shared& sh = *p->sh;
-  if (sh.exchange == Shared::kNone) return FRC_OK;
+  if (sh.variant.exchange == Variant::kNone) return FRC_OK;
   const size_t n = static_cast<size_t>(rg.s1 - rg.s0);
-  const int others = (sh.exchange == Shared::kNccl ? sh.world : sh.n_parts) - 1;
+  const int others = (sh.variant.exchange == Variant::kNccl ? sh.world : sh.n_parts) - 1;
   std::vector<void*> bufs;
   std::vector<size_t> bytes;
   for (const ShardArray& a : arrs) {
     p->info.gather_bytes += static_cast<int64_t>(n * a.sample_bytes) * others;
     if (a.copy) { bufs.push_back(a.on(p)); bytes.push_back(n * a.sample_bytes); }
   }
-  if (sh.exchange == Shared::kNccl) {
+  if (sh.variant.exchange == Variant::kNccl) {
     Comm* comm = p->job->ctx->comm;
     std::string cerr;
     const bool ok = bufs.empty() ? comm_barrier(comm, s, &cerr)
@@ -518,6 +481,7 @@ int exchange_shard(Part* p, const std::vector<ShardArray>& arrs, const Range& rg
 // part's sample shard has been made visible to the other devices.  Unsharded jobs run the whole embedding here.
 int embed_stage1(Part* p) {
   const Shared& sh = *p->sh;
+  const Variant& v = sh.variant;
   DevCtx* dc = p->dc;
   frc_ctx* c = p->job->ctx;
   cudaStream_t s = dc->stream[0];
@@ -527,7 +491,6 @@ int embed_stage1(Part* p) {
     PART_CUDA(p, cudaMemsetAsync(p->d_flag_counts, 0, sizeof(unsigned long long) * (p->mine.size() + 1), s));
   PART_CUDA(p, cudaEventRecord(p->ev_embed0, s));
   p->info.gather_bytes = 0;
-  const bool inproc = sh.exchange == Shared::kInProcess;
   if (sh.exact) {
     launches += launch_embed_f64(p->dtree, sh.level_ptr.data(), p->dcsr, p->d_E, sh.np, 0, s);
     // (normalisation cannot change membership, which is all the unweighted kernel reads -- and a
@@ -559,7 +522,7 @@ int embed_stage1(Part* p) {
     // what the other devices read of a shard, in the order of the NCCL group: panels (unless they stay sharded:
     // capacity mode), denominators, normalisers, key panels
     std::vector<ShardArray> arrs;
-    if (!sh.capacity) arrs.push_back({part_array<&Part::d_A>, sizeof(float) * sh.kp});
+    if (!v.capacity) arrs.push_back({part_array<&Part::d_A>, sizeof(float) * sh.kp});
     arrs.push_back({part_array<&Part::d_W>, sizeof(double)});
     if (norm) arrs.push_back({part_array<&Part::d_total>, sizeof(double)});
     if (sh.keyed) arrs.push_back({part_array<&Part::d_K>, sizeof(int32_t) * sh.kp});
@@ -583,7 +546,7 @@ int embed_stage1(Part* p) {
       if (exchange_shard(p, arrs, rg, s)) return p->rc;
     }
     p->pm = PanelMap{};
-    if (sh.capacity) {
+    if (v.capacity) {
       // own shards in their slots; the visiting shards are filled in by the rotation (start_pairs_capacity)
       p->pm.n_shards = sh.shards.n_shards;
       p->pm.tiles_per_shard = static_cast<int32_t>(sh.shards.shard_rows / kTile);
@@ -594,7 +557,7 @@ int embed_stage1(Part* p) {
     }
     // write each element once, read it once when folded into its parent (+ CSR; keyed: + the int32 keys)
     p->info.embed_bytes = 2LL * sh.B * built * (sh.keyed ? 12 : 8) + 12LL * (p->csr_k1 - p->csr_k0);
-  } else if (sh.fused_embed) {
+  } else if (v.fused_embed) {
     const int cur = static_cast<int>(p->run_count & 1);
     if (p->peer_push) {
       p->d_bits = p->d_bits2[cur];
@@ -606,7 +569,7 @@ int embed_stage1(Part* p) {
     ++p->run_count;
     PeerPtrs peers;  // n = 0: local stores only
     if (p->peer_push) peers = p->peers[cur];
-    else if (inproc && !sh.bits_feed) {
+    else if (v.peer_store) {
       // in-process sharding: the kernel stores its finished bit columns straight into every device's
       // bitsT (peer access over NVLink): the all-gather is fused into the producing kernel
       peers.n = sh.n_parts; peers.self = p->index;
@@ -614,37 +577,33 @@ int embed_stage1(Part* p) {
     }
     launches += launch_embed_presence_fused(p->dtree, p->d_level_ptr, p->dcsr, sh.nw, p->shard_w0, p->shard_nw,
                                             sh.kp, p->d_order, p->d_node_scratch, p->d_bits, p->d_bitsS, peers, s);
-    // Row sums.  Integer mode with materialised operands (the default): the operand expansion of stage 2
-    // produces them for every sample from the words it holds anyway -- nothing to do here, nothing to
-    // exchange but the bit columns.  Otherwise (fp64 row sums of the bf16 / wide-scale modes, bits-fed kernel)
-    // a separate pass over this part's shard: it runs beside the expansion on the second compute stream
-    // unless an exchange sits between.
-    const bool rowsum_in_expand = sh.cols.intacc && !sh.bits_feed;
-    const bool split = sh.exchange == Shared::kNone && !rowsum_in_expand;
-    cudaStream_t rs = split ? dc->stream[1] : s;
-    if (split) {
+    // Row sums: made by the operand expansion of stage 2 (integer mode with materialised operands: nothing to
+    // exchange but the bit columns), or by a pass over this part's shard here (Variant::rowsum_split: beside the
+    // expansion on the second compute stream).
+    cudaStream_t rs = v.rowsum_split ? dc->stream[1] : s;
+    if (v.rowsum_split) {
       PART_CUDA(p, cudaEventRecord(p->ev_bits, s));
       PART_CUDA(p, cudaStreamWaitEvent(rs, p->ev_bits, 0));
     }
-    if (!rowsum_in_expand)
+    if (!v.rowsum_in_expand)
       launches += launch_presence_rowsum_t(p->d_bits, sh.B, sh.nw, p->shard_w0, p->shard_nw, sh.kp, p->d_lenq,
                                            sh.cols.i8 ? p->d_qam : nullptr, p->d_col_exp, p->d_scratch, p->d_r,
                                            sh.cols.e_min, sh.cols.intacc ? p->d_r_int : nullptr, rs);
     // what the other parts read of the shard: row sums (unless the expansion makes them) and bit columns (2.5 GB at
     // cfg4 instead of 120 GB of operands; bits-fed: the bit rows, same size), unless the kernel above stored them.
     std::vector<ShardArray> arrs;
-    if (!rowsum_in_expand)
+    if (!v.rowsum_in_expand)
       arrs.push_back({sh.cols.intacc ? part_array<&Part::d_r_int> : part_array<&Part::d_r>, sizeof(double)});
-    arrs.push_back({sh.bits_feed ? part_array<&Part::d_bitsS> : part_array<&Part::d_bits>, sizeof(uint32_t) * sh.kp / 32,
+    arrs.push_back({v.bits_feed ? part_array<&Part::d_bitsS> : part_array<&Part::d_bits>, sizeof(uint32_t) * sh.kp / 32,
                     peers.n == 0});
     if (exchange_shard(p, arrs, sh.shards.ranges[p->owner][0], s)) return p->rc;
-    if (sh.exchange != Shared::kNone) {
+    if (v.exchange != Variant::kNone) {
       // bits written + read once per level pass (+ CSR cols): this part's shard
       p->info.embed_bytes = 2LL * sh.B * p->shard_nw * 4 + 4LL * (p->csr_k1 - p->csr_k0);
     }
   }
   PART_CUDA(p, cudaGetLastError());
-  if (inproc) PART_CUDA(p, cudaEventRecord(p->ev_shard, s));
+  if (v.exchange == Variant::kInProcess) PART_CUDA(p, cudaEventRecord(p->ev_shard, s));
   p->info.kernel_launches += launches;
   return FRC_OK;
 }
@@ -655,25 +614,23 @@ int embed_stage2(Part* p) {
   DevCtx* dc = p->dc;
   cudaStream_t s = dc->stream[0];
   int launches = 0;
-  if (sh.exchange == Shared::kInProcess)
+  const Variant& v = sh.variant;
+  if (v.exchange == Variant::kInProcess)
     for (auto& o : p->job->parts)
       if (o.get() != p) PART_CUDA(p, cudaStreamWaitEvent(s, o->ev_shard, 0));
   if (!sh.exact && !sh.weighted) {
-    if (sh.fused_embed) {
-      const bool rowsum_in_expand = sh.cols.intacc && !sh.bits_feed;
-      if (!sh.bits_feed)
+    if (v.fused_embed) {
+      if (!v.bits_feed)
         launches += launch_expand_operands_t(p->d_bits, sh.nw, sh.kp, sh.np, sh.cols.i8, p->d_q0, p->d_q1, p->d_q2,
                                              p->d_P, p->d_Bh, p->d_Bl, p->d_need, p->d_qam, p->d_col_exp, sh.cols.e_min,
-                                             rowsum_in_expand ? p->d_r_int : nullptr, s);
-      if (sh.exchange == Shared::kNone) {
-        if (!rowsum_in_expand) {
-          PART_CUDA(p, cudaEventRecord(p->ev_rsum, dc->stream[1]));
-          PART_CUDA(p, cudaStreamWaitEvent(s, p->ev_rsum, 0));
-        }
-        p->info.embed_bytes = 2LL * sh.B * sh.nw * 4 + 4LL * sh.nnz;
+                                             v.rowsum_in_expand ? p->d_r_int : nullptr, s);
+      if (v.rowsum_split) {
+        PART_CUDA(p, cudaEventRecord(p->ev_rsum, dc->stream[1]));
+        PART_CUDA(p, cudaStreamWaitEvent(s, p->ev_rsum, 0));
       }
+      if (v.exchange == Variant::kNone) p->info.embed_bytes = 2LL * sh.B * sh.nw * 4 + 4LL * sh.nnz;
       // + three operands written once, the bit columns read once more
-      if (!sh.bits_feed) p->info.embed_bytes += 3LL * sh.np * sh.kp * (sh.cols.i8 ? 1 : 2) + 4LL * sh.nw * sh.kp;
+      if (!v.bits_feed) p->info.embed_bytes += 3LL * sh.np * sh.kp * (sh.cols.i8 ? 1 : 2) + 4LL * sh.nw * sh.kp;
     } else {
       launches += launch_embed_bits(p->dtree, sh.level_ptr.data(), p->dcsr, p->d_bits, sh.nw, s);
       launches += launch_presence_rowsum(p->d_bits, sh.B, sh.nw, p->d_lenq, p->d_r, p->d_scratch, s);
@@ -749,7 +706,7 @@ int enqueue_band(Part* p, size_t idx) {
   const int si = static_cast<int>(idx % 2);
   cudaStream_t s = dc->stream[si];
   int launches = 0;
-  if (sh.capacity) {
+  if (sh.variant.capacity) {
     // the band was (or is being) computed by the rotation into its group's record
     Part::CapGroup& cb = p->cap[p->band_group[idx]];
     sl.out = &cb.out;
@@ -851,7 +808,7 @@ int start_pairs(Part* p) {
     PART_CUDA(p, cudaEventRecord(p->ev_run1, p->dc->stream[0]));
     return FRC_OK;
   }
-  if (p->sh->capacity && start_pairs_capacity(p)) return p->rc;
+  if (p->sh->variant.capacity && start_pairs_capacity(p)) return p->rc;
   // keep one slot free for the band the caller is still reading
   while (p->next_enqueue < p->mine.size() && p->next_enqueue < static_cast<size_t>(p->n_slots - 1)) {
     if (enqueue_band(p, p->next_enqueue)) return p->rc;
@@ -1249,86 +1206,43 @@ void scan_lengths(const frc_tree_t* caller, const frc_tree_t* tree, bool* bad, b
   *bad = b; *neg = n;
 }
 
-// How the sample shards of the embedding meet.  It depends on nothing the staging produces, so it is decided before
-// the staging starts, which then knows the rows a sharded rank reads (Shared::rows_read).
-void plan_exchange(Shared& sh, const frc_ctx* c) {
-  sh.fused_embed = !sh.knobs.embed_levels;
-  sh.exchange = Shared::kNone;
-  if (sh.exact) return;
-  if (sh.n_parts > 1 && c->peer_ok && sh.knobs.shard != 0 && (sh.weighted || sh.fused_embed)) sh.exchange = Shared::kInProcess;
-  if (sh.n_parts == 1 && sh.world > 1 && (sh.opts.flags & FRC_FLAG_SHARD_EMBED)) sh.exchange = Shared::kNccl;
+// What the variant of the job depends on (plan_exchange, plan_variant).
+VariantIn variant_in(const Shared& sh, const frc_ctx* c) {
+  VariantIn in;
+  in.exact = sh.exact; in.weighted = sh.weighted; in.keyed = sh.keyed; in.rect = sh.geo.rect;
+  in.flags = sh.opts.flags; in.world = sh.world; in.rank = sh.rank0; in.N = sh.N;
+  in.n_parts = sh.n_parts; in.peer_ok = c->peer_ok;
+  if (c->comm) { in.comm_world = comm_world(c->comm); in.comm_rank = comm_rank(c->comm); }
+  return in;
 }
 
-// (3) the plan that does not depend on the table: operand columns; then bands + owners.
+// (3) the plan that does not depend on the table: the variant and the operand columns; then bands + owners.
 int plan_job(frc_job* j, const frc_tree_t* tree, bool neg_len) {
   Shared& sh = j->sh;
   frc_ctx* c = j->ctx;
-  const int n_parts = sh.n_parts;
-  const bool fast_uw = !sh.exact && !sh.weighted;
-  if (sh.exchange == Shared::kNccl) {
-    if (!c->comm || comm_world(c->comm) != sh.world || comm_rank(c->comm) != sh.rank0)
-      return fail(j, FRC_ERR_STATE, "FRC_FLAG_SHARD_EMBED needs a context whose communicator "
-                                    "(frc_ctx_comm_init) matches opts->rank / opts->world");
-    if (fast_uw && !sh.fused_embed) return fail(j, FRC_ERR_UNSUPPORTED, "FRC_EMBED_LEVELS=1 cannot build a sample shard");
-  }
+  auto free_hbm = [c](size_t* free_b) {
+    size_t total_b = 0;
+    cudaSetDevice(c->devs[0]->device);
+    const bool ok = cudaMemGetInfo(free_b, &total_b) == cudaSuccess;
+    cudaGetLastError();
+    return ok;
+  };
+  std::string err;
+  if (int rc = plan_variant(sh.variant, variant_in(sh, c), sh.knobs, neg_len, tree->length, sh.B, tc_chunk_kblocks(),
+                            free_hbm, &sh.cols, &err))
+    return fail(j, rc, err);
   const int owners = sh.owners();
-  ShardPlan::Mode mode = sh.exchange == Shared::kNone ? ShardPlan::kWhole : ShardPlan::kSharded;
-  // Capacity mode of the fast weighted path: the fp32 panels of ALL samples (kp x np x 4 bytes: 320 GB at
-  // BASELINE config 5) would not fit one device -> they stay sharded where they are built (two shards per
-  // device) and the pair tiles read remote column panels over NVLink (PanelMap, weighted.cu).
-  if (sh.exchange == Shared::kInProcess && sh.weighted && sh.knobs.capacity != 0 && sh.N >= 2) {
-    bool want = sh.knobs.capacity == 1;
-    if (!want) {
-      // (keyed -l tiles: an int32 key next to every fp32 value)
-      const double panels = (sh.keyed ? 8.0 : 4.0) * static_cast<double>(round_up(sh.B, kKBlock)) * static_cast<double>(plan_shards(sh.N, n_parts, ShardPlan::kCapacity).np);
-      if (panels > 24.0 * (1 << 30)) {  // (cudaMemGetInfo costs milliseconds: only asked when it can matter)
-        size_t free_b = 0, total_b = 0;
-        cudaSetDevice(c->devs[0]->device);
-        if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && panels > 0.55 * static_cast<double>(free_b)) want = true;
-        cudaGetLastError();
-      }
-    }
-    if (want && sh.geo.rect)
-      return fail(j, FRC_ERR_UNSUPPORTED, "frc_create_cross keeps the weighted panels of all samples on every device; the "
-                                          "capacity mode, which shards them over the devices when they exceed about half "
-                                          "of one device's free HBM (or with FRC_CAPACITY=1), only runs triangle jobs");
-    if (want && sh.keyed)
-      return fail(j, FRC_ERR_UNSUPPORTED, "the key-matched tiles of -l as coded (FRC_FLAG_L_TILES) keep the value and key "
-                                          "panels of all samples on every device; the capacity mode, which shards them "
-                                          "over the devices when they exceed about half of one device's free HBM (or with "
-                                          "FRC_CAPACITY=1), does not carry keys");
-    sh.capacity = want;
-    if (want) mode = ShardPlan::kCapacity;
-  }
-  sh.shards = plan_shards(sh.N, owners, mode);
+  sh.shards = plan_shards(sh.N, owners, sh.variant.shard_mode);
   sh.np = sh.shards.np;
   sh.nw = static_cast<int32_t>(sh.np / 32);
-  sh.kp = static_cast<int32_t>(round_up(sh.B, kKBlock));
+  sh.kp = !sh.exact && !sh.weighted ? sh.cols.kp : static_cast<int32_t>(round_up(sh.B, kKBlock));
   sh.prescale = !neg_len;
-  if (fast_uw) {
-    const bool want_i8 = sh.fused_embed && !neg_len && !(sh.opts.flags & FRC_FLAG_UW_BF16) && !sh.knobs.uw_bf16;
-    sh.cols = plan_columns(tree->length, sh.B, want_i8, sh.knobs.group_binades, sh.knobs.u8_acc_f64, tc_chunk_kblocks());
-    sh.kp = sh.cols.kp;
-    sh.bits_feed = sh.cols.intacc && ((sh.opts.flags & FRC_FLAG_UW_BITS) != 0 || sh.knobs.feed_bits);
-    if (sh.cols.intacc && !sh.bits_feed) {
-      // capacity: when the three u8 operand arrays would not fit the free HBM (with room for the
-      // output ring), the pair kernel expands its tiles from the bit rows instead (8x less memory,
-      // about half the speed: DESIGN.md)
-      const double need = 3.0 * static_cast<double>(sh.np) * sh.kp;
-      if (need > 32.0 * (1 << 30)) {  // (cudaMemGetInfo costs milliseconds: only asked when it can matter)
-        size_t free_b = 0, total_b = 0;
-        cudaSetDevice(c->devs[0]->device);
-        if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && need > 0.80 * static_cast<double>(free_b)) sh.bits_feed = true;
-        cudaGetLastError();
-      }
-    }
-  }
   if (sh.geo.rect)
     sh.bands = make_bands_cross(sh.geo.q0, sh.N - sh.geo.q0, sh.geo.n_ref, sh.opts.band_rows, owners, sh.d2h,
                                 sh.knobs.bands_per_rank, 8);
   else
-    sh.bands = sh.capacity ? make_bands_capacity(sh.N, sh.shards, sh.opts.band_rows, sh.d2h)
-                           : make_bands(sh.N, sh.opts.band_rows, owners, sh.d2h, sh.knobs.bands_per_rank, 8);
+    sh.bands = sh.variant.capacity ? make_bands_capacity(sh.N, sh.shards, sh.opts.band_rows, sh.d2h)
+                                   : make_bands(sh.N, sh.opts.band_rows, owners, sh.d2h, sh.knobs.bands_per_rank, 8);
   for (const Band& b : sh.bands)
     if (b.count >= (1LL << 32)) return fail(j, FRC_ERR_UNSUPPORTED, "band too large; lower band_rows");
   return FRC_OK;
@@ -1384,8 +1298,7 @@ int prepare_part(Part* p) {
       p->info.n_pairs_mine += sh.bands[k].count;
       p->max_band = std::max(p->max_band, sh.bands[k].count);
     }
-  const bool fast_uw = !sh.exact && !sh.weighted;
-  if (sh.capacity) {
+  if (sh.variant.capacity) {
     // one group per row shard of this part (csrc/plan.cpp): its bands, and its tiles grouped by COLUMN SHARD (the
     // order the shards visit in), column-major inside a column shard (the CTAs of a wave share a column panel)
     const std::vector<CapGroupPlan> groups =
@@ -1398,10 +1311,10 @@ int prepare_part(Part* p) {
     }
   } else if (!sh.exact) {
     const int32_t col_tiles = sh.geo.rect ? static_cast<int32_t>((sh.geo.n_ref + kTile - 1) / kTile) : 0;
-    for (Band& b : p->bands) append_band_tiles(b, fast_uw, p->tiles, col_tiles);
+    for (Band& b : p->bands) append_band_tiles(b, !sh.weighted, p->tiles, col_tiles);
   }
   std::vector<uint8_t> need;
-  if (fast_uw && sh.shards.ranges.size() > 1 && sh.fused_embed) need = operand_need_blocks(p->tiles, sh.np, true);
+  if (sh.variant.need_blocks) need = operand_need_blocks(p->tiles, sh.np, true);
   // ---- sample shard: the first range of this owner (capacity: the second one is as large)
   const Range& own = sh.shards.ranges[p->owner][0];
   p->shard_w0 = static_cast<int32_t>(own.s0 / 32);
@@ -1479,10 +1392,11 @@ int prepare_part(Part* p) {
     if (sh.unsorted_l && !(p->d_list_ptr = dev_alloc<int64_t>(p, sh.N + 2))) return p->rc;
     if (!sh.exact) {
       // resident: the panels of all samples; capacity: of this device's two shards only
-      const size_t a_samples = sh.capacity ? static_cast<size_t>(2 * sh.shards.shard_rows) : static_cast<size_t>(sh.np);
+      const size_t a_samples =
+          sh.variant.capacity ? static_cast<size_t>(2 * sh.shards.shard_rows) : static_cast<size_t>(sh.np);
       if (!(p->d_A = dev_alloc<float>(p, static_cast<size_t>(sh.kp) * a_samples))) return p->rc;
       if (sh.keyed && !(p->d_K = dev_alloc<int32_t>(p, static_cast<size_t>(sh.kp) * a_samples))) return p->rc;
-      if (sh.capacity) {
+      if (sh.variant.capacity) {
         for (int k = 0; k < 2; ++k)
           if (!(p->d_V[k] = dev_alloc<float>(p, static_cast<size_t>(sh.kp) * sh.shards.shard_rows))) return p->rc;
         p->ev_fetch.assign(sh.shards.n_shards, nullptr);
@@ -1508,8 +1422,8 @@ int prepare_part(Part* p) {
   } else {
     // fused: published columns bitsT[nw][kp] (+ node-indexed scratch for trees beyond shared memory);
     // FRC_EMBED_LEVELS=1: node-major bits[B][nw], one launch per tree level
-    const size_t words = sh.fused_embed ? static_cast<size_t>(sh.kp) * sh.nw : static_cast<size_t>(B) * sh.nw;
-    p->peer_push = sh.exchange == Shared::kNccl && !sh.bits_feed && sh.world <= 8 && sh.knobs.peer_push != 0;
+    const size_t words = sh.variant.fused_embed ? static_cast<size_t>(sh.kp) * sh.nw : static_cast<size_t>(B) * sh.nw;
+    p->peer_push = sh.variant.peer_push;
     if (p->peer_push) {
       // two buffers from the symmetric heap (same block + offset on every rank), mapped from the peers
       for (int k = 0; k < 2; ++k) {
@@ -1535,13 +1449,13 @@ int prepare_part(Part* p) {
       }
       p->d_bits = p->d_bits2[0];
     } else if (!(p->d_bits = dev_alloc<uint32_t>(p, std::max<size_t>(words, 64)))) return p->rc;
-    const size_t ns = sh.fused_embed ? static_cast<size_t>(presence_node_scratch_words(B, p->shard_nw)) : 0;
+    const size_t ns = sh.variant.fused_embed ? static_cast<size_t>(presence_node_scratch_words(B, p->shard_nw)) : 0;
     if (ns && !(p->d_node_scratch = dev_alloc<uint32_t>(p, ns))) return p->rc;
-    const size_t opsz = sh.bits_feed ? 256 : static_cast<size_t>(sh.np) * sh.kp * (i8 ? 1 : 2);
+    const size_t opsz = sh.variant.bits_feed ? 256 : static_cast<size_t>(sh.np) * sh.kp * (i8 ? 1 : 2);
     if (!(p->d_P = dev_alloc<char>(p, opsz))) return p->rc;
     if (!(p->d_Bh = dev_alloc<char>(p, opsz))) return p->rc;
     if (!(p->d_Bl = dev_alloc<char>(p, opsz))) return p->rc;
-    if (sh.bits_feed && !(p->d_bitsS = dev_alloc<uint32_t>(p, static_cast<size_t>(sh.np) * (sh.kp / 32)))) return p->rc;
+    if (sh.variant.bits_feed && !(p->d_bitsS = dev_alloc<uint32_t>(p, static_cast<size_t>(sh.np) * (sh.kp / 32)))) return p->rc;
     if (!(p->d_r = dev_alloc<double>(p, sh.np))) return p->rc;
     if (!(p->d_scratch = dev_alloc<double>(p, static_cast<size_t>(chunks) * sh.np))) return p->rc;
     if (!(p->d_flag_counts = dev_alloc<unsigned long long>(p, p->mine.size() + 1))) return p->rc;
@@ -1550,7 +1464,7 @@ int prepare_part(Part* p) {
     if (i8 && !(p->d_qam = dev_alloc<uint32_t>(p, sh.kp))) return p->rc;
     if (intacc && !(p->d_r_int = dev_alloc<long long>(p, sh.np))) return p->rc;
     std::string terr;
-    if (sh.bits_feed) {
+    if (sh.variant.bits_feed) {
       p->tc = tc_operands_create_bits(p->d_bitsS, sh.np, sh.kp, static_cast<const uint8_t*>(p->d_q0),
                                       static_cast<const uint8_t*>(p->d_q1), static_cast<const uint8_t*>(p->d_q2),
                                       p->d_chunks, p->d_len_col, p->d_flag_u, p->d_r_int,
@@ -1582,7 +1496,7 @@ int prepare_part(Part* p) {
     } else {
       if (sh.d2h && !(sl.host32 = pin_alloc<float>(p, p->max_band))) return p->rc;
       // (capacity mode: a band lives in its row-shard group's record, Part::CapGroup)
-      if (!sh.capacity && alloc_pair_out(p, sl.own, p->max_band)) return p->rc;
+      if (!sh.variant.capacity && alloc_pair_out(p, sl.own, p->max_band)) return p->rc;
     }
     for (cudaEvent_t* e : {&sl.k0, &sl.k1, &sl.k2, &sl.done}) PART_CUDA(p, cudaEventCreate(e));
   }
@@ -1628,7 +1542,7 @@ void aggregate_info(frc_job* j) {
   a.tree_height = sh.tree_height;
   a.n_pairs_total = sh.geo.rect ? (sh.N - sh.geo.q0) * sh.geo.n_ref : sh.N >= 2 ? tri(sh.N) : 0;
   a.n_nodes_padded = sh.exact ? sh.B : sh.kp;
-  a.operand_kind = (!sh.exact && !sh.weighted) ? (sh.cols.i8 ? (sh.bits_feed ? 3 : 2) : 1) : 0;
+  a.operand_kind = sh.variant.operand_kind;
   a.n_devices = static_cast<int32_t>(j->parts.size());
   a.value_bytes = sh.exact ? 8 : 4;
   a.create_ms = j->create_ms;
@@ -1676,7 +1590,7 @@ int attach_context(frc_job* j, frc_ctx_t* ctx, const frc_opts_t* opts) {
     p->job = j; p->sh = &sh; p->dc = c->devs[k]; p->index = k;
     p->owner = sh.n_parts > 1 ? k : sh.rank0;
   }
-  plan_exchange(sh, c);
+  sh.variant = plan_exchange(variant_in(sh, c), sh.knobs);
   return FRC_OK;
 }
 
@@ -1874,7 +1788,7 @@ int part_wait_band(Part* p, size_t idx, Slot** out) {
   const auto tn0 = std::chrono::steady_clock::now();
   PART_CUDA(p, cudaEventSynchronize(sl.done));
   float ms = 0.f;
-  const bool spans = !sh.capacity;  // (capacity mode: a group's kernels serve all of its bands; no per-band span)
+  const bool spans = !sh.variant.capacity;  // (capacity mode: a group's kernels serve all of its bands; no per-band span)
   if (spans && (p->mine.size() <= 2 || sh.knobs.trace)) {
     // per-band kernel spans (info.pairs_ms / fixup_ms): meaningful for a job of one or two bands (bench.py's
     // roofline leg); a many-band stream skips the four driver calls per band on the consumer's thread

@@ -5,6 +5,7 @@
 #include <climits>
 #include <cmath>
 #include <cstdio>
+#include <cstdlib>
 #include <cstring>
 
 #if defined(__x86_64__)
@@ -363,6 +364,95 @@ ColumnPlan plan_columns(const double* length, int32_t B, bool want_i8, int gb, b
   p.e_min = lo;
   for (double sc : p.chunk_scale) p.chunk_shift.push_back(std::ilogb(sc) - lo);
   return p;
+}
+
+Knobs Knobs::read() {
+  Knobs k;
+  auto num = [](const char* name, int dflt) { const char* e = getenv(name); return e && *e ? atoi(e) : dflt; };
+  auto is = [](const char* name, const char* v) { const char* e = getenv(name); return e && !strcmp(e, v); };
+  k.trace = getenv("FRC_TRACE") != nullptr;
+  k.bands_per_rank = std::max(0, num("FRC_BANDS", 0));
+  k.widen_threads = std::max(0, num("FRC_WIDEN_THREADS", 0));
+  k.ws_slab = std::max(0, num("FRC_WS_SLAB", 0));
+  k.uw_bf16 = is("FRC_UW_KERNEL", "bf16");
+  k.u8_acc_f64 = is("FRC_U8_ACC", "f64");
+  k.feed_bits = is("FRC_UW_FEED", "bits");
+  k.embed_levels = num("FRC_EMBED_LEVELS", 0) == 1;
+  k.peer_push = num("FRC_PEER_PUSH", -1);
+  k.group_binades = num("FRC_U8_GROUP_BINADES", 3);
+  k.shard = num("FRC_SHARD", -1);
+  k.capacity = num("FRC_CAPACITY", -1);
+  return k;
+}
+
+Variant plan_exchange(const VariantIn& in, const Knobs& k) {
+  Variant v;
+  v.fused_embed = !k.embed_levels;
+  if (in.exact) return v;
+  if (in.n_parts > 1 && in.peer_ok && k.shard != 0 && (in.weighted || v.fused_embed)) v.exchange = Variant::kInProcess;
+  if (in.n_parts == 1 && in.world > 1 && (in.flags & FRC_FLAG_SHARD_EMBED)) v.exchange = Variant::kNccl;
+  v.sharded_fast_uw = v.exchange != Variant::kNone && !in.weighted;
+  return v;
+}
+
+int plan_variant(Variant& v, const VariantIn& in, const Knobs& k, bool neg_len, const double* length, int32_t B,
+                 int bf16_chunk_kblocks, const std::function<bool(size_t*)>& free_hbm, ColumnPlan* cols,
+                 std::string* err) {
+  const bool fast_uw = !in.exact && !in.weighted;
+  auto refuse = [&](int code, const char* msg) { *err = msg; return code; };
+  if (v.exchange == Variant::kNccl) {
+    if (in.comm_world != in.world || in.comm_rank != in.rank)
+      return refuse(FRC_ERR_STATE, "FRC_FLAG_SHARD_EMBED needs a context whose communicator "
+                                   "(frc_ctx_comm_init) matches opts->rank / opts->world");
+    if (fast_uw && !v.fused_embed) return refuse(FRC_ERR_UNSUPPORTED, "FRC_EMBED_LEVELS=1 cannot build a sample shard");
+  }
+  v.shard_mode = v.exchange == Variant::kNone ? ShardPlan::kWhole : ShardPlan::kSharded;
+  // (free_hbm costs milliseconds, a cudaMemGetInfo: only asked when it can matter)
+  size_t free_b = 0;
+  // Capacity mode of the fast weighted path: the fp32 panels of ALL samples (kp x np x 4 bytes: 320 GB at
+  // BASELINE config 5) would not fit one device -> they stay sharded where they are built (two shards per
+  // device) and the pair tiles read remote column panels over NVLink (PanelMap, weighted.cu).
+  if (v.exchange == Variant::kInProcess && in.weighted && k.capacity != 0 && in.N >= 2) {
+    bool want = k.capacity == 1;
+    if (!want) {
+      // (keyed -l tiles: an int32 key next to every fp32 value)
+      const double panels = (in.keyed ? 8.0 : 4.0) * static_cast<double>(round_up(B, kKBlock)) *
+                            static_cast<double>(plan_shards(in.N, in.n_parts, ShardPlan::kCapacity).np);
+      if (panels > 24.0 * (1 << 30) && free_hbm(&free_b) && panels > 0.55 * static_cast<double>(free_b)) want = true;
+    }
+    if (want && in.rect)
+      return refuse(FRC_ERR_UNSUPPORTED, "frc_create_cross keeps the weighted panels of all samples on every device; the "
+                                         "capacity mode, which shards them over the devices when they exceed about half "
+                                         "of one device's free HBM (or with FRC_CAPACITY=1), only runs triangle jobs");
+    if (want && in.keyed)
+      return refuse(FRC_ERR_UNSUPPORTED, "the key-matched tiles of -l as coded (FRC_FLAG_L_TILES) keep the value and key "
+                                         "panels of all samples on every device; the capacity mode, which shards them "
+                                         "over the devices when they exceed about half of one device's free HBM (or with "
+                                         "FRC_CAPACITY=1), does not carry keys");
+    v.capacity = want;
+    if (want) v.shard_mode = ShardPlan::kCapacity;
+  }
+  if (!fast_uw) return FRC_OK;
+  v.want_i8 = v.fused_embed && !neg_len && !(in.flags & FRC_FLAG_UW_BF16) && !k.uw_bf16;
+  *cols = plan_columns(length, B, v.want_i8, k.group_binades, k.u8_acc_f64, bf16_chunk_kblocks);
+  v.bits_feed = cols->intacc && ((in.flags & FRC_FLAG_UW_BITS) != 0 || k.feed_bits);
+  if (cols->intacc && !v.bits_feed) {
+    // capacity: when the three u8 operand arrays would not fit the free HBM (with room for the
+    // output ring), the pair kernel expands its tiles from the bit rows instead (8x less memory,
+    // about half the speed: DESIGN.md)
+    const double need = 3.0 * static_cast<double>(plan_shards(in.N, in.owners(), v.shard_mode).np) * cols->kp;
+    if (need > 32.0 * (1 << 30) && free_hbm(&free_b) && need > 0.80 * static_cast<double>(free_b)) v.bits_feed = true;
+  }
+  // Row sums.  Integer mode with materialised operands: the operand expansion produces them for every sample from
+  // the words it holds anyway.  Otherwise a separate pass over this part's shard, beside the expansion on the second
+  // compute stream unless an exchange sits between.
+  v.rowsum_in_expand = cols->intacc && !v.bits_feed;
+  v.rowsum_split = v.fused_embed && v.exchange == Variant::kNone && !v.rowsum_in_expand;
+  v.peer_store = v.exchange == Variant::kInProcess && !v.bits_feed;
+  v.peer_push = v.exchange == Variant::kNccl && !v.bits_feed && in.world <= 8 && k.peer_push != 0;
+  v.need_blocks = v.fused_embed && in.owners() > 1;
+  v.operand_kind = cols->i8 ? (v.bits_feed ? 3 : 2) : 1;
+  return FRC_OK;
 }
 
 void append_band_tiles(Band& b, bool pair_tiles, std::vector<Tile>& tiles, int32_t col_tiles) {
@@ -764,6 +854,38 @@ int64_t frc_debug_stage(const int32_t* parent, int32_t n_nodes, int64_t n_ref, c
 void frc_debug_rows_read(int64_t n_samples, int32_t owners, int32_t owner, int32_t sharded_fast_uw, int64_t* out2) {
   const std::pair<int64_t, int64_t> r = frc::rows_read(n_samples, owners, owner, sharded_fast_uw != 0);
   out2[0] = r.first; out2[1] = r.second;
+}
+
+// The variant frc_create plans (plan_exchange, then plan_variant), with the knobs read from the environment and
+// free_hbm as device 0's free HBM (negative: the query fails).  out16 = {exchange, fused_embed, sharded_fast_uw,
+// capacity, shard_mode, want_i8, bits_feed, rowsum_in_expand, rowsum_split, peer_store, peer_push, need_blocks,
+// operand_kind, columns' intacc, columns' kp, free-HBM queries}.  Returns the error code and writes its message
+// (NUL-terminated, cut to msg_cap) into msg.
+int32_t frc_debug_plan_variant(int32_t weighted, int32_t exact, int32_t keyed, int32_t rect, uint32_t flags, int32_t world,
+                               int32_t rank, int64_t n_samples, const double* length, int32_t n_nodes, int32_t n_parts,
+                               int32_t peer_ok, int32_t comm_world, int32_t comm_rank, int32_t neg_len, int64_t free_hbm,
+                               int64_t* out16, char* msg, int64_t msg_cap) {
+  frc::VariantIn in;
+  in.exact = exact != 0; in.weighted = weighted != 0; in.keyed = keyed != 0; in.rect = rect != 0;
+  in.flags = flags; in.world = world; in.rank = rank; in.N = n_samples;
+  in.n_parts = n_parts; in.peer_ok = peer_ok != 0; in.comm_world = comm_world; in.comm_rank = comm_rank;
+  const frc::Knobs k = frc::Knobs::read();
+  int64_t asked = 0;
+  auto query = [&](size_t* bytes) {
+    ++asked;
+    *bytes = free_hbm < 0 ? 0 : static_cast<size_t>(free_hbm);
+    return free_hbm >= 0;
+  };
+  frc::Variant v = frc::plan_exchange(in, k);
+  frc::ColumnPlan cols;
+  std::string err;
+  const int rc = frc::plan_variant(v, in, k, neg_len != 0, length, n_nodes, 64, query, &cols, &err);
+  const int64_t f[16] = {v.exchange, v.fused_embed, v.sharded_fast_uw, v.capacity, v.shard_mode, v.want_i8, v.bits_feed,
+                         v.rowsum_in_expand, v.rowsum_split, v.peer_store, v.peer_push, v.need_blocks, v.operand_kind,
+                         cols.intacc, cols.kp, asked};
+  memcpy(out16, f, sizeof(f));
+  snprintf(msg, static_cast<size_t>(msg_cap), "%s", err.c_str());
+  return rc;
 }
 
 }  // extern "C"

@@ -8,8 +8,10 @@
 //   tree walk      pre-order check, children lists, level order (what enumerateNodes' numbering implies,
 //                  frcfrc/unifrac.go:127-133)
 //   table staging  the caller's CSR entries checked and copied into the staged table (tests/test_stage.py)
+//   variant        which variant of the fast path a job runs (tests/test_variant.py)
 #pragma once
 #include <cstdint>
+#include <functional>
 #include <string>
 #include <utility>
 #include <vector>
@@ -18,6 +20,24 @@
 #include "frc_internal.h"
 
 namespace frc {
+
+// Environment knobs (tests and experiments; DESIGN.md has the table).  Read ONCE per frc_create: nothing
+// on the per-band path calls getenv.
+struct Knobs {
+  bool trace = false;
+  int bands_per_rank = 0;     // FRC_BANDS
+  int widen_threads = 0;      // FRC_WIDEN_THREADS
+  int ws_slab = 0;            // FRC_WS_SLAB
+  bool uw_bf16 = false;       // FRC_UW_KERNEL=bf16
+  bool u8_acc_f64 = false;    // FRC_U8_ACC=f64
+  bool feed_bits = false;     // FRC_UW_FEED=bits
+  bool embed_levels = false;  // FRC_EMBED_LEVELS=1
+  int peer_push = -1;         // FRC_PEER_PUSH (multi-process sharding: 0 = NCCL all-gather of the bits)
+  int group_binades = 3;      // FRC_U8_GROUP_BINADES
+  int shard = -1;             // FRC_SHARD (in-process multi-GPU: 0 = every device rebuilds the embedding)
+  int capacity = -1;          // FRC_CAPACITY (in-process multi-GPU, fast weighted: 1 / 0 = force / forbid the sharded-panel mode)
+  static Knobs read();
+};
 
 struct Band {
   int64_t row0 = 0, row1 = 0;   // rows [row0, row1) of the triangle
@@ -98,6 +118,45 @@ struct ColumnPlan {
 };
 ColumnPlan plan_columns(const double* length, int32_t n_nodes, bool want_i8, int group_binades, bool force_f64_acc,
                         int bf16_chunk_kblocks);
+
+// Which variant of the fast path a job runs.  plan_exchange fills the first three fields before the staging starts
+// (the staging needs rows_read); plan_variant the rest once the branch lengths are known.  Every stage reads it.
+struct Variant {
+  enum Exchange { kNone, kInProcess, kNccl };
+  Exchange exchange = kNone;     // how the sample shards of the embedding meet
+  bool fused_embed = true;       // unweighted embedding: one fused kernel (FRC_EMBED_LEVELS=1: one launch per level)
+  bool sharded_fast_uw = false;  // rows_read: an owner reads only its own shard's rows
+  bool capacity = false;         // fast weighted over several devices: panels stay sharded (PanelMap), tiles read peers' HBM
+  ShardPlan::Mode shard_mode = ShardPlan::kWhole;
+  // fast unweighted only (false / 0 otherwise)
+  bool want_i8 = false;          // u8 operands (plan_columns) rather than bf16
+  bool bits_feed = false;        // integer mode: the pair kernel expands its tiles from the bit rows
+  bool rowsum_in_expand = false; // the operand expansion makes the integer row sums
+  bool rowsum_split = false;     // fused, no exchange: the row-sum pass runs on the second compute stream
+  bool peer_store = false;       // kInProcess: the embedding kernel stores its bit columns into every device
+  bool peer_push = false;        // kNccl: the same into every rank over IPC (wanted; prepare_part may fall back)
+  bool need_blocks = false;      // several owners: the expansion fills only the operand rows this owner's tiles read
+  int operand_kind = 0;          // frc_info_t::operand_kind: 0 none, 1 bf16, 2 u8, 3 u8 from the bits
+};
+// What the variant depends on: the options, the path taken, the context.
+struct VariantIn {
+  bool exact = false, weighted = false, keyed = false, rect = false;
+  uint32_t flags = 0;
+  int world = 1, rank = 0;              // opts (world <= 0: 1)
+  int64_t N = 0;
+  int n_parts = 1;                      // devices of the context
+  bool peer_ok = false;
+  int comm_world = -1, comm_rank = -1;  // the context's communicator (-1: none)
+  int owners() const { return n_parts > 1 ? n_parts : world; }
+};
+Variant plan_exchange(const VariantIn& in, const Knobs& k);
+// The rest of `v` (from plan_exchange), and for the fast unweighted path the column plan of length[B] into *cols.
+// free_hbm(&bytes) gives device 0's free HBM (false: the query failed, which chooses neither mode); it is asked at
+// most once, and only when the panels or the u8 operands are large enough for the answer to matter.  Returns FRC_OK
+// or an error code with its message in *err.
+int plan_variant(Variant& v, const VariantIn& in, const Knobs& k, bool neg_len, const double* length, int32_t B,
+                 int bf16_chunk_kblocks, const std::function<bool(size_t*)>& free_hbm, ColumnPlan* cols,
+                 std::string* err);
 
 // Tiles of one band, appended to `tiles`: pair tiles (ti, tj) + (ti, tj + 1), tj even, walked in
 // super-tiles of ~9 tile rows x ~8 tile-pair columns when `pair_tiles` (tensor-core kernel), plain
